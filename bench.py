@@ -4,6 +4,7 @@ latency) of the cones_perception hot path on 130k-point scans.
 
     python bench.py --gpus N --steps K --warmup W            # ours (CUDA, libconesgpu.so)
     python bench.py --impl reference --gpus N ...            # the CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                   # also writes the last timed step's results as .npy
 
 A step = one pass of the whole hot path (ground removal -> crop -> VoxelGrid -> Euclidean
 clustering -> centroids) over one batch of synthetic scans: BASELINE.json config 3, the
@@ -241,6 +242,34 @@ def run_reference(args):
 
 
 # ------------------------------------------------------------------ ours
+DUMP_BYTES_MAX = 64_000_000
+NPY_HEADER_MAX = 4096            # an .npy header of a 1-D array is 128 bytes; counted generously
+
+
+def dump_outputs(out_dir: str, ctr, k_off, clusters, prefix: str = "", budget: int = DUMP_BYTES_MAX) -> None:
+    """Writes one step's results, what ConesGpu.results() hands a caller, as float .npy files so that two builds
+    can be compared output for output: per-frame counters, cluster offsets and the cluster records field by field.
+    Integers are stored as float64 (exact below 2**53).  Cluster lists larger than the byte budget are cut to a
+    seeded random subset of records, whose indices are stored beside them.  `budget` bounds the files' total size,
+    headers included."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {f"counters_{n}": ctr[n].astype(np.float64) for n in ctr.dtype.names}
+    arrays["cluster_offsets"] = k_off.astype(np.float64)
+    fixed = sum(a.nbytes for a in arrays.values()) + (len(arrays) + 5) * NPY_HEADER_MAX
+    per_record = 4 + 4 + 8 + 8 + 8          # x, y (float32) + size, min_index, sample index (float64)
+    keep = max(0, (budget - fixed) // per_record)
+    if len(clusters) > keep:
+        idx = np.sort(np.random.default_rng(0).choice(len(clusters), keep, replace=False))
+        clusters = clusters[idx]
+        arrays["clusters_sample_index"] = idx.astype(np.float64)
+    for n in ("x", "y"):
+        arrays[f"clusters_{n}"] = np.ascontiguousarray(clusters[n], np.float32)
+    for n in ("size", "min_index"):
+        arrays[f"clusters_{n}"] = clusters[n].astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), a)
+
+
 class _DevArray:
     """Zero-copy torch view of a raw device pointer (result buffers of the library)."""
 
@@ -421,6 +450,11 @@ def run_ours(args):
     gpu.sync()
     for h in lanes:
         h.sync()
+    if args.dump_outputs:
+        # the handle that ran the last timed step still holds its results (nothing has run on it since); every
+        # rank writes its own, and together they stay within the byte budget
+        dump_outputs(args.dump_outputs, *lanes[(args.steps - 1) % len(lanes)].results(),
+                     prefix=f"rank{rank}_" if world > 1 else "", budget=DUMP_BYTES_MAX // world)
     if gather_mode == "peer" and rank == 0:
         last = lanes[(args.steps - 1) % len(lanes)]
         seq = last.gather_seq()
@@ -1039,7 +1073,17 @@ def main():
     ap.add_argument("--strong-frames", type=int, default=4096, help="global batch of the strong-scaling sub-record")
     ap.add_argument("--cpu-step-frames", type=int, default=0,
                     help="frames per step of --impl reference (0 = --frames-per-gpu, the CUDA arm's batch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's counters, cluster offsets and clusters as "
+                         "DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's results (--impl ours)")
+    if args.dump_outputs and os.path.isdir(args.dump_outputs) and os.listdir(args.dump_outputs):
+        # files of an earlier run (another --gpus, a sample) would sit beside the new ones and be compared too
+        ap.error(f"--dump-outputs {args.dump_outputs} is not empty")
     if args.impl == "reference":
         run_reference(args)
     else:

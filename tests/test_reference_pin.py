@@ -1,9 +1,13 @@
-"""The oracle against the REFERENCE'S OWN CODE: oracle/_ref/libconesref.so is built from
-/root/reference/src/{ground_removal,cone_detection}.cpp and src/perception_handling/utils.cpp, compiled
+"""The oracle against the REFERENCE'S OWN CODE: oracle/_ref/libconesref.so is built from the reference project's
+src/{ground_removal,cone_detection}.cpp and src/perception_handling/utils.cpp, compiled
 unmodified (-O0, the reference's default catkin build) against the stand-in ROS/PCL surface in oracle/ref_shim.
 Everything the reference wrote itself runs for real; only PCL's VoxelGrid / EuclideanClusterExtraction inside
-it are the oracle's pcl_faithful restatement (PCL is not installed).  CPU only; skipped where neither the
-prebuilt library nor /root/reference exists."""
+it are the oracle's pcl_faithful restatement (PCL is not installed).  CPU only.
+
+Those sources are not part of this repository (oracle/Makefile `ref` builds the library where they are).  Without
+the library, a case runs against what the real nodes published for the same input where
+tests/golden/reference_nodes.npz holds that recording, and skips otherwise."""
+import hashlib
 import os
 
 import numpy as np
@@ -15,7 +19,13 @@ from oracle import oracle as O
 from oracle import ref as R
 from tests.util import TrackerReference, boundary_cloud
 
-pytestmark = pytest.mark.skipif(not R.available(), reason="oracle/_ref/libconesref.so not built and no /root/reference")
+NO_NODES = ("the reference's compiled nodes (oracle/_ref/libconesref.so, built from the reference project's sources) "
+            "are not present, and tests/golden/reference_nodes.npz holds no recording of this case")
+needs_nodes = pytest.mark.skipif(not R.available(), reason=NO_NODES)
+
+
+def _recorded():
+    return np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_nodes.npz"))
 
 
 def outside_sector_16(xyzi):
@@ -38,6 +48,7 @@ def as_arrays(clouds):
     return [np.array([(p[0], p[1]) for p in c], np.float32).reshape(-1, 2) for c in clouds]
 
 
+@needs_nodes
 def test_euclidan_dist_is_the_references():
     rng = np.random.default_rng(0)
     pts = rng.normal(0, 5, (2000, 6)).astype(np.float32)
@@ -49,17 +60,28 @@ def test_euclidan_dist_is_the_references():
 @pytest.mark.parametrize("cfg_idx,seed,intensity", [(2, 0, True), (2, 9, False), (1, 3, True)])
 def test_ground_node_bit_exact(cfg_idx, seed, intensity):
     frame = outside_sector_16(scans.generate(scans.config(cfg_idx), 1, base_seed=seed)[0])
-    node = R.GroundNode()
-    got, (step, n_fields, nsec) = node.handle(frame, with_intensity_field=intensity)
-    node.close()
     view = O.view_of_xyzi(frame, with_intensity=intensity)
     exp, kept, _, _ = O.ground_node(view, GroundParams())
     e = np.stack([exp[n] for n in ("x", "y", "z", "pad", "intensity", "c1", "c2", "c3")], 1)
-    assert np.array_equal(got.view(np.uint32), e.view(np.uint32))
+    if R.available():
+        node = R.GroundNode()
+        got, (step, n_fields, nsec) = node.handle(frame, with_intensity_field=intensity)
+        node.close()
+        assert np.array_equal(got.view(np.uint32), e.view(np.uint32))
+    else:
+        # recorded: config 2 with an intensity field (full cloud as sha256, first 256 points verbatim)
+        z, key = _recorded(), f"ground_seed{seed}"
+        if cfg_idx != 2 or not intensity or f"{key}_sha256" not in z.files:
+            pytest.skip(NO_NODES)
+        assert hashlib.sha256(frame.tobytes()).hexdigest() == str(z[f"{key}_input_sha256"])
+        assert np.array_equal(e[:256].view(np.uint32), z[f"{key}_head"].view(np.uint32))
+        assert hashlib.sha256(e.tobytes()).hexdigest() == str(z[f"{key}_sha256"])
+        step, n_fields, nsec = (int(v) for v in z[f"{key}_meta"])
     assert 0 < kept < len(frame)
     assert step == 32 and n_fields == 4 and nsec == 123456000      # PCL layout out, stamp truncated to microseconds
 
 
+@needs_nodes
 def test_ground_node_on_threshold_points():
     """Points on / one ulp around every sector boundary and around low[s] + 0.1: the reference's float atan2,
     float division, floor and double comparison against the oracle's definitions."""
@@ -81,11 +103,15 @@ def test_detect_node_sequence_bit_exact(buffer):
     radial extension and temporal gate are the reference's compiled code."""
     cfg = scans.config(1)
     d = cfg.detect
-    node = R.DetectNode(service=False, **node_params(d, classify_colors=False, use_points_buffer=buffer))
+    node = R.DetectNode(service=False, **node_params(d, classify_colors=False, use_points_buffer=buffer)) \
+        if R.available() else None
+    z = _recorded()
     ref = TrackerReference(False, buffer, d.cones_matching_dist_theshold, d.cone_position_extension_length)
     published = 0
-    for f in scans.generate(cfg, 5, base_seed=40):
-        got = node.handle(f)
+    for fi, f in enumerate(scans.generate(cfg, 5, base_seed=40)):
+        # recorded: the node's cones topic; without classify_colors it publishes nothing on the colour topics
+        got = node.handle(f) if node else \
+            [z[f"detect_buffer{int(buffer)}_frame{fi}"]] + [np.zeros((0, 2), np.float32)] * 3
         cl, _, _ = O.detect(O.view_of_xyzi(f), d, None, O.PCL_FAITHFUL)
         canon, _, _ = O.detect(O.view_of_xyzi(f), d, None, O.CANONICAL)
         exp = as_arrays(ref.update([(c["x"], c["y"]) for c in cl]))
@@ -98,10 +124,12 @@ def test_detect_node_sequence_bit_exact(buffer):
         assert a.shape == b.shape and np.allclose(a, b, rtol=0, atol=1e-5)
         assert sorted(cl["size"].tolist()) == sorted(canon["size"].tolist())
         published += sum(len(g) for g in got)
-    node.close()
+    if node:
+        node.close()
     assert published > 20
 
 
+@needs_nodes
 def test_ground_then_detect_chain_matches_fused_oracle():
     """ground_removal node -> cone_detection node chained like the launch file does (32-byte PCL cloud with zero
     padding in between) against the oracle's fused call."""
@@ -129,6 +157,7 @@ def test_ground_then_detect_chain_matches_fused_oracle():
     dnode.close()
 
 
+@needs_nodes
 def test_detect_node_crop_thresholds():
     """Isolated points on / one ulp around the level, distance and angle thresholds, min_cluster_size = 1: what
     survives the reference's crop lambda (src/cone_detection.cpp:191-203) shows up as one-point clusters."""
@@ -155,6 +184,7 @@ def test_detect_node_crop_thresholds():
     assert 10 < ctr.n_cropped < len(cloud)
 
 
+@needs_nodes
 @pytest.mark.parametrize("intensity_field", [True, False])
 def test_detect_node_colour_path(intensity_field):
     """classify_colors:=true with a deterministic stand-in service: get_reconstructed_cone (:222-238), the
@@ -198,6 +228,7 @@ def test_detect_node_colour_path(intensity_field):
     assert coloured > 10
 
 
+@needs_nodes
 def test_random_scenes_and_parameters_against_the_real_nodes():
     """Differential run: unstructured random clouds, random crop / cluster / leaf / gate parameters, two frames
     each, through the real nodes and through the oracle (+ tracker restatement).  (150 scenes were run once with
