@@ -31,6 +31,7 @@ ABI_SYMBOLS = [
     "cp_last_rows_loaded", "cp_last_pairs", "cp_cone_crops", "cp_cone_images", "cp_rasterize_crops",
     "cp_pinned_alloc", "cp_pinned_free",
     "cp_color_net_load", "cp_color_net_load_tflite", "cp_cone_colors", "cp_classify_images",
+    "cp_batch_cone_colors",
 ]
 
 CONE_IMG_ROWS, CONE_IMG_COLS = 15, 12
@@ -124,6 +125,7 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.cp_color_net_load_tflite.argtypes = [vp, vp, C.c_size_t, C.c_float]
     lib.cp_cone_colors.argtypes = [vp, C.POINTER(CCloudView), u32, vp, u32, C.c_float, vp, vp, vp]
     lib.cp_classify_images.argtypes = [vp, vp, u32, vp, vp, vp]
+    lib.cp_batch_cone_colors.argtypes = [vp, C.c_float, C.c_double, vp, vp, vp, vp, u64]
     lib.cp_pinned_alloc.argtypes = [C.c_int32, C.c_size_t, C.c_int32, C.POINTER(vp)]
     lib.cp_pinned_free.argtypes = [vp]
     lib.cp_pinned_free.restype = None
@@ -329,6 +331,20 @@ class ConesGpu:
         self._ck(self.lib.cp_cone_colors(self._h, C.byref(view) if view is not None else None, frame, c.ctypes.data,
                                          len(c), cone_width, colors.ctypes.data, probs.ctypes.data, flags.ctypes.data))
         return colors, probs, flags
+
+    def batch_cone_colors(self, cone_width: float = 0.228, extension_length: float = 0.05, n_classes: int = 3):
+        """handle_classify_color for every cluster record of the last run, at its centroid extended by
+        extension_length (src/cone_detection.cpp:276-278), on the run's own input.  Returns (colors u8 [K] with
+        255 = no answer, probs [K, classes], flags u32 [K], counts u32 [K] crop points), aligned with results()."""
+        total = C.c_uint64()
+        self._ck(self.lib.cp_batch_results(self._h, None, None, None, 0, C.byref(total)))
+        K = total.value
+        nc = getattr(self, "_n_classes", None) or n_classes
+        colors, probs = np.zeros(K, np.uint8), np.zeros((K, nc), np.float32)
+        flags, counts = np.zeros(K, np.uint32), np.zeros(K, np.uint32)
+        self._ck(self.lib.cp_batch_cone_colors(self._h, cone_width, extension_length, colors.ctypes.data,
+                                               probs.ctypes.data, flags.ctypes.data, counts.ctypes.data, K))
+        return colors, probs, flags, counts
 
     # ---- batches ----------------------------------------------------------------------
     def set_device_input(self, d_ptr: int, frame_points, point_step: int = 16, off=(0, 4, 8, 12), keep=None):

@@ -14,12 +14,13 @@
 // per cone travel back.
 //
 // Exactness.  The box test is the reference's double-precision comparison folded into four
-// fp32 bounds on the host (largest / smallest float on the right side of each double bound),
+// fp32 bounds by box_bounds (largest / smallest float on the right side of each double bound),
 // so the crops are bit-exact.  The raster evaluates the numpy formulas in fp64; the only
 // operation that is not correctly rounded on the device is atan2 (<= 2 ulp), which matters
 // only if a pixel coordinate lands within a guard band of a rounding boundary (x.5): such a
 // cone is flagged CP_CONE_AMBIGUOUS instead of being silently different.
 #pragma once
+#include "cluster_kernels.cuh"
 #include "stream_kernels.cuh"
 
 namespace cp {
@@ -136,6 +137,221 @@ __global__ void __launch_bounds__(kStreamThreads) cone_box_gather_kernel(
           crop_pts[dst] = load_point<MODE>(in, first_point + idx, L);
         }
       }
+    }
+  }
+}
+
+// src/cone_detection.cpp:226-227 as fp32 bounds: `c + hw >= (double)p` <=> p <= largest float <= c + hw, and
+// `c - hw <= (double)p` <=> p >= smallest float >= c - hw (every float is exactly representable as a double)
+__host__ __device__ inline void box_bounds(float c, double hw, float* lo, float* hi) {
+  const double dhi = (double)c + hw, dlo = (double)c - hw;
+  float fhi = (float)dhi, flo = (float)dlo;
+  if ((double)fhi > dhi) fhi = nextafterf(fhi, -INFINITY);
+  if ((double)flo < dlo) flo = nextafterf(flo, INFINITY);
+  *lo = flo;  // NaN centres give NaN bounds: nothing matches, like the reference
+  *hi = fhi;
+}
+
+// ---- every cluster of a batch run (cp_batch_cone_colors) ---------------------------------
+//   batch_box_kernel     extended centre (src/cone_detection.cpp:276-278) + box bounds + frame of each cluster
+//   batch_mark_kernel    one pass over the raw batch: a (cluster, frame row, ballot) triple for every non-empty
+//                        32-point row of every box of the row's frame, sort key cluster << row_bits | row
+//   batch_scan_kernel    crop offsets (points per cluster) and triple offsets (rows per cluster)
+//   (stable radix sort of the triples: cluster-major, rows in cloud order)
+//   batch_gather_kernel  one warp per cluster re-reads its matched rows into the packed crops
+// Scratch is O(K + triples); a triple holds at least one crop point, so the crop capacity bounds both.
+// batch ctl words: [0] triples found, [1] live sort-key bits, [2] triples to sort (min(found, capacity))
+constexpr u32 kBatchScanThreads = 1024;
+
+__global__ void __launch_bounds__(256) batch_box_kernel(const ClusterRec* __restrict__ cl, const u32* __restrict__ k_off,
+                                                        u32 n_frames, u32 K, double ext, double hw, u32 key_bits,
+                                                        float4* __restrict__ box, u32* __restrict__ kframe,
+                                                        u32* __restrict__ cnt, u32* __restrict__ tcnt, u32* __restrict__ ctl) {
+  const u32 k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k == 0) {
+    ctl[0] = 0u;
+    ctl[1] = key_bits;
+  }
+  if (k >= K) return;
+  u32 lo = 0, hi = n_frames;  // last frame f with k_off[f] <= k (empty frames share their offset with the next)
+  while (hi - lo > 1) {
+    const u32 mid = (lo + hi) >> 1;
+    if (k_off[mid] <= k) lo = mid; else hi = mid;
+  }
+  // vector_len = euclidan_dist(p.x, p.y, 0) in double, narrowed; p.x / len in float; the sum promotes to double.
+  // Explicit _rn intrinsics: no FMA contraction.
+  const float x = cl[k].x, y = cl[k].y;
+  const double s = __dadd_rn(__dmul_rn((double)x, (double)x), __dmul_rn((double)y, (double)y));
+  const float len = __double2float_rn(__dsqrt_rn(s));
+  const float ex = __double2float_rn(__dadd_rn((double)x, __dmul_rn((double)__fdiv_rn(x, len), ext)));
+  const float ey = __double2float_rn(__dadd_rn((double)y, __dmul_rn((double)__fdiv_rn(y, len), ext)));
+  float4 b;
+  box_bounds(ex, hw, &b.x, &b.y);
+  box_bounds(ey, hw, &b.z, &b.w);
+  box[k] = b;
+  kframe[k] = lo;
+  cnt[k] = 0u;
+  tcnt[k] = 0u;
+}
+
+__device__ __forceinline__ u64 frame_first_point(const Geom& g, u32 f) {
+  return g.uniform_n ? (u64)f * g.uniform_n : g.frame_off[f];
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(kStreamThreads) batch_mark_kernel(
+    const uint8_t* __restrict__ in, Layout L, const Geom g, const u32* __restrict__ k_off,
+    const float4* __restrict__ box, u32 row_bits, u32 cap, u64* __restrict__ keys, u32* __restrict__ vals,
+    u32* __restrict__ cnt, u32* __restrict__ tcnt, u32* __restrict__ ctl) {
+  const u32 warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (u32 tile = blockIdx.x; tile < g.n_tiles; tile += gridDim.x) {
+    u32 frame, local0, count;
+    u64 first;
+    tile_lookup(g, tile, frame, local0, count, first);
+    const u32 kb = k_off[frame], ke = k_off[frame + 1];
+    if (kb == ke) continue;  // a frame without clusters is never read
+    float4 p[kStreamRows];
+    bool valid[kStreamRows];
+#pragma unroll
+    for (int r = 0; r < kStreamRows; ++r) {
+      const u32 i = (warp * kStreamRows + r) * 32 + lane;
+      valid[r] = i < count;
+      p[r] = valid[r] ? load_point<MODE>(in, first + local0 + i, L) : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+    // NaN coordinates fail every comparison, like the reference's double comparisons
+    auto inside = [&](int r, const float4& b) {
+      return valid[r] && p[r].x >= b.x && p[r].x <= b.y && p[r].y >= b.z && p[r].y <= b.w;
+    };
+    // bounding rectangle of the warp's points (fminf / fmaxf skip NaN): a box that misses it holds none of them
+    float mnx = INFINITY, mxx = -INFINITY, mny = INFINITY, mxy = -INFINITY;
+#pragma unroll
+    for (int r = 0; r < kStreamRows; ++r)
+      if (valid[r]) {
+        mnx = fminf(mnx, p[r].x); mxx = fmaxf(mxx, p[r].x);
+        mny = fminf(mny, p[r].y); mxy = fmaxf(mxy, p[r].y);
+      }
+#pragma unroll
+    for (int d = 16; d; d >>= 1) {
+      mnx = fminf(mnx, __shfl_xor_sync(kFull, mnx, d)); mxx = fmaxf(mxx, __shfl_xor_sync(kFull, mxx, d));
+      mny = fminf(mny, __shfl_xor_sync(kFull, mny, d)); mxy = fmaxf(mxy, __shfl_xor_sync(kFull, mxy, d));
+    }
+    auto misses = [&](const float4& b) { return b.y < mnx || b.x > mxx || b.w < mny || b.z > mxy; };
+    // count the warp's non-empty (box, row) ballots, reserve that many slots with one atomic, then write them
+    u32 n = 0;
+    for (u32 k = kb; k < ke; ++k) {
+      const float4 b = box[k];
+      if (misses(b)) continue;  // uniform over the warp
+#pragma unroll
+      for (int r = 0; r < kStreamRows; ++r) n += __ballot_sync(kFull, inside(r, b)) != 0u;
+    }
+    if (n == 0) continue;
+    u32 slot = 0;
+    if (lane == 0) slot = atomicAdd(&ctl[0], n);
+    slot = __shfl_sync(kFull, slot, 0);
+    const u32 row0 = local0 / 32 + warp * kStreamRows;
+    for (u32 k = kb; k < ke; ++k) {
+      const float4 b = box[k];
+      if (misses(b)) continue;
+      u32 pts = 0, rows = 0;
+#pragma unroll
+      for (int r = 0; r < kStreamRows; ++r) {
+        const u32 bal = __ballot_sync(kFull, inside(r, b));
+        if (bal) {
+          if (lane == 0 && slot < cap) {
+            keys[slot] = ((u64)k << row_bits) | (row0 + r);
+            vals[slot] = bal;
+          }
+          ++slot;
+          pts += __popc(bal);
+          ++rows;
+        }
+      }
+      if (lane == 0 && rows) {
+        atomicAdd(&cnt[k], pts);
+        atomicAdd(&tcnt[k], rows);
+      }
+    }
+  }
+}
+
+// One CTA: exclusive scans of the per-cluster point and row counts (saturating: the host reports capacity).
+__global__ void __launch_bounds__(kBatchScanThreads) batch_scan_kernel(u32 K, const u32* __restrict__ cnt,
+                                                                       const u32* __restrict__ tcnt,
+                                                                       u32* __restrict__ off, u32* __restrict__ toff,
+                                                                       u32 cap, u32* __restrict__ ctl) {
+  __shared__ u64 wsum[2][kBatchScanThreads / 32];
+  const u32 tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  u64 carry0 = 0, carry1 = 0;
+  for (u32 base = 0; base < K; base += kBatchScanThreads) {
+    const u32 k = base + tid;
+    const u64 c0 = k < K ? cnt[k] : 0u, c1 = k < K ? tcnt[k] : 0u;
+    u64 s0 = c0, s1 = c1;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const u64 a = __shfl_up_sync(kFull, s0, d), b = __shfl_up_sync(kFull, s1, d);
+      if ((int)lane >= d) { s0 += a; s1 += b; }
+    }
+    if (lane == 31) { wsum[0][warp] = s0; wsum[1][warp] = s1; }
+    __syncthreads();
+    u64 w0 = 0, w1 = 0, t0 = 0, t1 = 0;
+    for (u32 w = 0; w < kBatchScanThreads / 32; ++w) {
+      if (w < warp) { w0 += wsum[0][w]; w1 += wsum[1][w]; }
+      t0 += wsum[0][w];
+      t1 += wsum[1][w];
+    }
+    if (k < K) {
+      const u64 e0 = carry0 + w0 + s0 - c0, e1 = carry1 + w1 + s1 - c1;
+      off[k] = e0 > 0xFFFFFFFFull ? 0xFFFFFFFFu : (u32)e0;
+      toff[k] = e1 > 0xFFFFFFFFull ? 0xFFFFFFFFu : (u32)e1;
+    }
+    carry0 += t0;
+    carry1 += t1;
+    __syncthreads();
+  }
+  if (tid == 0) {
+    off[K] = carry0 > 0xFFFFFFFFull ? 0xFFFFFFFFu : (u32)carry0;
+    toff[K] = carry1 > 0xFFFFFFFFull ? 0xFFFFFFFFu : (u32)carry1;
+    ctl[2] = min(ctl[0], cap);
+  }
+}
+
+// One warp per cluster, over its triples in sorted (cloud) order; crops land at off[k] in the layout of
+// cone_box_gather_kernel.  Nothing is written past `cap`; when the triples did not fit, nothing is gathered at
+// all (the sorted prefix does not line up with the triple offsets) and the host grows the buffers and runs again.
+template <int MODE>
+__global__ void __launch_bounds__(256) batch_gather_kernel(
+    const uint8_t* __restrict__ in, Layout L, const Geom g, u32 K, const u32* __restrict__ kframe,
+    const u64* __restrict__ keys, const u32* __restrict__ vals, const u32* __restrict__ toff,
+    const u32* __restrict__ off, u32 row_bits, u32 cap, const u32* __restrict__ ctl, float4* __restrict__ crop_pts) {
+  if (ctl[0] > cap) return;
+  const u32 lane = threadIdx.x & 31;
+  const u32 nwarps = gridDim.x * (blockDim.x >> 5);
+  const u64 row_mask = (1ull << row_bits) - 1ull;
+  for (u32 k = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); k < K; k += nwarps) {
+    const u32 t0 = toff[k], t1 = min(toff[k + 1], cap);
+    const u64 first = frame_first_point(g, kframe[k]);
+    u64 dst0 = off[k];
+    for (u32 tb = t0; tb < t1; tb += 32) {
+      const u32 t = tb + lane;
+      const u32 word = t < t1 ? vals[t] : 0u;
+      const u32 row = t < t1 ? (u32)(keys[t] & row_mask) : 0u;
+      const u32 c = __popc(word);
+      u32 incl = c;
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) {
+        const u32 o = __shfl_up_sync(kFull, incl, d);
+        if ((int)lane >= d) incl += o;
+      }
+      const u32 m = min(32u, t1 - tb);
+      for (u32 j = 0; j < m; ++j) {
+        const u32 wj = __shfl_sync(kFull, word, j), rj = __shfl_sync(kFull, row, j);
+        const u32 ej = __shfl_sync(kFull, incl - c, j);
+        if ((wj >> lane) & 1u) {
+          const u64 dst = dst0 + ej + __popc(wj & ((1u << lane) - 1u));
+          if (dst < cap) crop_pts[dst] = load_point<MODE>(in, first + (u64)rj * 32 + lane, L);
+        }
+      }
+      dst0 += __shfl_sync(kFull, incl, 31);
     }
   }
 }

@@ -229,7 +229,8 @@ uint64_t cp_last_rows_loaded(const cp_handle* h);
  * left early because both voxels already hung under the same root).  The reference's kd-tree visits
  * O(V * k log k) instead (src/cone_detection.cpp:206-220). */
 void cp_last_pairs(const cp_handle* h, uint64_t* visited, uint64_t* tested);
-/* Kernel launches enqueued by the last cp_batch_run / cp_detect / cp_ground_remove. */
+/* Kernel launches enqueued by the last cp_batch_run / cp_detect / cp_ground_remove / cp_batch_cone_colors (the
+ * latter counts its own launches only; it does not grow with the number of frames or clusters). */
 uint32_t cp_last_launch_count(const cp_handle* h);
 /* The handle's stream as a cudaStream_t, for callers that time with their own events. */
 void* cp_stream(cp_handle* h);
@@ -297,6 +298,23 @@ cp_status cp_color_net_load_tflite(cp_handle* h, const void* data, size_t bytes,
 #define CP_CONE_LOW_CONFIDENCE 16 /* the largest probability lies within 2e-6 of the threshold */
 cp_status cp_cone_colors(cp_handle* h, const cp_cloud_view* cloud, uint32_t frame, const cp_cone_center* centers,
                          uint32_t n_centers, float cone_width, uint8_t* colors, float* probs, uint32_t* flags);
+/* After a batch run (cp_batch_run, cp_detect_batch or cp_detect): handle_classify_color
+ * (scripts/color_classifier_server.py:78-126) for EVERY cluster record of the run, entirely on the device.
+ * Cluster k (the k-th record cp_batch_results returns, frame-major, canonical order) is classified at its
+ * centroid moved radially by extension_length (src/cone_detection.cpp:276-278, restated exactly), using the
+ * raw cloud of its own frame from the run's staged input.  One pass over the batch finds every crop.
+ *   colors[k]: 0 unknown, 1 yellow, 2 blue, 3 orange, 255 no answer (as cp_cone_colors)
+ *   probs  (optional) [K][n_classes], flags (optional) CP_CONE_* bits, counts (optional) crop points per cluster.
+ * The output is per cluster: the service's response rules (a shorter response when a crop is empty, a failed
+ * call when a crop is bad) depend on which cones a node sends, and `flags` holds what is needed to apply them.
+ * extension_length is the node parameter cone_position_extension_length (default 0.05).
+ * Calls cp_sync first (the final records can come from the back-half retry) and leaves the run's results
+ * (cp_batch_results, cp_device_results, the gather slot) untouched.  Device input must stay valid until this
+ * call returns.  CP_E_PARAM: non-finite extension_length, cone_width not positive and finite, NULL colors with
+ * clusters present.  CP_E_STATE: no run, input re-staged since the run, or no colour net loaded.
+ * CP_E_CAPACITY: cap < number of clusters. */
+cp_status cp_batch_cone_colors(cp_handle* h, float cone_width, double extension_length, uint8_t* colors,
+                               float* probs, uint32_t* flags, uint32_t* counts, uint64_t cap);
 /* The network alone on host images [n][15][12] uint8 (parity tests; logits optional, before the softmax). */
 cp_status cp_classify_images(cp_handle* h, const uint8_t* images, uint32_t n_images, uint8_t* colors, float* probs,
                              float* logits);
