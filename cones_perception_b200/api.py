@@ -31,7 +31,7 @@ ABI_SYMBOLS = [
     "cp_last_rows_loaded", "cp_last_pairs", "cp_cone_crops", "cp_cone_images", "cp_rasterize_crops",
     "cp_pinned_alloc", "cp_pinned_free",
     "cp_color_net_load", "cp_color_net_load_tflite", "cp_cone_colors", "cp_classify_images",
-    "cp_batch_cone_colors",
+    "cp_batch_cone_colors", "cp_batch_track", "cp_track_reset", "cp_debug_track",
 ]
 
 CONE_IMG_ROWS, CONE_IMG_COLS = 15, 12
@@ -39,6 +39,7 @@ CONE_EMPTY, CONE_BAD_INDEX, CONE_BAD_INTENSITY, CONE_AMBIGUOUS, CONE_LOW_CONFIDE
 COLOR_NO_ANSWER = 255   # cp_cone_colors: the service would skip this cone (empty crop) or raise (bad crop)
 
 CLUSTER_DTYPE = np.dtype([("x", np.float32), ("y", np.float32), ("size", np.uint32), ("min_index", np.uint32)])
+TRACKED_CONE_DTYPE = np.dtype([("x", np.float32), ("y", np.float32), ("cluster", np.uint32), ("color", np.uint32)])
 COUNTER_DTYPE = np.dtype([(n, np.uint32) for n in (
     "n_points", "n_ground_kept", "n_cropped", "n_voxels", "n_components", "n_clusters", "key_bits", "passthrough")])
 
@@ -53,6 +54,22 @@ class CColorNet(C.Structure):
     _fields_ = [("c1", C.c_uint32), ("c2", C.c_uint32), ("n_classes", C.c_uint32)] + \
                [(n, C.c_void_p) for n in ("conv1_w", "conv1_b", "conv2_w", "conv2_b", "bn_scale", "bn_shift",
                                           "dense_w", "dense_b")] + [("threshold", C.c_float)]
+
+
+class CTrackParams(C.Structure):
+    """cp_track_params: the ConeDetector members that decide what is published (src/cone_detection.cpp:276-340)."""
+    _fields_ = [("classify_colors", C.c_int32), ("use_points_buffer", C.c_int32),
+                ("cones_matching_dist_theshold", C.c_double), ("cone_position_extension_length", C.c_double),
+                ("cone_width", C.c_float)]
+
+
+def track_params(classify_colors=False, use_points_buffer=False, match=0.5, ext=0.05, cone_width=0.228):
+    return CTrackParams(int(classify_colors), int(use_points_buffer), match, ext, cone_width)
+
+
+class CTrackedCone(C.Structure):
+    """cp_tracked_cone."""
+    _fields_ = [("x", C.c_float), ("y", C.c_float), ("cluster", C.c_uint32), ("color", C.c_uint32)]
 
 
 class ConesGpuError(RuntimeError):
@@ -126,6 +143,10 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.cp_cone_colors.argtypes = [vp, C.POINTER(CCloudView), u32, vp, u32, C.c_float, vp, vp, vp]
     lib.cp_classify_images.argtypes = [vp, vp, u32, vp, vp, vp]
     lib.cp_batch_cone_colors.argtypes = [vp, C.c_float, C.c_double, vp, vp, vp, vp, u64]
+    lib.cp_batch_track.argtypes = [vp, C.POINTER(CTrackParams), vp, u32, vp, vp, u64, C.POINTER(u64)]
+    lib.cp_track_reset.argtypes = [vp]
+    lib.cp_debug_track.argtypes = [vp, C.POINTER(CTrackParams), vp, vp, u32, vp, vp, vp, u32, vp, vp, u64,
+                                   C.POINTER(u64)]
     lib.cp_pinned_alloc.argtypes = [C.c_int32, C.c_size_t, C.c_int32, C.POINTER(vp)]
     lib.cp_pinned_free.argtypes = [vp]
     lib.cp_pinned_free.restype = None
@@ -248,6 +269,7 @@ class ConesGpu:
         cg = to_c_ground(g) if g is not None else None
         self._ck(self.lib.cp_detect(self._h, C.byref(view), C.byref(cd), C.byref(cg) if cg is not None else None,
                                     out.ctypes.data, cap, C.byref(k), ctr.ctypes.data))
+        self.n_frames = 1   # the run is one frame (results(), batch_track())
         return out[:k.value].copy(), ctr[0].copy()
 
     # ---- colour path inputs (SURVEY §8 f3) ----------------------------------------------
@@ -345,6 +367,49 @@ class ConesGpu:
         self._ck(self.lib.cp_batch_cone_colors(self._h, cone_width, extension_length, colors.ctypes.data,
                                                probs.ctypes.data, flags.ctypes.data, counts.ctypes.data, K))
         return colors, probs, flags, counts
+
+    # ---- what the node publishes, over frame sequences ----------------------------------
+    @staticmethod
+    def _seqs(seq_offsets):
+        if seq_offsets is None:
+            return None, 1
+        so = np.ascontiguousarray(seq_offsets, np.uint32)
+        return so, len(so) - 1
+
+    def batch_track(self, params: CTrackParams, seq_offsets=None):
+        """The radial extension, temporal gate / points buffer, colour carry-over and response rules of the
+        cone-detection node (src/cone_detection.cpp:276-340) for every frame of the last run; sequence s continues
+        state slot s.  Returns (cones TRACKED_CONE_DTYPE [n], cloud_offsets u32 [4F + 1]): cloud c of frame f is
+        cones[cloud_offsets[4f + c]:cloud_offsets[4f + c + 1]]."""
+        total = C.c_uint64()
+        self._ck(self.lib.cp_batch_results(self._h, None, None, None, 0, C.byref(total)))
+        so, n_seqs = self._seqs(seq_offsets)
+        out = np.zeros(total.value, TRACKED_CONE_DTYPE)
+        coff = np.zeros(4 * self.n_frames + 1, np.uint32)
+        n = C.c_uint64()
+        self._ck(self.lib.cp_batch_track(self._h, C.byref(params), so.ctypes.data if so is not None else None, n_seqs,
+                                         out.ctypes.data, coff.ctypes.data, len(out), C.byref(n)))
+        return out[:n.value].copy(), coff
+
+    def track_reset(self):
+        """Clears every state slot: each behaves like a node that has just started."""
+        self._ck(self.lib.cp_track_reset(self._h))
+
+    def debug_track(self, params: CTrackParams, records, record_offsets, colors=None, flags=None, seq_offsets=None):
+        """cp_batch_track's kernels on caller-supplied records (CLUSTER_DTYPE) and per-record service answers."""
+        rec = np.ascontiguousarray(records, CLUSTER_DTYPE)
+        roff = np.ascontiguousarray(record_offsets, np.uint32)
+        F = len(roff) - 1
+        col = np.ascontiguousarray(colors if colors is not None else np.zeros(len(rec)), np.uint8)
+        fl = np.ascontiguousarray(flags if flags is not None else np.zeros(len(rec)), np.uint32)
+        so, n_seqs = self._seqs(seq_offsets)
+        out = np.zeros(len(rec), TRACKED_CONE_DTYPE)
+        coff = np.zeros(4 * F + 1, np.uint32)
+        n = C.c_uint64()
+        self._ck(self.lib.cp_debug_track(self._h, C.byref(params), rec.ctypes.data, roff.ctypes.data, F,
+                                         col.ctypes.data, fl.ctypes.data, so.ctypes.data if so is not None else None,
+                                         n_seqs, out.ctypes.data, coff.ctypes.data, len(out), C.byref(n)))
+        return out[:n.value].copy(), coff
 
     # ---- batches ----------------------------------------------------------------------
     def set_device_input(self, d_ptr: int, frame_points, point_step: int = 16, off=(0, 4, 8, 12), keep=None):

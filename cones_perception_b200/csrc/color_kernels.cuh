@@ -152,6 +152,22 @@ __host__ __device__ inline void box_bounds(float c, double hw, float* lo, float*
   *hi = fhi;
 }
 
+// src/cone_detection.cpp:276-278, the centroid moved radially by ext: vector_len = euclidan_dist(p.x, p.y, 0) in
+// double, narrowed; p.x / len in float; the sum promotes to double.  On the device explicit _rn intrinsics: no FMA
+// contraction.  A centroid at the origin gives NaN, as in the reference.
+__host__ __device__ inline void extend_center(float x, float y, double ext, float* ex, float* ey) {
+#ifdef __CUDA_ARCH__
+  const double s = __dadd_rn(__dmul_rn((double)x, (double)x), __dmul_rn((double)y, (double)y));
+  const float len = __double2float_rn(__dsqrt_rn(s));
+  *ex = __double2float_rn(__dadd_rn((double)x, __dmul_rn((double)__fdiv_rn(x, len), ext)));
+  *ey = __double2float_rn(__dadd_rn((double)y, __dmul_rn((double)__fdiv_rn(y, len), ext)));
+#else
+  const float len = (float)sqrt((double)x * (double)x + (double)y * (double)y);
+  *ex = (float)((double)x + (double)(x / len) * ext);
+  *ey = (float)((double)y + (double)(y / len) * ext);
+#endif
+}
+
 // ---- every cluster of a batch run (cp_batch_cone_colors) ---------------------------------
 //   batch_box_kernel     extended centre (src/cone_detection.cpp:276-278) + box bounds + frame of each cluster
 //   batch_mark_kernel    one pass over the raw batch: a (cluster, frame row, ballot) triple for every non-empty
@@ -178,13 +194,8 @@ __global__ void __launch_bounds__(256) batch_box_kernel(const ClusterRec* __rest
     const u32 mid = (lo + hi) >> 1;
     if (k_off[mid] <= k) lo = mid; else hi = mid;
   }
-  // vector_len = euclidan_dist(p.x, p.y, 0) in double, narrowed; p.x / len in float; the sum promotes to double.
-  // Explicit _rn intrinsics: no FMA contraction.
-  const float x = cl[k].x, y = cl[k].y;
-  const double s = __dadd_rn(__dmul_rn((double)x, (double)x), __dmul_rn((double)y, (double)y));
-  const float len = __double2float_rn(__dsqrt_rn(s));
-  const float ex = __double2float_rn(__dadd_rn((double)x, __dmul_rn((double)__fdiv_rn(x, len), ext)));
-  const float ey = __double2float_rn(__dadd_rn((double)y, __dmul_rn((double)__fdiv_rn(y, len), ext)));
+  float ex, ey;
+  extend_center(cl[k].x, cl[k].y, ext, &ex, &ey);
   float4 b;
   box_bounds(ex, hw, &b.x, &b.y);
   box_bounds(ey, hw, &b.z, &b.w);

@@ -25,6 +25,7 @@
 #include "single_frame.cuh"
 #include "stream_kernels.cuh"
 #include "tflite_reader.hpp"
+#include "track_kernels.cuh"
 #include "voxel_kernels.cuh"
 
 using namespace cp;
@@ -144,6 +145,25 @@ struct cp_handle {
     size_t box_n = 0, kframe_n = 0, cnt_n = 0, tcnt_n = 0, toff_n = 0, bctl_n = 0;
     size_t keys_a_n = 0, keys_b_n = 0, vals_a_n = 0, vals_b_n = 0, sort_hdr_n = 0, sort_state_n = 0;
   } color;
+  // frame sequences (cp_batch_track, track_kernels.cuh): the slot state is double-buffered (the call writes the other
+  // buffer and the host swaps only when the call succeeds); scratch is grown on demand
+  struct TrackBufs {
+    TrackCone* st[2] = {nullptr, nullptr};
+    size_t st_n[2] = {0, 0};
+    int cur = 0;
+    std::vector<u32> st_off, st_prev;  // layout of st[cur]: slot s = [st_off[s], st_off[s+1]); st_prev[s]: seen a frame
+    std::vector<u32> par, coff;        // per-call parameter block (one upload), cloud offsets read back
+    u32 *par_d = nullptr, *kframe = nullptr, *bits = nullptr, *rank = nullptr, *cnt = nullptr, *coff_d = nullptr;
+    float2* ext = nullptr;
+    uint8_t *info = nullptr, *fcol = nullptr, *ans = nullptr;
+    TrackCone* out = nullptr;
+    ClusterRec* rec = nullptr;  // cp_debug_track inputs
+    u32 *rec_off = nullptr, *flags = nullptr;
+    uint8_t* colors = nullptr;
+    size_t par_n = 0, kframe_n = 0, bits_n = 0, rank_n = 0, cnt_n = 0, coff_n = 0, ext_n = 0, info_n = 0, fcol_n = 0,
+           ans_n = 0, out_n = 0, rec_n = 0, rec_off_n = 0, flags_n = 0, colors_n = 0;
+  } track;
+  bool tracked = false;  // the current run's frames have advanced the slot state
   const uint8_t* in_ptr = nullptr;  // current batch input (d_in or caller memory)
   Layout layout{};
   HostGeom hg;
@@ -1871,6 +1891,11 @@ void cp_destroy(cp_handle* h) {
                   (void*)h->color.vals_b, (void*)h->color.sort_hdr, (void*)h->color.sort_state})
     if (q) cudaFree(q);
   if (h->color.pin) cudaFreeHost(h->color.pin);
+  const cp_handle::TrackBufs& tb = h->track;
+  for (void* q : {(void*)tb.st[0], (void*)tb.st[1], (void*)tb.par_d, (void*)tb.kframe, (void*)tb.bits, (void*)tb.rank,
+                  (void*)tb.cnt, (void*)tb.coff_d, (void*)tb.ext, (void*)tb.info, (void*)tb.fcol, (void*)tb.ans,
+                  (void*)tb.out, (void*)tb.rec, (void*)tb.rec_off, (void*)tb.flags, (void*)tb.colors})
+    if (q) cudaFree(q);
   if (h->graph_exec) cudaGraphExecDestroy(h->graph_exec);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
@@ -2043,6 +2068,7 @@ static RunKey make_key(const cp_handle* h, const cp_detect_params* d, const cp_g
 
 cp_status cp_batch_run(cp_handle* h, const cp_detect_params* d, const cp_ground_params* ground) try {
   if (!h) return CP_E_PARAM;
+  h->tracked = false;
   CK(cudaSetDevice(h->cfg.device));
   const bool eligible = h->use_graph && d && h->batch_ready && !h->taps && !h->stage_timing && h->hg.uniform_n != 0;
   if (!eligible) {
@@ -2907,36 +2933,14 @@ cp_status cp_cone_colors(cp_handle* h, const cp_cloud_view* cloud, uint32_t fram
   return abi_exception(h);
 }
 
-cp_status cp_batch_cone_colors(cp_handle* h, float cone_width, double extension_length, uint8_t* colors, float* probs,
-                               uint32_t* flags, uint32_t* counts, uint64_t cap) try {
-  if (!h) return CP_E_PARAM;
-  if (!std::isfinite(extension_length) || !std::isfinite(cone_width) || !(cone_width > 0.0f)) {
-    h->err = "extension_length must be finite, cone_width positive and finite";
-    return CP_E_PARAM;
-  }
-  if (!h->ran) {
-    h->err = "no run on the staged input (cp_batch_run / cp_detect_batch / cp_detect), or input staged since";
-    return CP_E_STATE;
-  }
-  if (!h->color.net_loaded) {
-    h->err = "no colour net loaded (cp_color_net_load / cp_color_net_load_tflite)";
-    return CP_E_STATE;
-  }
-  cp_status st = cp_sync(h);  // the final records: cp_sync may re-run the back half
-  if (st) return st;
-  const u64 K64 = h->h_ctl->n_clusters;
-  if (K64 > cap) {
-    h->err = "colour outputs hold fewer entries than the run has clusters";
-    return CP_E_CAPACITY;
-  }
-  if (K64 && !colors) {
-    h->err = "NULL colors";
-    return CP_E_PARAM;
-  }
-  h->launches = 0;
-  if (K64 == 0) return CP_OK;
-  const u32 K = (u32)K64;
+// The colour chain of cp_batch_cone_colors over the K > 0 records of the run.  Colours stay in cb.colors, flags in
+// cb.net_flags, and the crop offsets come back to pin_off.  With colors NULL nothing else is copied back
+// (cp_batch_track reads the per-cluster answers on the device).
+static cp_status batch_colors(cp_handle* h, float cone_width, double extension_length, u32 K, uint8_t* colors,
+                              float* probs, uint32_t* flags) {
+  cp_status st;
   u32 max_rows = 0;
+
   for (u32 n : h->hg.frame_n) max_rows = std::max(max_rows, (n + 31) / 32);
   const u32 row_bits = ceil_log2_host(max_rows);
   const u32 key_bits = ceil_log2_host(K) + row_bits;
@@ -2971,7 +2975,11 @@ cp_status cp_batch_cone_colors(cp_handle* h, float cone_width, double extension_
     h->launches += 1;
     if ((st = enqueue_color_net(h, cb.img, cb.flags, K))) return st;
     CK(cudaMemcpyAsync(pin_off(h), cb.off, sizeof(u32) * ((size_t)K + 1), cudaMemcpyDeviceToHost, h->stream));
-    if ((st = fetch_colors(h, K, colors, probs, nullptr, flags))) return st;
+    if (colors) {
+      if ((st = fetch_colors(h, K, colors, probs, nullptr, flags))) return st;
+    } else {
+      CK(cudaStreamSynchronize(h->stream));
+    }
     // every triple holds at least one crop point: crops that fit mean the triples fitted too
     const u32 total = pin_off(h)[K];
     if (total <= cb.pts_n) break;
@@ -2981,9 +2989,260 @@ cp_status cp_batch_cone_colors(cp_handle* h, float cone_width, double extension_
     }
     want = total;
   }
+  return CP_OK;
+}
+
+cp_status cp_batch_cone_colors(cp_handle* h, float cone_width, double extension_length, uint8_t* colors, float* probs,
+                               uint32_t* flags, uint32_t* counts, uint64_t cap) try {
+  if (!h) return CP_E_PARAM;
+  if (!std::isfinite(extension_length) || !std::isfinite(cone_width) || !(cone_width > 0.0f)) {
+    h->err = "extension_length must be finite, cone_width positive and finite";
+    return CP_E_PARAM;
+  }
+  if (!h->ran) {
+    h->err = "no run on the staged input (cp_batch_run / cp_detect_batch / cp_detect), or input staged since";
+    return CP_E_STATE;
+  }
+  if (!h->color.net_loaded) {
+    h->err = "no colour net loaded (cp_color_net_load / cp_color_net_load_tflite)";
+    return CP_E_STATE;
+  }
+  cp_status st = cp_sync(h);  // the final records: cp_sync may re-run the back half
+  if (st) return st;
+  const u64 K64 = h->h_ctl->n_clusters;
+  if (K64 > cap) {
+    h->err = "colour outputs hold fewer entries than the run has clusters";
+    return CP_E_CAPACITY;
+  }
+  if (K64 && !colors) {
+    h->err = "NULL colors";
+    return CP_E_PARAM;
+  }
+  h->launches = 0;
+  if (K64 == 0) return CP_OK;
+  const u32 K = (u32)K64;
+  if ((st = batch_colors(h, cone_width, extension_length, K, colors, probs, flags))) return st;
   if (counts)
     for (u32 k = 0; k < K; ++k) counts[k] = pin_off(h)[k + 1] - pin_off(h)[k];
   return CP_OK;
+} catch (...) {
+  return abi_exception(h);
+}
+
+// ---- frame sequences (cp_batch_track, track_kernels.cuh) ----------------------------------------------
+static_assert(sizeof(cp_tracked_cone) == sizeof(TrackCone), "cp_tracked_cone is TrackCone");
+static_assert(sizeof(cp_cluster) == sizeof(ClusterRec), "cp_cluster is ClusterRec");
+
+static cp_status track_check(cp_handle* h, const cp_track_params* t, const uint32_t* seq_offsets, uint32_t n_seqs,
+                             u32 n_frames, const uint32_t* cloud_offsets, const uint64_t* n_out) {
+  if (!t || !cloud_offsets || !n_out) {
+    h->err = "NULL params, cloud_offsets or n_out";
+    return CP_E_PARAM;
+  }
+  if (!std::isfinite(t->cones_matching_dist_theshold) || !std::isfinite(t->cone_position_extension_length) ||
+      (t->classify_colors && !(std::isfinite(t->cone_width) && t->cone_width > 0.0f))) {
+    h->err = "cones_matching_dist_theshold and cone_position_extension_length must be finite, cone_width positive "
+             "and finite when classifying colours";
+    return CP_E_PARAM;
+  }
+  if (n_seqs == 0 || n_seqs > h->cfg.max_frames || (!seq_offsets && n_seqs != 1)) {
+    h->err = "n_seqs must be in [1, max_frames] (1 when seq_offsets is NULL)";
+    return CP_E_PARAM;
+  }
+  if (seq_offsets) {
+    bool ok = seq_offsets[0] == 0 && seq_offsets[n_seqs] == n_frames;
+    for (u32 s = 0; ok && s < n_seqs; ++s) ok = seq_offsets[s] <= seq_offsets[s + 1];
+    if (!ok) {
+      h->err = "seq_offsets must be a non-decreasing partition of [0, n_frames]";
+      return CP_E_PARAM;
+    }
+  }
+  return CP_OK;
+}
+
+// The tracking kernels over K = k_off[F] records (rec, k_off_d on the device; k_off on the host) and, in colour mode,
+// the per-record answers colors_d / flags_d of the service.  The new slot state goes to the other state buffer; the
+// handle switches to it only when everything succeeded.
+static cp_status track_run(cp_handle* h, const cp_track_params* t, const ClusterRec* rec, const u32* k_off_d,
+                           const u32* k_off, u32 F, const uint8_t* colors_d, const u32* flags_d,
+                           const uint32_t* seq_offsets, uint32_t n_seqs, cp_tracked_cone* out, uint32_t* cloud_offsets,
+                           uint64_t cap, uint64_t* n_out) {
+  cp_handle::TrackBufs& tb = h->track;
+  const u32 M = h->cfg.max_frames, K = k_off[F];
+  const bool classify = t->classify_colors != 0;
+  if (tb.st_off.empty()) {
+    tb.st_off.assign((size_t)M + 1, 0u);
+    tb.st_prev.assign(M, 0u);
+  }
+  // parameter block: fslot[F] mbase[F+1] seq[n_seqs+1] new_off[M+1] new_src[M] old_off[M+1] old_prev[M]
+  const size_t o_fslot = 0, o_mbase = o_fslot + F, o_seq = o_mbase + F + 1, o_noff = o_seq + n_seqs + 1,
+               o_nsrc = o_noff + M + 1, o_ooff = o_nsrc + M, o_oprev = o_ooff + M + 1, n_par = o_oprev + M;
+  std::vector<u32>& par = tb.par;
+  par.assign(n_par, 0u);
+  u32* so = par.data() + o_seq;
+  for (u32 s = 0; s <= n_seqs; ++s) so[s] = seq_offsets ? seq_offsets[s] : (s ? F : 0u);
+  for (u32 f = 0; f < F; ++f) par[o_fslot + f] = kTrackNoIndex;
+  for (u32 s = 0; s < n_seqs; ++s)
+    if (so[s] < so[s + 1]) par[o_fslot + so[s]] = s;
+  u64 words = 0;  // match bit sets: every record of a later frame holds one bit per record of the frame before
+  for (u32 f = 0; f < F; ++f) {
+    par[o_mbase + f] = (u32)words;
+    if (classify && par[o_fslot + f] == kTrackNoIndex)
+      words += (u64)(k_off[f + 1] - k_off[f]) * ((k_off[f] - k_off[f - 1] + 31) / 32);
+    if (words > 0xFFFFFFFFull) {
+      h->err = "match sets of consecutive frames exceed 2^32 words";
+      return CP_E_NOMEM;
+    }
+  }
+  par[o_mbase + F] = (u32)words;
+  std::vector<u32> new_prev(tb.st_prev);
+  u64 total = 0;
+  for (u32 s = 0; s < M; ++s) {
+    const bool touched = s < n_seqs && so[s] < so[s + 1];
+    const u32 last = touched ? so[s + 1] - 1 : 0u;
+    par[o_noff + s] = (u32)total;
+    par[o_nsrc + s] = touched ? last : kTrackNoIndex;
+    total += touched ? k_off[last + 1] - k_off[last] : tb.st_off[s + 1] - tb.st_off[s];
+    if (touched) new_prev[s] = 1u;
+    if (total > 0xFFFFFFFFull) {
+      h->err = "slot state exceeds 2^32 cones";
+      return CP_E_NOMEM;
+    }
+  }
+  par[o_noff + M] = (u32)total;
+  std::copy(tb.st_off.begin(), tb.st_off.end(), par.begin() + o_ooff);
+  std::copy(tb.st_prev.begin(), tb.st_prev.end(), par.begin() + o_oprev);
+  const int nxt = 1 - tb.cur;
+  cp_status st;
+  if ((st = grow(h, &tb.par_d, &tb.par_n, n_par))) return st;
+  if ((st = grow(h, &tb.ext, &tb.ext_n, K))) return st;
+  if ((st = grow(h, &tb.kframe, &tb.kframe_n, K))) return st;
+  if ((st = grow(h, &tb.info, &tb.info_n, K))) return st;
+  if ((st = grow(h, &tb.fcol, &tb.fcol_n, K))) return st;
+  if ((st = grow(h, &tb.ans, &tb.ans_n, K))) return st;
+  if ((st = grow(h, &tb.rank, &tb.rank_n, K))) return st;
+  if ((st = grow(h, &tb.out, &tb.out_n, K))) return st;
+  if ((st = grow(h, &tb.bits, &tb.bits_n, words))) return st;
+  if ((st = grow(h, &tb.cnt, &tb.cnt_n, 4 * (size_t)F))) return st;
+  if ((st = grow(h, &tb.coff_d, &tb.coff_n, 4 * (size_t)F + 1))) return st;
+  if ((st = grow(h, &tb.st[tb.cur], &tb.st_n[tb.cur], 1))) return st;
+  if ((st = grow(h, &tb.st[nxt], &tb.st_n[nxt], total))) return st;
+  CK(cudaMemcpyAsync(tb.par_d, par.data(), sizeof(u32) * n_par, cudaMemcpyHostToDevice, h->stream));
+  const u32* pd = tb.par_d;
+  const u32 grid = std::max<u32>(1, std::min<u32>((K + 255) / 256, (u32)h->sms * 8));
+  track_ext_kernel<<<grid, 256, 0, h->stream>>>(rec, k_off_d, F, K, t->cone_position_extension_length, tb.ext,
+                                                tb.kframe);
+  track_match_kernel<<<grid, 256, 0, h->stream>>>(tb.ext, tb.kframe, k_off_d, K, pd + o_fslot, pd + o_mbase,
+                                                  tb.st[tb.cur], pd + o_ooff, pd + o_oprev,
+                                                  t->cones_matching_dist_theshold, t->use_points_buffer ? 1u : 0u,
+                                                  classify ? 1u : 0u, tb.info, tb.bits);
+  track_route_kernel<<<(n_seqs + 7) / 8, 256, 0, h->stream>>>(n_seqs, pd + o_seq, k_off_d, pd + o_mbase, tb.info,
+                                                              tb.bits, classify ? 1u : 0u, colors_d, flags_d, tb.fcol,
+                                                              tb.rank, tb.ans, tb.cnt);
+  track_scan_kernel<<<1, kTrackScanThreads, 0, h->stream>>>(4 * F, tb.cnt, tb.coff_d);
+  const u32 egrid = std::max<u32>(1, std::min<u64>((std::max<u64>(K, total) + 255) / 256, (u64)h->sms * 8));
+  track_emit_kernel<<<egrid, 256, 0, h->stream>>>(K, tb.ext, tb.kframe, k_off_d, tb.fcol, tb.rank, tb.coff_d,
+                                                  tb.out, M, (u32)total, pd + o_noff, pd + o_nsrc, pd + o_ooff,
+                                                  tb.st[tb.cur], tb.st[nxt]);
+  CK(cudaGetLastError());
+  h->launches += 5;
+  tb.coff.resize(4 * (size_t)F + 1);
+  CK(cudaMemcpyAsync(tb.coff.data(), tb.coff_d, sizeof(u32) * tb.coff.size(), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaStreamSynchronize(h->stream));
+  const u32 n = tb.coff[4 * (size_t)F];
+  *n_out = n;
+  if (n > cap) {
+    h->err = "the published cones do not fit the output (cap < n_out)";
+    return CP_E_CAPACITY;
+  }
+  if (n && !out) {
+    h->err = "NULL out";
+    return CP_E_PARAM;
+  }
+  if (n) {
+    CK(cudaMemcpyAsync(out, tb.out, sizeof(TrackCone) * n, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+  }
+  memcpy(cloud_offsets, tb.coff.data(), sizeof(u32) * tb.coff.size());
+  tb.cur = nxt;
+  tb.st_off.assign(par.begin() + o_noff, par.begin() + o_noff + M + 1);
+  tb.st_prev.swap(new_prev);
+  return CP_OK;
+}
+
+cp_status cp_batch_track(cp_handle* h, const cp_track_params* t, const uint32_t* seq_offsets, uint32_t n_seqs,
+                         cp_tracked_cone* out, uint32_t* cloud_offsets, uint64_t cap, uint64_t* n_out) try {
+  if (!h) return CP_E_PARAM;
+  cp_status st = track_check(h, t, seq_offsets, n_seqs, h->ran ? h->hg.n_frames : 0u, cloud_offsets, n_out);
+  if (st) return st;
+  if (!h->ran) {
+    h->err = "no run on the staged input (cp_batch_run / cp_detect_batch / cp_detect), or input staged since";
+    return CP_E_STATE;
+  }
+  if (t->classify_colors && !h->color.net_loaded) {
+    h->err = "no colour net loaded (cp_color_net_load / cp_color_net_load_tflite)";
+    return CP_E_STATE;
+  }
+  CK(cudaSetDevice(h->cfg.device));
+  if ((st = cp_sync(h))) return st;  // the final records: cp_sync may re-run the back half
+  if (h->tracked) {
+    h->err = "this run's frames have already advanced the slot state (run again to track new frames)";
+    return CP_E_STATE;
+  }
+  const u32 F = h->hg.n_frames;
+  const u32* k_off = h->h_result;
+  const u32 K = k_off[F];
+  h->launches = 0;
+  if (t->classify_colors && K)
+    if ((st = batch_colors(h, t->cone_width, t->cone_position_extension_length, K, nullptr, nullptr, nullptr)))
+      return st;
+  st = track_run(h, t, h->d_clusters, h->d_k_off, k_off, F, h->color.colors, h->color.net_flags, seq_offsets, n_seqs,
+                 out, cloud_offsets, cap, n_out);
+  if (st == CP_OK) h->tracked = true;
+  return st;
+} catch (...) {
+  return abi_exception(h);
+}
+
+cp_status cp_track_reset(cp_handle* h) try {
+  if (!h) return CP_E_PARAM;
+  h->track.st_off.assign((size_t)h->cfg.max_frames + 1, 0u);
+  h->track.st_prev.assign(h->cfg.max_frames, 0u);
+  return CP_OK;
+} catch (...) {
+  return abi_exception(h);
+}
+
+cp_status cp_debug_track(cp_handle* h, const cp_track_params* t, const cp_cluster* records,
+                         const uint32_t* record_offsets, uint32_t n_frames, const uint8_t* colors,
+                         const uint32_t* flags, const uint32_t* seq_offsets, uint32_t n_seqs, cp_tracked_cone* out,
+                         uint32_t* cloud_offsets, uint64_t cap, uint64_t* n_out) try {
+  if (!h) return CP_E_PARAM;
+  cp_status st = track_check(h, t, seq_offsets, n_seqs, n_frames, cloud_offsets, n_out);
+  if (st) return st;
+  bool ok = record_offsets && record_offsets[0] == 0;
+  for (u32 f = 0; ok && f < n_frames; ++f) ok = record_offsets[f] <= record_offsets[f + 1];
+  const u32 K = ok ? record_offsets[n_frames] : 0u;
+  if (!ok || (K && !records) || (t->classify_colors && K && (!colors || !flags))) {
+    h->err = "record_offsets must be a non-decreasing partition starting at 0; records, colors and flags non-NULL";
+    return CP_E_PARAM;
+  }
+  CK(cudaSetDevice(h->cfg.device));
+  cp_handle::TrackBufs& tb = h->track;
+  if ((st = grow(h, &tb.rec, &tb.rec_n, K))) return st;
+  if ((st = grow(h, &tb.rec_off, &tb.rec_off_n, (size_t)n_frames + 1))) return st;
+  if ((st = grow(h, &tb.colors, &tb.colors_n, K))) return st;
+  if ((st = grow(h, &tb.flags, &tb.flags_n, K))) return st;
+  CK(cudaMemcpyAsync(tb.rec_off, record_offsets, sizeof(u32) * ((size_t)n_frames + 1), cudaMemcpyHostToDevice,
+                     h->stream));
+  if (K) CK(cudaMemcpyAsync(tb.rec, records, sizeof(cp_cluster) * K, cudaMemcpyHostToDevice, h->stream));
+  if (K && t->classify_colors) {
+    CK(cudaMemcpyAsync(tb.colors, colors, K, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(tb.flags, flags, sizeof(u32) * K, cudaMemcpyHostToDevice, h->stream));
+  }
+  h->launches = 0;
+  return track_run(h, t, tb.rec, tb.rec_off, record_offsets, n_frames, tb.colors, tb.flags, seq_offsets, n_seqs, out,
+                   cloud_offsets, cap, n_out);
 } catch (...) {
   return abi_exception(h);
 }

@@ -71,6 +71,53 @@ int ch_tracker_update(void* tp, const float* xy, uint32_t n, int forced_color, f
   return 0;
 }
 
+// colour mode with per-record service answers (cp_batch_cone_colors output for this frame's n records): the need list
+// is mapped back to records by the exact bits of their extended centres, then the response rules of
+// ConeDetector::gpu_colors apply (a bad crop: no answer at all; empty crops skipped)
+int ch_tracker_update_answers(void* tp, const float* xy, uint32_t n, const uint8_t* colors, const uint32_t* flags,
+                              float* out_xy, uint32_t* counts, uint32_t cap) {
+  auto* t = static_cast<ConeTracker*>(tp);
+  std::vector<std::pair<float, float>> c(n);
+  std::map<std::pair<uint32_t, uint32_t>, uint32_t> index;
+  for (uint32_t i = 0; i < n; ++i) {
+    c[i] = {xy[2 * i], xy[2 * i + 1]};
+    Point p;
+    p.x = c[i].first;
+    p.y = c[i].second;
+    float vector_len = euclidan_dist(p.x, p.y, p.z, 0, 0, 0);  // as ConeTracker::update
+    p.x = p.x + p.x / vector_len * t->cone_position_extension_length;
+    p.y = p.y + p.y / vector_len * t->cone_position_extension_length;
+    uint32_t bx, by;
+    std::memcpy(&bx, &p.x, 4);
+    std::memcpy(&by, &p.y, 4);
+    index.emplace(std::make_pair(bx, by), i);
+  }
+  t->classify_centers = [&](const std::vector<Point>& need) {
+    std::vector<Color> out;
+    for (const Point& p : need) {
+      uint32_t bx, by;
+      std::memcpy(&bx, &p.x, 4);
+      std::memcpy(&by, &p.y, 4);
+      const uint32_t k = index.at({bx, by});
+      if (flags[k] & (CP_CONE_BAD_INDEX | CP_CONE_BAD_INTENSITY)) return std::vector<Color>();
+      if (flags[k] & CP_CONE_EMPTY) continue;
+      out.push_back(static_cast<Color>(colors[k] < kNumberOfColors ? colors[k] : 0));
+    }
+    return out;
+  };
+  auto clouds = t->update(c, nullptr);
+  t->classify_centers = nullptr;
+  for (int k = 0; k < kNumberOfColors; ++k) {
+    counts[k] = static_cast<uint32_t>(clouds[k].size());
+    if (clouds[k].size() > cap) return 3;
+    for (size_t i = 0; i < clouds[k].size(); ++i) {
+      out_xy[(static_cast<size_t>(k) * cap + i) * 2] = clouds[k][i].x;
+      out_xy[(static_cast<size_t>(k) * cap + i) * 2 + 1] = clouds[k][i].y;
+    }
+  }
+  return 0;
+}
+
 // ---- ConeDetector / GroundRemover (GPU) -----------------------------------------------------
 }  // extern "C"
 namespace {
@@ -143,10 +190,12 @@ void ch_detector_color_probe(void* dp, uint64_t* n_inputs, uint64_t* n_points, u
   *digest = pr.digest;
 }
 
-void* ch_detector_create(uint64_t max_points, int device, const cp_detect_params* d, int classify_colors,
-                         int use_points_buffer, int fused_ground) {
+}  // extern "C"
+namespace {
+void* create_detector(uint64_t max_points, uint32_t max_frames, int device, const cp_detect_params* d,
+                      int classify_colors, int use_points_buffer, int fused_ground) {
   try {
-    auto* det = new ConeDetector(max_points, device, 32);
+    auto* det = new ConeDetector(max_points, device, 32, max_frames);
     det->distance_treshold_max = d->distance_treshold_max;
     det->distance_treshold_min = d->distance_treshold_min;
     det->level_threshold = d->level_threshold;
@@ -164,6 +213,13 @@ void* ch_detector_create(uint64_t max_points, int device, const cp_detect_params
     g_err = e.what();
     return nullptr;
   }
+}
+}  // namespace
+extern "C" {
+
+void* ch_detector_create(uint64_t max_points, int device, const cp_detect_params* d, int classify_colors,
+                         int use_points_buffer, int fused_ground) {
+  return create_detector(max_points, 1, device, d, classify_colors, use_points_buffer, fused_ground);
 }
 void ch_detector_destroy(void* d) {
   g_probes.erase(d);
@@ -192,6 +248,53 @@ int ch_detector_handle(void* dp, const float* xyzi, uint32_t n, int with_intensi
     *out_point_step = clouds[0].point_step;
     *out_n_fields = static_cast<uint32_t>(clouds[0].fields.size());
     *out_stamp_nsec = clouds[0].header.stamp_nsec;
+    return 0;
+  } catch (const std::exception& e) {
+    g_err = e.what();
+    return 4;
+  }
+}
+
+// ConeDetector::replay: messages 0..n_msgs-1 (compact xyzi, frame_n[i] points each) in device batches of up to
+// max_frames.  ch_detector_publish: the same messages through replay (replay != 0) or through cloud_handler, one call
+// per message; out receives every published message serialised (header, layout, fields, data), 4 per input message.
+void* ch_detector_create_replay(uint64_t max_points, uint32_t max_frames, int device, const cp_detect_params* d,
+                                int classify_colors, int use_points_buffer, int fused_ground) {
+  return create_detector(max_points, max_frames, device, d, classify_colors, use_points_buffer, fused_ground);
+}
+
+int ch_detector_publish(void* dp, const float* xyzi, const uint32_t* frame_n, uint32_t n_msgs, int with_intensity_field,
+                        int replay, uint8_t* out, uint64_t cap, uint64_t* used) {
+  try {
+    auto* det = static_cast<ConeDetector*>(dp);
+    std::vector<PointCloud2> msgs;
+    size_t at = 0;
+    for (uint32_t i = 0; i < n_msgs; ++i) {
+      msgs.push_back(make_msg(xyzi + 4 * at, frame_n[i], with_intensity_field, 100 + i, 123456789 + i));
+      at += frame_n[i];
+    }
+    std::vector<std::vector<PointCloud2>> pub;
+    if (replay) {
+      pub = det->replay(msgs);
+    } else {
+      for (const PointCloud2& m : msgs) pub.push_back(det->cloud_handler(m));
+    }
+    std::vector<uint8_t> b;
+    auto put = [&b](const void* p, size_t n) { b.insert(b.end(), static_cast<const uint8_t*>(p), static_cast<const uint8_t*>(p) + n); };
+    for (const auto& clouds : pub)
+      for (const PointCloud2& m : clouds) {
+        put(&m.header.seq, 4); put(&m.header.stamp_sec, 4); put(&m.header.stamp_nsec, 4);
+        put(m.header.frame_id.data(), m.header.frame_id.size());
+        put(&m.height, 4); put(&m.width, 4);
+        for (const PointField& f : m.fields) {
+          put(f.name.data(), f.name.size()); put(&f.offset, 4); put(&f.datatype, 1); put(&f.count, 4);
+        }
+        put(&m.is_bigendian, 1); put(&m.point_step, 4); put(&m.row_step, 4);
+        put(m.data.data(), m.data.size()); put(&m.is_dense, 1);
+      }
+    *used = b.size();
+    if (b.size() > cap) return 3;
+    if (!b.empty()) std::memcpy(out, b.data(), b.size());
     return 0;
   } catch (const std::exception& e) {
     g_err = e.what();

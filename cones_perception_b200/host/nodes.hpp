@@ -246,14 +246,18 @@ class ConeDetector {
   std::function<std::vector<Color>(const std::vector<uint8_t>& images, const std::vector<uint32_t>& flags)>
       get_colors_from_images;
 
-  explicit ConeDetector(uint64_t max_points = 4u << 20, int device = 0, uint32_t max_point_step = 64) {
+  // max_frames > 1 only matters for replay(): messages per device batch (max_points bounds their points)
+  explicit ConeDetector(uint64_t max_points = 4u << 20, int device = 0, uint32_t max_point_step = 64,
+                        uint32_t max_frames = 1) {
     cp_config cfg{};
     cfg.device = device;
     cfg.max_points = max_points;
-    cfg.max_frames = 1;
+    cfg.max_frames = max_frames;
     cfg.max_point_step = max_point_step;
     cp_status st = cp_create(&gpu_, &cfg);
     if (st != CP_OK) throw GpuError(st, cp_create_error());
+    max_points_ = max_points;
+    max_frames_ = max_frames;
   }
   ~ConeDetector() { cp_destroy(gpu_); }
   // Loads the classifier the reference's service reads from its ~model_path parameter (a .tflite file,
@@ -279,6 +283,7 @@ class ConeDetector {
   // src/cone_detection.cpp:130-187; returns the four clouds the node publishes
   // (cones_cloud_unknowns, _yellows, _blues, _oranges)
   std::vector<PointCloud2> cloud_handler(const PointCloud2& cloud_msg) {
+    use_entry(kPerMessage);
     if (!intensity_in_cloud_checked_) {  // :131-136
       if (!cones_host::intensity_in_cloud(cloud_msg)) intensity_in_cloud_ = false;
       intensity_in_cloud_checked_ = true;
@@ -324,6 +329,36 @@ class ConeDetector {
       out[i] = to_msg(clouds[i]);
       out[i].header = cloud_msg.header;
       out[i].fields = cloud_msg.fields;  // Q6: the input's field list over 32-byte PCL points
+    }
+    return out;
+  }
+
+  // cloud_handler for a series of consecutive messages to this node, in device batches of up to max_frames messages:
+  // cp_detect_batch, then cp_batch_track continues the node's state on the device (the gate, the colour carry-over
+  // and the publish order of ConeTracker::update).  Returns, per message, the four clouds cloud_handler would publish.
+  // Colours: classify_colors = false, or the device net (load_color_model); the external-service colour modes
+  // stay on cloud_handler.  One object serves either cloud_handler or replay: the state of one is not the other's.
+  std::vector<std::vector<PointCloud2>> replay(const std::vector<PointCloud2>& msgs) {
+    use_entry(kReplay);
+    if (classify_colors && color_inputs != kGpuColors)
+      throw GpuError(CP_E_PARAM, "replay classifies colours with the device net only (load_color_model)");
+    std::vector<std::vector<PointCloud2>> out;
+    out.reserve(msgs.size());
+    size_t i = 0;
+    while (i < msgs.size()) {
+      if (!intensity_in_cloud_checked_) {  // :131-136
+        if (!cones_host::intensity_in_cloud(msgs[i])) intensity_in_cloud_ = false;
+        intensity_in_cloud_checked_ = true;
+      }
+      std::vector<cp_cloud_view> views;
+      uint64_t pts = 0;
+      for (; i < msgs.size() && views.size() < max_frames_; ++i) {
+        const uint64_t n = static_cast<uint64_t>(msgs[i].width) * msgs[i].height;
+        if (!views.empty() && pts + n > max_points_) break;
+        views.push_back(make_view(msgs[i], !intensity_in_cloud_));
+        pts += n;
+      }
+      replay_batch(msgs, i - views.size(), views, &out);
     }
     return out;
   }
@@ -401,7 +436,53 @@ class ConeDetector {
     }
     return out;
   }
+  enum Entry { kUnused, kPerMessage, kReplay };
+  void use_entry(Entry e) {
+    if (entry_ != kUnused && entry_ != e)
+      throw GpuError(CP_E_STATE, "cloud_handler and replay keep separate node states: use one per ConeDetector");
+    entry_ = e;
+  }
+  void replay_batch(const std::vector<PointCloud2>& msgs, size_t first, const std::vector<cp_cloud_view>& views,
+                    std::vector<std::vector<PointCloud2>>* out) {
+    cp_detect_params d{distance_treshold_max, distance_treshold_min, level_threshold, angle_threshold,
+                       voxel_filter_leaf_size_x, voxel_filter_leaf_size_y, voxel_filter_leaf_size_z,
+                       min_cluster_size, max_cluster_size, CONE_WIDTH, CONE_HEIGHT};
+    cp_ground_params g{num_of_sectors, default_lowest_point};
+    const uint32_t F = static_cast<uint32_t>(views.size());
+    std::vector<uint32_t> k_off(F + 1);
+    uint64_t K = 0;
+    cp_status st = cp_detect_batch(gpu_, views.data(), F, &d, fused_ground_removal ? &g : nullptr, nullptr,
+                                   k_off.data(), nullptr, 0, &K);
+    if (st != CP_OK) throw GpuError(st, cp_last_error(gpu_));
+    cp_track_params t{classify_colors ? 1 : 0, use_points_buffer ? 1 : 0, cones_matching_dist_theshold,
+                      cone_position_extension_length, CONE_WIDTH};
+    std::vector<cp_tracked_cone> cones(K);
+    std::vector<uint32_t> coff(4 * static_cast<size_t>(F) + 1);
+    uint64_t n = 0;
+    st = cp_batch_track(gpu_, &t, nullptr, 1, cones.data(), coff.data(), K, &n);
+    if (st != CP_OK) throw GpuError(st, cp_last_error(gpu_));
+    for (uint32_t f = 0; f < F; ++f) {
+      std::vector<PointCloud2> clouds(kNumberOfColors);
+      for (int c = 0; c < kNumberOfColors; ++c) {
+        std::vector<Point> pts;
+        for (uint32_t j = coff[4 * f + c]; j < coff[4 * f + c + 1]; ++j) {
+          Point p;
+          p.x = cones[j].x;
+          p.y = cones[j].y;
+          p.z = 0.0;
+          pts.push_back(p);
+        }
+        clouds[c] = to_msg(pts);  // :177-186
+        clouds[c].header = msgs[first + f].header;
+        clouds[c].fields = msgs[first + f].fields;  // Q6
+      }
+      out->push_back(std::move(clouds));
+    }
+  }
   cp_handle* gpu_ = nullptr;
+  Entry entry_ = kUnused;
+  uint64_t max_points_ = 0;
+  uint32_t max_frames_ = 1;
   bool intensity_in_cloud_checked_ = false, intensity_in_cloud_ = true;
   std::vector<float> crop_buf_ = std::vector<float>(4 * 16384);
   std::vector<cp_cluster> clusters_;

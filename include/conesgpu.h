@@ -315,6 +315,50 @@ cp_status cp_cone_colors(cp_handle* h, const cp_cloud_view* cloud, uint32_t fram
  * CP_E_CAPACITY: cap < number of clusters. */
 cp_status cp_batch_cone_colors(cp_handle* h, float cone_width, double extension_length, uint8_t* colors,
                                float* probs, uint32_t* flags, uint32_t* counts, uint64_t cap);
+/* --- what the cone-detection node publishes, over frame sequences (src/cone_detection.cpp:276-340) ---------------
+ * After a run (cp_batch_run, cp_detect_batch or cp_detect): the radial extension, the temporal gate / points buffer,
+ * the colour carry-over from the previous frame's colour clouds, the colour service's response rules and the four
+ * published clouds, for every frame of the run, on the device.
+ *   seq_offsets[n_seqs + 1]: the run's frames as contiguous sequences, each a series of consecutive messages to one
+ *     node (NULL with n_seqs = 1: the whole run is one sequence).  Sequence s continues the handle's state slot s
+ *     (s < cp_config.max_frames): the last frame that slot saw, its extended cones and the colour cloud each was
+ *     published in.  A fresh slot (or one cleared by cp_track_reset) is a node that has just started: its first frame
+ *     publishes nothing.  An empty sequence leaves its slot unchanged.
+ *   out: the published cones, frame-major, then by cloud 0..3 (unknown, yellow, blue, orange); within a cloud the
+ *     node's push_back order (cones with a carried colour in record order, then the cones that needed a colour).
+ *   cloud_offsets[4 * n_frames + 1]: cloud c of frame f is out[cloud_offsets[4 f + c] .. cloud_offsets[4 f + c + 1]).
+ * Colour mode (classify_colors != 0) classifies every record on the device (the chain of cp_batch_cone_colors, needs
+ * a loaded net) and applies the service's response rules to each frame's need list: a bad crop (CP_CONE_BAD_*) leaves
+ * every needed cone unknown; otherwise the answers of the non-empty crops fill the need list from the front.
+ * Calls cp_sync first and leaves the run's results untouched.  No slot changes on any error.
+ * CP_E_PARAM: non-finite threshold or extension length, cone_width not positive and finite in colour mode, n_seqs
+ * 0 or > max_frames, seq_offsets not a non-decreasing partition of [0, n_frames], NULL cloud_offsets / n_out, NULL
+ * out with cones to publish.  CP_E_STATE: no run (or input staged since), no colour net in colour mode, or the run
+ * was already tracked.  CP_E_CAPACITY: cap < *n_out (set); cap = number of clusters always suffices. */
+typedef struct cp_track_params {
+  int32_t classify_colors;               /* node parameter classify_colors                      */
+  int32_t use_points_buffer;             /* node parameter use_points_buffer                    */
+  double cones_matching_dist_theshold;   /* 0.5 (reference spelling)                            */
+  double cone_position_extension_length; /* 0.05                                                */
+  float cone_width;                      /* CONE_WIDTH, box of the colour crops (colour mode only) */
+} cp_track_params;
+typedef struct cp_tracked_cone {
+  float x, y;       /* the extended centroid as published (z = 0)                          */
+  uint32_t cluster; /* index of its record in the run (cp_batch_results order)             */
+  uint32_t color;   /* 0 unknown, 1 yellow, 2 blue, 3 orange: the cloud it is published in  */
+} cp_tracked_cone;
+cp_status cp_batch_track(cp_handle* h, const cp_track_params* t, const uint32_t* seq_offsets, uint32_t n_seqs,
+                         cp_tracked_cone* out, uint32_t* cloud_offsets, uint64_t cap, uint64_t* n_out);
+/* Clears every state slot (each behaves like a node that has just started). */
+cp_status cp_track_reset(cp_handle* h);
+/* Test hook, like cp_debug_sort: the kernels of cp_batch_track on caller-supplied records (record_offsets[n_frames+1],
+ * frame-major) and per-record service answers (colors as cp_batch_cone_colors returns them, CP_CONE_* flags; read in
+ * colour mode only).  Uses and advances the same state slots; needs no run. */
+cp_status cp_debug_track(cp_handle* h, const cp_track_params* t, const cp_cluster* records,
+                         const uint32_t* record_offsets, uint32_t n_frames, const uint8_t* colors,
+                         const uint32_t* flags, const uint32_t* seq_offsets, uint32_t n_seqs,
+                         cp_tracked_cone* out, uint32_t* cloud_offsets, uint64_t cap, uint64_t* n_out);
+
 /* The network alone on host images [n][15][12] uint8 (parity tests; logits optional, before the softmax). */
 cp_status cp_classify_images(cp_handle* h, const uint8_t* images, uint32_t n_images, uint8_t* colors, float* probs,
                              float* logits);
