@@ -32,6 +32,7 @@ ABI_SYMBOLS = [
     "cp_pinned_alloc", "cp_pinned_free",
     "cp_color_net_load", "cp_color_net_load_tflite", "cp_cone_colors", "cp_classify_images",
     "cp_batch_cone_colors", "cp_batch_track", "cp_track_reset", "cp_debug_track",
+    "cp_batch_ground_remove", "cp_batch_ground_device_output",
 ]
 
 CONE_IMG_ROWS, CONE_IMG_COLS = 15, 12
@@ -147,6 +148,8 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.cp_track_reset.argtypes = [vp]
     lib.cp_debug_track.argtypes = [vp, C.POINTER(CTrackParams), vp, vp, u32, vp, vp, vp, u32, vp, vp, u64,
                                    C.POINTER(u64)]
+    lib.cp_batch_ground_remove.argtypes = [vp, C.POINTER(CGroundParams), vp, u64, vp, vp]
+    lib.cp_batch_ground_device_output.argtypes = [vp, C.POINTER(vp), C.POINTER(u64)]
     lib.cp_pinned_alloc.argtypes = [C.c_int32, C.c_size_t, C.c_int32, C.POINTER(vp)]
     lib.cp_pinned_free.argtypes = [vp]
     lib.cp_pinned_free.restype = None
@@ -252,6 +255,7 @@ class ConesGpu:
         cg = to_c_ground(g)
         self._ck(self.lib.cp_ground_remove(self._h, C.byref(view), C.byref(cg), out.ctypes.data, C.byref(kept),
                                            low.ctypes.data))
+        self.n_frames, self.n_points = 1, n   # the frame stays staged
         return out.copy() if copy else out, kept.value, low
 
     def detect(self, msg: PointCloud2, d: DetectParams, g: GroundParams | None = None, cap: int = 4096,
@@ -269,7 +273,7 @@ class ConesGpu:
         cg = to_c_ground(g) if g is not None else None
         self._ck(self.lib.cp_detect(self._h, C.byref(view), C.byref(cd), C.byref(cg) if cg is not None else None,
                                     out.ctypes.data, cap, C.byref(k), ctr.ctypes.data))
-        self.n_frames = 1   # the run is one frame (results(), batch_track())
+        self.n_frames, self.n_points = 1, msg.n_points   # the run is one frame (results(), batch_track())
         return out[:k.value].copy(), ctr[0].copy()
 
     # ---- colour path inputs (SURVEY §8 f3) ----------------------------------------------
@@ -418,12 +422,33 @@ class ConesGpu:
         self._ck(self.lib.cp_batch_set_device_input(self._h, C.c_void_p(d_ptr), len(fp), fp.ctypes.data, point_step,
                                                     off[0], off[1], off[2], off[3]))
         self.n_frames = len(fp)
+        self.n_points = int(fp.sum(dtype=np.uint64))
 
     def set_host_input(self, msgs, fake_missing_intensity: bool = True):
         views = (CCloudView * len(msgs))(*[make_view(m, fake_missing_intensity) for m in msgs])
         self._keep = msgs
         self._ck(self.lib.cp_batch_set_host_input(self._h, views, len(msgs)))
         self.n_frames = len(msgs)
+        self.n_points = sum(m.n_points for m in msgs)
+
+    def batch_ground_remove(self, g: GroundParams, host: bool = True):
+        """GroundRemover::cloud_handler (src/ground_removal.cpp:54-79) for every frame of the staged batch (stage host
+        clouds with fake_missing_intensity=False, as the ground node reads them).  Returns (cloud32 [sum N_f, 8]
+        float32, frame f's message at rows P_f .. P_f + N_f, or None when host is False; n_kept u32 [F];
+        low f32 [F, 17]).  The messages stay on the device: ground_device_output()."""
+        out = np.empty((self.n_points, 8), np.float32) if host else None
+        kept = np.zeros(self.n_frames, np.uint32)
+        low = np.zeros((self.n_frames, 17), np.float32)
+        cg = to_c_ground(g)
+        self._ck(self.lib.cp_batch_ground_remove(self._h, C.byref(cg), out.ctypes.data if host else None,
+                                                 self.n_points if host else 0, kept.ctypes.data, low.ctypes.data))
+        return out, kept, low
+
+    def ground_device_output(self):
+        """(device pointer, n_points) of the messages of the last batch_ground_remove (32 B per point)."""
+        p, n = C.c_void_p(), C.c_uint64()
+        self._ck(self.lib.cp_batch_ground_device_output(self._h, C.byref(p), C.byref(n)))
+        return p.value, n.value
 
     def run(self, d: DetectParams, g: GroundParams | None = None):
         cd = to_c_detect(d)

@@ -118,7 +118,10 @@ struct cp_handle {
   Ctl* d_ctl = nullptr;
   uint8_t* d_in = nullptr;  // staged input (host batches)
   size_t d_in_bytes = 0;
-  uint8_t* d_out32 = nullptr;
+  uint8_t* d_out32 = nullptr;   // the ground node's messages (max_points x 32 B), allocated on first use
+  u64 ground_points = 0;        // points of the messages cp_batch_ground_remove left in d_out32 ...
+  bool ground_out = false;      // ... valid until the next staging, run or ground call
+  u32* h_ground = nullptr;      // pinned readback of cp_batch_ground_remove: G_f, then the sector minima
   // colour path (color_kernels.cuh): allocated on first use, grown on demand
   struct ColorBufs {
     u32 *mask = nullptr, *tcount = nullptr, *texcl = nullptr, *off = nullptr, *flags = nullptr;
@@ -584,24 +587,23 @@ void launch_keep_mask(cp_handle* h, const Geom& g, const CropK& c, const GroundK
 }
 
 // part 2: tile scan -> ordered gather (+bbox) into the global survivor arrays
-// (general back half, node-equivalent ground removal, parity taps)
-template <bool OUT32>
-void launch_scan_gather(cp_handle* h, const Geom& g, const GroundK& gk, u32 cap, uint8_t* out32) {
+// (general back half, parity taps)
+void launch_scan_gather(cp_handle* h, const Geom& g, const GroundK& gk, u32 cap) {
   GatherOut go;
   go.pts = h->d_pts;
   go.src = h->d_src;
   go.frame = h->d_frame;
   go.cap = cap;
   go.bbox_key = h->d_bbox;
-  go.out32 = out32;
+  go.out32 = nullptr;
   const u32 stiles = (g.n_tiles + kScanTile - 1) / kScanTile;
   tile_scan_kernel<<<(h->tile_ctas || stiles < (u32)h->sms * 4) ? stiles : (u32)h->sms * 4, kScanThreads, 0, h->stream>>>(
       g, h->d_tile_count, h->d_tile_excl, h->d_c_off, h->d_desc_a, h->d_ctl, cap);
   const u32 ggrid = grid_for((u64)g.n_tiles * 32, 256, h->sms, 8);
   switch (h->layout.mode) {
-    case 0: gather_survivors_kernel<0, OUT32><<<ggrid, 256, 0, h->stream>>>(h->in_ptr, h->layout, g, gk, h->d_mask, h->d_tile_count, h->d_tile_excl, go); break;
-    case 1: gather_survivors_kernel<1, OUT32><<<ggrid, 256, 0, h->stream>>>(h->in_ptr, h->layout, g, gk, h->d_mask, h->d_tile_count, h->d_tile_excl, go); break;
-    default: gather_survivors_kernel<2, OUT32><<<ggrid, 256, 0, h->stream>>>(h->in_ptr, h->layout, g, gk, h->d_mask, h->d_tile_count, h->d_tile_excl, go); break;
+    case 0: gather_survivors_kernel<0><<<ggrid, 256, 0, h->stream>>>(h->in_ptr, h->layout, g, gk, h->d_mask, h->d_tile_count, h->d_tile_excl, go); break;
+    case 1: gather_survivors_kernel<1><<<ggrid, 256, 0, h->stream>>>(h->in_ptr, h->layout, g, gk, h->d_mask, h->d_tile_count, h->d_tile_excl, go); break;
+    default: gather_survivors_kernel<2><<<ggrid, 256, 0, h->stream>>>(h->in_ptr, h->layout, g, gk, h->d_mask, h->d_tile_count, h->d_tile_excl, go); break;
   }
   h->launches += 2;
   h->gathered = true;
@@ -1106,7 +1108,7 @@ void enqueue_back_fast(cp_handle* h, const RunParams& rp) {
   fa.tap_labels = h->taps ? h->d_tap_labels : nullptr;
   // the crop taps (survivor arrays, offsets) come from the global keep mask + gather
   if (h->taps && !h->masked) launch_keep_mask(h, fa.geom, rp.crop, rp.gk, h->run_sgrid);
-  if (h->taps && !h->gathered) launch_scan_gather<false>(h, fa.geom, rp.gk, (u32)h->cap_c, nullptr);
+  if (h->taps && !h->gathered) launch_scan_gather(h, fa.geom, rp.gk, (u32)h->cap_c);
   switch (h->layout.mode) {
     case 0: launch_frame_kernel<CMAX, VMAX, 0, T>(h, fa); break;
     case 1: launch_frame_kernel<CMAX, VMAX, 1, T>(h, fa); break;
@@ -1188,7 +1190,7 @@ cp_status enqueue_back(cp_handle* h, bool retry) {
       launch_mask_compact<false>(h, device_geom(h), rp.crop, rp.gk, (u32)h->cap_c, nullptr);
     } else {   // a keep mask exists already (single-pass front ends, a retried one-launch frame)
       if (!h->masked) launch_keep_mask(h, device_geom(h), rp.crop, rp.gk, h->run_sgrid);
-      if (!h->gathered) launch_scan_gather<false>(h, device_geom(h), rp.gk, (u32)h->cap_c, nullptr);
+      if (!h->gathered) launch_scan_gather(h, device_geom(h), rp.gk, (u32)h->cap_c);
     }
     enqueue_back_general(h, rp);
   }
@@ -1942,6 +1944,7 @@ cp_status cp_batch_set_device_input(cp_handle* h, const void* d_points, uint32_t
   }
   CK(cudaSetDevice(h->cfg.device));
   h->batch_ready = false;
+  h->ground_out = false;
   cp_status st = set_geometry(h, frame_points, n_frames);
   if (st) return st;
   h->layout = make_layout(point_step, off_x, off_y, off_z, off_intensity);
@@ -1962,6 +1965,7 @@ cp_status cp_batch_set_host_input(cp_handle* h, const cp_cloud_view* frames, uin
   }
   CK(cudaSetDevice(h->cfg.device));
   h->batch_ready = false;
+  h->ground_out = false;
   std::vector<u32> fp(n_frames);
   size_t bytes = 0;
   for (u32 f = 0; f < n_frames; ++f) {
@@ -2069,6 +2073,7 @@ static RunKey make_key(const cp_handle* h, const cp_detect_params* d, const cp_g
 cp_status cp_batch_run(cp_handle* h, const cp_detect_params* d, const cp_ground_params* ground) try {
   if (!h) return CP_E_PARAM;
   h->tracked = false;
+  h->ground_out = false;
   CK(cudaSetDevice(h->cfg.device));
   const bool eligible = h->use_graph && d && h->batch_ready && !h->taps && !h->stage_timing && h->hg.uniform_n != 0;
   if (!eligible) {
@@ -2238,19 +2243,14 @@ cp_status cp_detect(cp_handle* h, const cp_cloud_view* in, const cp_detect_param
   return abi_exception(h);
 }
 
-cp_status cp_ground_remove(cp_handle* h, const cp_cloud_view* in, const cp_ground_params* g, void* out_xyzi32,
-                           uint32_t* n_kept, float* low17) try {
-  if (!h) return CP_E_PARAM;
-  if (!g || !out_xyzi32) {
-    h->err = "NULL ground params or output";
-    return CP_E_PARAM;
-  }
-  cp_status st = cp_batch_set_host_input(h, in, 1);
-  if (st) return st;
-  const u32 n = h->hg.frame_n[0];
+namespace {
+// The ground node over the staged batch (cp_ground_remove, cp_batch_ground_remove): pass 1 (sector minima), then
+// every frame's complete message into d_out32 in one pass (mask_compact_kernel<*, true>).  Enqueued only.
+cp_status enqueue_ground(cp_handle* h, const cp_ground_params* g) {
   if (!h->d_out32) {
     cudaError_t e = cudaMalloc(&h->d_out32, (size_t)h->cfg.max_points * 32);
     if (e != cudaSuccess) {
+      cudaGetLastError();
       h->err = "cudaMalloc of the 32-byte output cloud failed";
       return CP_E_NOMEM;
     }
@@ -2260,6 +2260,7 @@ cp_status cp_ground_remove(cp_handle* h, const cp_cloud_view* in, const cp_groun
   launch_init(h, g->default_lowest_point);
   const u32 sgrid = grid_for((u64)geo.n_tiles * kStreamThreads, kStreamThreads, h->sms, 8);
   launch_sector_min(h, geo, sgrid);
+  h->launches++;
   h->rowmax_valid = h->use_rowskip;
   CropK crop;
   memset(&crop, 0, sizeof(crop));
@@ -2267,17 +2268,15 @@ cp_status cp_ground_remove(cp_handle* h, const cp_cloud_view* in, const cp_groun
   gk.do_ground = 1;
   gk.want_count = 1;
   gk.pad_survives = 0;
-  launch_mask_compact<true>(h, geo, crop, gk, n, h->d_out32);
-  CK(cudaMemcpyAsync(h->h_ctl, h->d_ctl, sizeof(Ctl), cudaMemcpyDeviceToHost, h->stream));
-  static_assert(kNSect <= kSectStride, "h_frame_u32 holds at least kSectStride words");
-  if (low17) CK(cudaMemcpyAsync(h->h_frame_u32, h->d_low_key, sizeof(u32) * kNSect, cudaMemcpyDeviceToHost, h->stream));
-  // Only the G survivors cross PCIe.  The N - G padding points the node appends (:79: value-initialised
-  // PointXYZI, 1.0f at offset 12) are the same 32 bytes over and over: the host writes them into the caller's buffer
-  // itself — in parallel, while the GPU is still working — instead of the GPU writing them to HBM and a 4 MB
-  // device-to-host copy carrying them back (that copy was most of the call).
-  uint8_t* out8 = static_cast<uint8_t*>(out_xyzi32);
-  const size_t out_bytes = (size_t)n * 32;
-  bool filled = false;
+  launch_mask_compact<true>(h, geo, crop, gk, (u32)h->hg.n_points, h->d_out32);
+  return CP_OK;
+}
+
+// Only the survivors cross PCIe.  The padding points the node appends (:79: value-initialised PointXYZI, 1.0f at
+// offset 12) are the same 32 bytes over and over: the host writes them into the caller's buffer itself — in
+// parallel, while the GPU is still working — instead of a device-to-host copy carrying them back (for one frame
+// that copy was most of the call).  The survivors are copied over the fill afterwards.
+void fill_pad_host(cp_handle* h, uint8_t* out8, size_t out_bytes) {
   if (h->stage_threads > 1 && out_bytes >= kParallelStageMin) {
     if (!h->copy_pool) {
       try {
@@ -2291,10 +2290,30 @@ cp_status cp_ground_remove(cp_handle* h, const cp_cloud_view* in, const cp_groun
       b->work();
       for (u32 gi = 0; gi < b->n_groups; ++gi)
         while (!b->group_done(gi)) std::this_thread::yield();
-      filled = true;
+      return;
     }
   }
-  if (!filled) fill_pad_points(out8, out_bytes);
+  fill_pad_points(out8, out_bytes);
+}
+}  // namespace
+
+cp_status cp_ground_remove(cp_handle* h, const cp_cloud_view* in, const cp_ground_params* g, void* out_xyzi32,
+                           uint32_t* n_kept, float* low17) try {
+  if (!h) return CP_E_PARAM;
+  if (!g || !out_xyzi32) {
+    h->err = "NULL ground params or output";
+    return CP_E_PARAM;
+  }
+  cp_status st = cp_batch_set_host_input(h, in, 1);
+  if (st) return st;
+  const u32 n = h->hg.frame_n[0];
+  st = enqueue_ground(h, g);
+  if (st) return st;
+  CK(cudaMemcpyAsync(h->h_ctl, h->d_ctl, sizeof(Ctl), cudaMemcpyDeviceToHost, h->stream));
+  static_assert(kNSect <= kSectStride, "h_frame_u32 holds at least kSectStride words");
+  if (low17) CK(cudaMemcpyAsync(h->h_frame_u32, h->d_low_key, sizeof(u32) * kNSect, cudaMemcpyDeviceToHost, h->stream));
+  uint8_t* out8 = static_cast<uint8_t*>(out_xyzi32);
+  fill_pad_host(h, out8, (size_t)n * 32);
   CK(cudaStreamSynchronize(h->stream));
   CK(cudaGetLastError());
   const u32 kept = h->h_ctl->n_surv;
@@ -2306,6 +2325,83 @@ cp_status cp_ground_remove(cp_handle* h, const cp_cloud_view* in, const cp_groun
   if (low17)
     for (int s = 0; s < kNSect; ++s) low17[s] = ord2f(h->h_frame_u32[s]);
   h->ran = false;
+  return CP_OK;
+} catch (...) {
+  return abi_exception(h);
+}
+
+cp_status cp_batch_ground_remove(cp_handle* h, const cp_ground_params* g, void* out_xyzi32, uint64_t cap_points,
+                                 uint32_t* n_kept, float* low17) try {
+  if (!h) return CP_E_PARAM;
+  h->ground_out = false;   // from here on d_out32 is being rewritten
+  if (!g) {
+    h->err = "NULL ground params";
+    return CP_E_PARAM;
+  }
+  if (!h->batch_ready) {
+    h->err = "cp_batch_ground_remove before cp_batch_set_device_input / cp_batch_set_host_input";
+    return CP_E_STATE;
+  }
+  const u32 F = h->hg.n_frames;
+  const u64 n = h->hg.n_points;
+  if (out_xyzi32 && cap_points < n) {
+    h->err = "output buffer holds fewer points than the staged batch";
+    return CP_E_CAPACITY;
+  }
+  CK(cudaSetDevice(h->cfg.device));
+  if (!h->h_ground) {
+    cp_status sa = palloc(h, &h->h_ground, (size_t)h->cfg.max_frames * (1 + kSectStride));
+    if (sa) return sa;
+  }
+  cp_status st = enqueue_ground(h, g);
+  if (st) return st;
+  h->ran = false;   // the run's intermediate buffers now hold the ground call's
+  u32* h_kept = h->h_ground;
+  u32* h_low = h->h_ground + F;
+  CK(cudaMemcpyAsync(h->h_ctl, h->d_ctl, sizeof(Ctl), cudaMemcpyDeviceToHost, h->stream));   // cp_last_rows_loaded
+  CK(cudaMemcpyAsync(h_kept, h->d_c_off + 1, sizeof(u32) * F, cudaMemcpyDeviceToHost, h->stream));
+  if (low17) CK(cudaMemcpyAsync(h_low, h->d_low_key, sizeof(u32) * kSectStride * F, cudaMemcpyDeviceToHost, h->stream));
+  uint8_t* out8 = static_cast<uint8_t*>(out_xyzi32);
+  if (out8) fill_pad_host(h, out8, (size_t)n * 32);
+  CK(cudaStreamSynchronize(h->stream));
+  CK(cudaGetLastError());
+  if (out8) {
+    // frame f's survivors lie at the start of its message; runs of frames that dropped nothing merge into one copy
+    u64 lo = 0, hi = 0;   // pending copy [lo, hi) in points
+    for (u32 f = 0; f < F; ++f) {
+      const u64 p0 = h->hg.frame_off[f];
+      if (p0 != hi) {
+        if (hi > lo) CK(cudaMemcpyAsync(out8 + lo * 32, h->d_out32 + lo * 32, (hi - lo) * 32, cudaMemcpyDeviceToHost, h->stream));
+        lo = p0;
+      }
+      hi = p0 + h_kept[f];
+    }
+    if (hi > lo) CK(cudaMemcpyAsync(out8 + lo * 32, h->d_out32 + lo * 32, (hi - lo) * 32, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+  }
+  if (n_kept) memcpy(n_kept, h_kept, sizeof(u32) * F);
+  if (low17)
+    for (u32 f = 0; f < F; ++f)
+      for (int s = 0; s < kNSect; ++s) low17[(size_t)f * kNSect + s] = ord2f(h_low[(size_t)f * kSectStride + s]);
+  h->ground_points = n;
+  h->ground_out = true;
+  return CP_OK;
+} catch (...) {
+  return abi_exception(h);
+}
+
+cp_status cp_batch_ground_device_output(cp_handle* h, const void** d_out_xyzi32, uint64_t* n_points) try {
+  if (!h) return CP_E_PARAM;
+  if (!d_out_xyzi32 || !n_points) {
+    h->err = "NULL d_out_xyzi32 or n_points";
+    return CP_E_PARAM;
+  }
+  if (!h->ground_out) {
+    h->err = "no cp_batch_ground_remove since the last staging or run";
+    return CP_E_STATE;
+  }
+  *d_out_xyzi32 = h->d_out32;
+  *n_points = h->ground_points;
   return CP_OK;
 } catch (...) {
   return abi_exception(h);

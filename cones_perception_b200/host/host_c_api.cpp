@@ -31,6 +31,37 @@ PointCloud2 make_msg(const float* xyzi, uint32_t n, int with_intensity_field, ui
   if (n) std::memcpy(m.data.data(), xyzi, static_cast<size_t>(n) * 16);
   return m;
 }
+
+// messages 0..n_msgs-1 of a series: compact xyzi, frame_n[i] points each, stamps 100 + i s, 123456789 + i ns
+std::vector<PointCloud2> make_msgs(const float* xyzi, const uint32_t* frame_n, uint32_t n_msgs, int with_intensity_field) {
+  std::vector<PointCloud2> msgs;
+  size_t at = 0;
+  for (uint32_t i = 0; i < n_msgs; ++i) {
+    msgs.push_back(make_msg(xyzi + 4 * at, frame_n[i], with_intensity_field, 100 + i, 123456789 + i));
+    at += frame_n[i];
+  }
+  return msgs;
+}
+
+// a published message, serialised field by field: header, layout, fields, data
+void serialise(const PointCloud2& m, std::vector<uint8_t>* b) {
+  auto put = [b](const void* p, size_t n) { b->insert(b->end(), static_cast<const uint8_t*>(p), static_cast<const uint8_t*>(p) + n); };
+  put(&m.header.seq, 4); put(&m.header.stamp_sec, 4); put(&m.header.stamp_nsec, 4);
+  put(m.header.frame_id.data(), m.header.frame_id.size());
+  put(&m.height, 4); put(&m.width, 4);
+  for (const PointField& f : m.fields) {
+    put(f.name.data(), f.name.size()); put(&f.offset, 4); put(&f.datatype, 1); put(&f.count, 4);
+  }
+  put(&m.is_bigendian, 1); put(&m.point_step, 4); put(&m.row_step, 4);
+  put(m.data.data(), m.data.size()); put(&m.is_dense, 1);
+}
+
+int copy_out(const std::vector<uint8_t>& b, uint8_t* out, uint64_t cap, uint64_t* used) {
+  *used = b.size();
+  if (b.size() > cap) return 3;
+  if (!b.empty()) std::memcpy(out, b.data(), b.size());
+  return 0;
+}
 }  // namespace
 
 extern "C" {
@@ -267,12 +298,7 @@ int ch_detector_publish(void* dp, const float* xyzi, const uint32_t* frame_n, ui
                         int replay, uint8_t* out, uint64_t cap, uint64_t* used) {
   try {
     auto* det = static_cast<ConeDetector*>(dp);
-    std::vector<PointCloud2> msgs;
-    size_t at = 0;
-    for (uint32_t i = 0; i < n_msgs; ++i) {
-      msgs.push_back(make_msg(xyzi + 4 * at, frame_n[i], with_intensity_field, 100 + i, 123456789 + i));
-      at += frame_n[i];
-    }
+    std::vector<PointCloud2> msgs = make_msgs(xyzi, frame_n, n_msgs, with_intensity_field);
     std::vector<std::vector<PointCloud2>> pub;
     if (replay) {
       pub = det->replay(msgs);
@@ -280,22 +306,9 @@ int ch_detector_publish(void* dp, const float* xyzi, const uint32_t* frame_n, ui
       for (const PointCloud2& m : msgs) pub.push_back(det->cloud_handler(m));
     }
     std::vector<uint8_t> b;
-    auto put = [&b](const void* p, size_t n) { b.insert(b.end(), static_cast<const uint8_t*>(p), static_cast<const uint8_t*>(p) + n); };
     for (const auto& clouds : pub)
-      for (const PointCloud2& m : clouds) {
-        put(&m.header.seq, 4); put(&m.header.stamp_sec, 4); put(&m.header.stamp_nsec, 4);
-        put(m.header.frame_id.data(), m.header.frame_id.size());
-        put(&m.height, 4); put(&m.width, 4);
-        for (const PointField& f : m.fields) {
-          put(f.name.data(), f.name.size()); put(&f.offset, 4); put(&f.datatype, 1); put(&f.count, 4);
-        }
-        put(&m.is_bigendian, 1); put(&m.point_step, 4); put(&m.row_step, 4);
-        put(m.data.data(), m.data.size()); put(&m.is_dense, 1);
-      }
-    *used = b.size();
-    if (b.size() > cap) return 3;
-    if (!b.empty()) std::memcpy(out, b.data(), b.size());
-    return 0;
+      for (const PointCloud2& m : clouds) serialise(m, &b);
+    return copy_out(b, out, cap, used);
   } catch (const std::exception& e) {
     g_err = e.what();
     return 4;
@@ -311,6 +324,38 @@ void* ch_ground_create(uint64_t max_points, int device) {
   }
 }
 void ch_ground_destroy(void* g) { delete static_cast<GroundRemover*>(g); }
+
+// GroundRemover::replay in device batches of up to max_frames messages.  ch_ground_publish: messages 0..n_msgs-1
+// (compact xyzi, frame_n[i] points each) through replay (replay != 0) or through cloud_handler, one call per
+// message; out receives every published message serialised as ch_detector_publish does, one per input message.
+void* ch_ground_create_replay(uint64_t max_points, uint32_t max_frames, int device) {
+  try {
+    return new GroundRemover(max_points, device, 32, max_frames);
+  } catch (const std::exception& e) {
+    g_err = e.what();
+    return nullptr;
+  }
+}
+
+int ch_ground_publish(void* gp, const float* xyzi, const uint32_t* frame_n, uint32_t n_msgs, int with_intensity_field,
+                      int replay, uint8_t* out, uint64_t cap, uint64_t* used) {
+  try {
+    auto* gr = static_cast<GroundRemover*>(gp);
+    std::vector<PointCloud2> msgs = make_msgs(xyzi, frame_n, n_msgs, with_intensity_field);
+    std::vector<PointCloud2> pub;
+    if (replay) {
+      pub = gr->replay(msgs);
+    } else {
+      for (const PointCloud2& m : msgs) pub.push_back(gr->cloud_handler(m));
+    }
+    std::vector<uint8_t> b;
+    for (const PointCloud2& m : pub) serialise(m, &b);
+    return copy_out(b, out, cap, used);
+  } catch (const std::exception& e) {
+    g_err = e.what();
+    return 4;
+  }
+}
 
 int ch_ground_handle(void* gp, const float* xyzi, uint32_t n, int with_intensity_field, void* out32,
                      uint32_t* kept, uint32_t* out_point_step, uint32_t* out_stamp_nsec, uint32_t* out_n_fields) {

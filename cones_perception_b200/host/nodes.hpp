@@ -46,14 +46,18 @@ class GroundRemover {
   std::string input_cloud_topic = "/cloud";
   std::string groundless_cloud_topic = "groundless_cloud";
 
-  explicit GroundRemover(uint64_t max_points = 4u << 20, int device = 0, uint32_t max_point_step = 64) {
+  // max_frames > 1 only matters for replay(): messages per device batch (max_points bounds their points)
+  explicit GroundRemover(uint64_t max_points = 4u << 20, int device = 0, uint32_t max_point_step = 64,
+                         uint32_t max_frames = 1) {
     cp_config cfg{};
     cfg.device = device;
     cfg.max_points = max_points;
-    cfg.max_frames = 1;
+    cfg.max_frames = max_frames;
     cfg.max_point_step = max_point_step;
     cp_status st = cp_create(&gpu_, &cfg);
     if (st != CP_OK) throw GpuError(st, cp_create_error());
+    max_points_ = max_points;
+    max_frames_ = max_frames;
   }
   ~GroundRemover() { cp_destroy(gpu_); }
   GroundRemover(const GroundRemover&) = delete;
@@ -63,9 +67,55 @@ class GroundRemover {
   PointCloud2 cloud_handler(const PointCloud2& cloud_msg) {
     cp_cloud_view in = make_view(cloud_msg, /*fake_missing_intensity=*/false);
     cp_ground_params g{num_of_sectors, default_lowest_point};
+    PointCloud2 out = published_shell(cloud_msg);
+    cp_status st = cp_ground_remove(gpu_, &in, &g, out.data.data(), &last_kept_, nullptr);
+    if (st != CP_OK) throw GpuError(st, cp_last_error(gpu_));
+    return out;
+  }
+
+  // cloud_handler for a series of messages, in device batches of up to max_frames messages and max_points points
+  // (cp_batch_ground_remove).  Returns, per message, the message cloud_handler would publish.  The node keeps no
+  // state between messages, so replay and cloud_handler may be mixed on one object.
+  std::vector<PointCloud2> replay(const std::vector<PointCloud2>& msgs) {
+    std::vector<PointCloud2> out;
+    out.reserve(msgs.size());
+    cp_ground_params g{num_of_sectors, default_lowest_point};
+    size_t i = 0;
+    while (i < msgs.size()) {
+      std::vector<cp_cloud_view> views;
+      uint64_t pts = 0;
+      for (; i < msgs.size() && views.size() < max_frames_; ++i) {
+        const uint64_t n = static_cast<uint64_t>(msgs[i].width) * msgs[i].height;
+        if (!views.empty() && pts + n > max_points_) break;
+        views.push_back(make_view(msgs[i], /*fake_missing_intensity=*/false));
+        pts += n;
+      }
+      const size_t first = i - views.size();
+      const uint32_t F = static_cast<uint32_t>(views.size());
+      cp_status st = cp_batch_set_host_input(gpu_, views.data(), F);
+      if (st != CP_OK) throw GpuError(st, cp_last_error(gpu_));
+      batch_buf_.resize(static_cast<size_t>(pts) * 32);
+      std::vector<uint32_t> kept(F);
+      st = cp_batch_ground_remove(gpu_, &g, batch_buf_.data(), pts, kept.data(), nullptr);
+      if (st != CP_OK) throw GpuError(st, cp_last_error(gpu_));
+      size_t at = 0;
+      for (uint32_t f = 0; f < F; ++f) {
+        PointCloud2 m = published_shell(msgs[first + f]);
+        if (!m.data.empty()) std::memcpy(m.data.data(), batch_buf_.data() + at, m.data.size());
+        at += m.data.size();
+        out.push_back(std::move(m));
+      }
+      last_kept_ = kept[F - 1];
+    }
+    return out;
+  }
+  uint32_t last_kept() const { return last_kept_; }
+
+ private:
+  // the published message around the data: toROSMsg (:86) overwrites the header/fields assigned at :83-84: PCL
+  // layout, and the stamp survives the ROS -> PCL -> ROS round trip at microsecond resolution (Q5)
+  static PointCloud2 published_shell(const PointCloud2& cloud_msg) {
     PointCloud2 out;
-    // toROSMsg (:86) overwrites the header/fields assigned at :83-84: PCL layout, and the stamp
-    // survives the ROS -> PCL -> ROS round trip at microsecond resolution (Q5)
     out.header = cloud_msg.header;
     out.header.stamp_nsec = cloud_msg.header.stamp_nsec / 1000u * 1000u;
     out.height = cloud_msg.height;
@@ -76,15 +126,13 @@ class GroundRemover {
     out.row_step = 32 * out.width;
     out.is_dense = cloud_msg.is_dense;
     out.data.resize(static_cast<size_t>(out.row_step) * out.height);
-    cp_status st = cp_ground_remove(gpu_, &in, &g, out.data.data(), &last_kept_, nullptr);
-    if (st != CP_OK) throw GpuError(st, cp_last_error(gpu_));
     return out;
   }
-  uint32_t last_kept() const { return last_kept_; }
-
- private:
   cp_handle* gpu_ = nullptr;
+  uint64_t max_points_ = 0;
+  uint32_t max_frames_ = 1;
   uint32_t last_kept_ = 0;
+  std::vector<uint8_t> batch_buf_;
 };
 
 // the stateful tail of get_centroid_clouds (src/cone_detection.cpp:276-340), separated so it

@@ -14,6 +14,8 @@
  *                       src/perception_handling/utils.cpp:32-34)
  *   cp_batch_*         the same path over many independent frames per launch
  *                      (BASELINE.json configs 3-5)
+ *   cp_batch_ground_remove  GroundRemover::cloud_handler for every frame of a batch:
+ *                      one groundless_cloud message per frame, on the device or the host
  *
  * Plain C types only: no exceptions, no C++ or torch types cross this boundary.
  * A handle is used by one thread at a time (the reference nodes are single-threaded
@@ -155,6 +157,27 @@ cp_status cp_batch_set_device_input(cp_handle* h, const void* d_points, uint32_t
  *     has returned. */
 cp_status cp_batch_set_host_input(cp_handle* h, const cp_cloud_view* frames, uint32_t n_frames);
 
+/* src/ground_removal.cpp:54-79 for every frame of the staged batch (cp_batch_set_device_input /
+ * cp_batch_set_host_input; stage host clouds without an intensity field with off_intensity < 0, as
+ * cp_ground_remove does).  Frame f's message is out_xyzi32[32*P_f .. 32*(P_f + N_f)), P_f = sum of N_g
+ * for g < f, N_f = width*height of frame f: exactly the bytes cp_ground_remove writes for that frame alone
+ * (survivors in input order, then N_f - G_f PCL padding points).  out_xyzi32 NULL: device output only
+ * (cp_batch_ground_device_output), cap_points is then not read.  n_kept[n_frames] (G_f) and
+ * low17[17*n_frames] (each frame's sector minima) are optional.
+ * Only the survivors are copied back; the host writes the padding into out_xyzi32 while the GPU works.
+ * Returns after the device work is complete, so another handle can read the device output at once (the
+ * two-node chain: cp_batch_set_device_input(d_out, ..., point_step 32, offsets 0/4/8/16)).
+ * Ends the run: cp_batch_results, cp_batch_cone_colors and cp_batch_track return CP_E_STATE until the next
+ * cp_batch_run.  The input stays staged, and a following cp_batch_run on it returns what it would have.
+ * CP_E_PARAM: NULL g.  CP_E_STATE: nothing staged.  CP_E_CAPACITY: cap_points < sum of N_f.
+ * CP_E_NOMEM: the max_points x 32 B device buffer of the messages cannot be allocated. */
+cp_status cp_batch_ground_remove(cp_handle* h, const cp_ground_params* g, void* out_xyzi32, uint64_t cap_points,
+                                 uint32_t* n_kept, float* low17);
+/* The complete messages of the last cp_batch_ground_remove on the device (sum N_f points x 32 B, padding
+ * included).  Valid until the next cp_ground_remove / cp_batch_ground_remove on this handle.
+ * CP_E_PARAM: NULL argument.  CP_E_STATE: no cp_batch_ground_remove since the last staging or run. */
+cp_status cp_batch_ground_device_output(cp_handle* h, const void** d_out_xyzi32, uint64_t* n_points);
+
 /* Enqueue the whole pipeline for the current batch on the handle's stream (async). */
 cp_status cp_batch_run(cp_handle* h, const cp_detect_params* d, const cp_ground_params* ground);
 
@@ -229,8 +252,9 @@ uint64_t cp_last_rows_loaded(const cp_handle* h);
  * left early because both voxels already hung under the same root).  The reference's kd-tree visits
  * O(V * k log k) instead (src/cone_detection.cpp:206-220). */
 void cp_last_pairs(const cp_handle* h, uint64_t* visited, uint64_t* tested);
-/* Kernel launches enqueued by the last cp_batch_run / cp_detect / cp_ground_remove / cp_batch_cone_colors (the
- * latter counts its own launches only; it does not grow with the number of frames or clusters). */
+/* Kernel launches enqueued by the last cp_batch_run / cp_detect / cp_ground_remove / cp_batch_ground_remove /
+ * cp_batch_cone_colors (the latter counts its own launches only; it does not grow with the number of frames or
+ * clusters, and neither does cp_batch_ground_remove's). */
 uint32_t cp_last_launch_count(const cp_handle* h);
 /* The handle's stream as a cudaStream_t, for callers that time with their own events. */
 void* cp_stream(cp_handle* h);
