@@ -32,11 +32,12 @@ ABI_SYMBOLS = [
     "cp_pinned_alloc", "cp_pinned_free",
     "cp_color_net_load", "cp_color_net_load_tflite", "cp_cone_colors", "cp_classify_images",
     "cp_batch_cone_colors", "cp_batch_track", "cp_track_reset", "cp_debug_track",
-    "cp_batch_ground_remove", "cp_batch_ground_device_output",
+    "cp_batch_ground_remove", "cp_batch_ground_device_output", "cp_set_color_cloud",
 ]
 
 CONE_IMG_ROWS, CONE_IMG_COLS = 15, 12
 CONE_EMPTY, CONE_BAD_INDEX, CONE_BAD_INTENSITY, CONE_AMBIGUOUS, CONE_LOW_CONFIDENCE = 1, 2, 4, 8, 16
+COLOR_CLOUD_STAGED, COLOR_CLOUD_GROUNDLESS = 0, 1   # cp_set_color_cloud
 COLOR_NO_ANSWER = 255   # cp_cone_colors: the service would skip this cone (empty crop) or raise (bad crop)
 
 CLUSTER_DTYPE = np.dtype([("x", np.float32), ("y", np.float32), ("size", np.uint32), ("min_index", np.uint32)])
@@ -150,6 +151,7 @@ def load_library(path: str | None = None) -> C.CDLL:
                                    C.POINTER(u64)]
     lib.cp_batch_ground_remove.argtypes = [vp, C.POINTER(CGroundParams), vp, u64, vp, vp]
     lib.cp_batch_ground_device_output.argtypes = [vp, C.POINTER(vp), C.POINTER(u64)]
+    lib.cp_set_color_cloud.argtypes = [vp, C.c_int32]
     lib.cp_pinned_alloc.argtypes = [C.c_int32, C.c_size_t, C.c_int32, C.POINTER(vp)]
     lib.cp_pinned_free.argtypes = [vp]
     lib.cp_pinned_free.restype = None
@@ -371,6 +373,12 @@ class ConesGpu:
         self._ck(self.lib.cp_batch_cone_colors(self._h, cone_width, extension_length, colors.ctypes.data,
                                                probs.ctypes.data, flags.ctypes.data, counts.ctypes.data, K))
         return colors, probs, flags, counts
+
+    def set_color_cloud(self, groundless: bool):
+        """Crop colours of the staged input (cone_* with msg=None, batch_cone_colors, batch_track in colour mode) from
+        the ground node's message of each frame after a run with ground removal (groundless=True), as the reference's
+        two-node launch does, or from the staged cloud itself (False, the default)."""
+        self._ck(self.lib.cp_set_color_cloud(self._h, COLOR_CLOUD_GROUNDLESS if groundless else COLOR_CLOUD_STAGED))
 
     # ---- what the node publishes, over frame sequences ----------------------------------
     @staticmethod

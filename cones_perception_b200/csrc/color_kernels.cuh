@@ -13,6 +13,12 @@
 // ROS service; here the cloud already sits in HBM from the detection pass and only 180 bytes
 // per cone travel back.
 //
+// Crops from the ground node's message (CP_COLOR_CLOUD_GROUNDLESS after a run with ground removal).  In the
+// reference's default launch the detector crops from the groundless_cloud message: the points the ground filter
+// keeps, in input order, then N - G zero points (src/ground_removal.cpp:79).  The mask kernels keep a point that lies
+// in a box only if ground_node_keeps() (evaluated for those points alone), and a box that contains (0, 0) gets the
+// N - G zero points after its kept points: counted with the crop offsets, written by the gather kernels.
+//
 // Exactness.  The box test is the reference's double-precision comparison folded into four
 // fp32 bounds by box_bounds (largest / smallest float on the right side of each double bound),
 // so the crops are bit-exact.  The raster evaluates the numpy formulas in fp64; the only
@@ -34,12 +40,29 @@ struct ConeBoxes {
   float xlo[kConeChunk], xhi[kConeChunk], ylo[kConeChunk], yhi[kConeChunk];
 };
 
+// The ground node's verdict on one point (src/ground_removal.cpp:70-77) as keep_point reaches it: non-finite points
+// are dropped, the sector is sector_of's, and the threshold is derived from the frame's sector minima
+// (low_key[kNSect], ordered keys) as ground_thresholds_kernel derives it.
+__device__ __forceinline__ bool ground_node_keeps(const float4& p, const u32* __restrict__ low_key) {
+  if (!finite3(p.x, p.y, p.z)) return false;
+  bool ok;
+  const float a = atan2_approx(p.y, p.x, ok);
+  const int s = sector_of(p.x, p.y, a, ok);
+  return !(p.z < __double2float_ru((double)ord2f(__ldg(&low_key[s])) + 0.1));
+}
+
+// The zero points the ground node pads frame f's message with: N_f - G_f from the run's cp_frame_counters
+// (fc[8 f] = N, fc[8 f + 1] = G); none without a groundless cloud (fc NULL).
+__device__ __forceinline__ u32 ground_pad(const u32* __restrict__ fc, u32 f) {
+  return fc ? fc[(size_t)f * 8] - fc[(size_t)f * 8 + 1] : 0u;
+}
+
 // mask[k][row] = ballot of "point row*32+lane lies in box k"; tile_count[k][tile] = matches of box k
 // in the 2048-point tile.  Both start from zero (only non-empty rows are written).
 template <int MODE>
 __global__ void __launch_bounds__(kStreamThreads) cone_box_mask_kernel(
     const uint8_t* __restrict__ in, Layout L, u64 first_point, u32 n_points, const __grid_constant__ ConeBoxes B,
-    u32 n_rows, u32 n_tiles, u32* __restrict__ mask, u32* __restrict__ tile_count) {
+    const u32* __restrict__ low_key, u32 n_rows, u32 n_tiles, u32* __restrict__ mask, u32* __restrict__ tile_count) {
   // one 32-point row per warp (a single frame is small: many short CTAs beat 64 long ones)
   const u32 warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const u32 row = blockIdx.x * kStreamWarps + warp;
@@ -56,6 +79,8 @@ __global__ void __launch_bounds__(kStreamThreads) cone_box_mask_kernel(
     if (k < 32) m0 |= (u32)inside << k;
     else m1 |= (u32)inside << (k - 32);
   }
+  // groundless cloud (low_key = the frame's sector minima): only points inside some box need the ground verdict
+  if (low_key && (m0 | m1) && !ground_node_keeps(p, low_key)) m0 = m1 = 0u;
   u32 any0 = __reduce_or_sync(0xFFFFFFFFu, m0), any1 = __reduce_or_sync(0xFFFFFFFFu, m1);
   while (any0 | any1) {
     const bool hi = any0 == 0;
@@ -72,8 +97,10 @@ __global__ void __launch_bounds__(kStreamThreads) cone_box_mask_kernel(
 }
 
 // One CTA.  Warp w scans the tile counts of centres w, w+32 of this chunk; thread 0 then chains the
-// chunk totals onto crop_off (crop_off[k0] was written by the previous chunk, 0 for the first).
-__global__ void __launch_bounds__(1024) cone_box_scan_kernel(u32 n_centers, u32 k0, u32 n_tiles,
+// chunk totals onto crop_off (crop_off[k0] was written by the previous chunk, 0 for the first).  Bit k of `origin`:
+// box k contains (0, 0) and its crop ends with the frame's ground_pad(fc, frame) zero points.
+__global__ void __launch_bounds__(1024) cone_box_scan_kernel(u32 n_centers, u32 k0, u32 n_tiles, u64 origin,
+                                                             const u32* __restrict__ fc, u32 frame,
                                                              const u32* __restrict__ tile_count,
                                                              u32* __restrict__ tile_excl, u32* __restrict__ crop_off) {
   __shared__ u32 total[kConeChunk];
@@ -96,9 +123,10 @@ __global__ void __launch_bounds__(1024) cone_box_scan_kernel(u32 n_centers, u32 
   }
   __syncthreads();
   if (threadIdx.x == 0) {
+    const u32 pad = origin ? ground_pad(fc, frame) : 0u;
     u64 run = crop_off[k0];
     for (u32 k = 0; k < n_centers; ++k) {
-      run += total[k];
+      run += total[k] + (((origin >> k) & 1u) ? pad : 0u);
       crop_off[k0 + k + 1] = run > 0xFFFFFFFFull ? 0xFFFFFFFFu : (u32)run;  // saturates: the host reports capacity
     }
   }
@@ -107,8 +135,9 @@ __global__ void __launch_bounds__(1024) cone_box_scan_kernel(u32 n_centers, u32 
 template <int MODE>
 __global__ void __launch_bounds__(kStreamThreads) cone_box_gather_kernel(
     const uint8_t* __restrict__ in, Layout L, u64 first_point, u32 n_centers, u32 k0, u32 n_rows, u32 n_tiles,
-    const u32* __restrict__ mask, const u32* __restrict__ tile_count, const u32* __restrict__ tile_excl,
-    const u32* __restrict__ crop_off, u32 cap, float4* __restrict__ crop_pts) {
+    u64 origin, const u32* __restrict__ fc, u32 frame, const u32* __restrict__ mask,
+    const u32* __restrict__ tile_count, const u32* __restrict__ tile_excl, const u32* __restrict__ crop_off, u32 cap,
+    float4* __restrict__ crop_pts) {
   const u32 warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const u32 tile = blockIdx.x;
   for (u32 k = 0; k < n_centers; ++k) {
@@ -137,6 +166,17 @@ __global__ void __launch_bounds__(kStreamThreads) cone_box_gather_kernel(
           crop_pts[dst] = load_point<MODE>(in, first_point + idx, L);
         }
       }
+    }
+  }
+  // the padding of the boxes that contain the origin, after their kept points, spread over all CTAs
+  if (origin) {
+    const u32 pad = ground_pad(fc, frame);
+    for (u32 k = 0; k < n_centers; ++k) {
+      if (!((origin >> k) & 1u)) continue;
+      const u64 end = crop_off[k0 + k + 1];
+      for (u64 d = end - pad + (u64)blockIdx.x * blockDim.x + threadIdx.x; d < end && d < cap;
+           d += (u64)gridDim.x * blockDim.x)
+        crop_pts[d] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
   }
 }
@@ -170,18 +210,20 @@ __host__ __device__ inline void extend_center(float x, float y, double ext, floa
 
 // ---- every cluster of a batch run (cp_batch_cone_colors) ---------------------------------
 //   batch_box_kernel     extended centre (src/cone_detection.cpp:276-278) + box bounds + frame of each cluster
+//                        (+ the ground node's padding count of a box that contains the origin)
 //   batch_mark_kernel    one pass over the raw batch: a (cluster, frame row, ballot) triple for every non-empty
 //                        32-point row of every box of the row's frame, sort key cluster << row_bits | row
 //   batch_scan_kernel    crop offsets (points per cluster) and triple offsets (rows per cluster)
 //   (stable radix sort of the triples: cluster-major, rows in cloud order)
-//   batch_gather_kernel  one warp per cluster re-reads its matched rows into the packed crops
+//   batch_gather_kernel  one warp per cluster re-reads its matched rows into the packed crops, then the padding
 // Scratch is O(K + triples); a triple holds at least one crop point, so the crop capacity bounds both.
 // batch ctl words: [0] triples found, [1] live sort-key bits, [2] triples to sort (min(found, capacity))
 constexpr u32 kBatchScanThreads = 1024;
 
 __global__ void __launch_bounds__(256) batch_box_kernel(const ClusterRec* __restrict__ cl, const u32* __restrict__ k_off,
                                                         u32 n_frames, u32 K, double ext, double hw, u32 key_bits,
-                                                        float4* __restrict__ box, u32* __restrict__ kframe,
+                                                        const u32* __restrict__ fc, float4* __restrict__ box,
+                                                        u32* __restrict__ kframe,
                                                         u32* __restrict__ cnt, u32* __restrict__ tcnt, u32* __restrict__ ctl) {
   const u32 k = blockIdx.x * blockDim.x + threadIdx.x;
   if (k == 0) {
@@ -201,7 +243,9 @@ __global__ void __launch_bounds__(256) batch_box_kernel(const ClusterRec* __rest
   box_bounds(ey, hw, &b.z, &b.w);
   box[k] = b;
   kframe[k] = lo;
-  cnt[k] = 0u;
+  // a box that contains (0, 0) ends with the ground node's padding (NaN bounds contain nothing)
+  const bool origin = b.x <= 0.0f && b.y >= 0.0f && b.z <= 0.0f && b.w >= 0.0f;
+  cnt[k] = origin ? ground_pad(fc, lo) : 0u;
   tcnt[k] = 0u;
 }
 
@@ -212,7 +256,8 @@ __device__ __forceinline__ u64 frame_first_point(const Geom& g, u32 f) {
 template <int MODE>
 __global__ void __launch_bounds__(kStreamThreads) batch_mark_kernel(
     const uint8_t* __restrict__ in, Layout L, const Geom g, const u32* __restrict__ k_off,
-    const float4* __restrict__ box, u32 row_bits, u32 cap, u64* __restrict__ keys, u32* __restrict__ vals,
+    const float4* __restrict__ box, const u32* __restrict__ low_key, u32 row_bits, u32 cap, u64* __restrict__ keys,
+    u32* __restrict__ vals,
     u32* __restrict__ cnt, u32* __restrict__ tcnt, u32* __restrict__ ctl) {
   const u32 warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (u32 tile = blockIdx.x; tile < g.n_tiles; tile += gridDim.x) {
@@ -247,6 +292,21 @@ __global__ void __launch_bounds__(kStreamThreads) batch_mark_kernel(
       mny = fminf(mny, __shfl_xor_sync(kFull, mny, d)); mxy = fmaxf(mxy, __shfl_xor_sync(kFull, mxy, d));
     }
     auto misses = [&](const float4& b) { return b.y < mnx || b.x > mxx || b.w < mny || b.z > mxy; };
+    if (low_key) {
+      // groundless cloud: a point in some box stays only if the ground node keeps it (low_key: the run's sector
+      // minima); points in no box are dropped outright, which changes no ballot
+      u32 cand = 0;
+      for (u32 k = kb; k < ke; ++k) {
+        const float4 b = box[k];
+        if (misses(b)) continue;
+#pragma unroll
+        for (int r = 0; r < kStreamRows; ++r) cand |= (u32)inside(r, b) << r;
+      }
+      if (!__any_sync(kFull, cand)) continue;
+#pragma unroll
+      for (int r = 0; r < kStreamRows; ++r)
+        valid[r] = ((cand >> r) & 1u) && ground_node_keeps(p[r], low_key + (size_t)frame * kSectStride);
+    }
     // count the warp's non-empty (box, row) ballots, reserve that many slots with one atomic, then write them
     u32 n = 0;
     for (u32 k = kb; k < ke; ++k) {
@@ -364,6 +424,8 @@ __global__ void __launch_bounds__(256) batch_gather_kernel(
       }
       dst0 += __shfl_sync(kFull, incl, 31);
     }
+    // the ground node's padding (batch_box_kernel counted it): zero points up to the next crop
+    for (u64 d = dst0 + lane; d < off[k + 1] && d < cap; d += 32) crop_pts[d] = make_float4(0.f, 0.f, 0.f, 0.f);
   }
 }
 

@@ -167,6 +167,7 @@ struct cp_handle {
            ans_n = 0, out_n = 0, rec_n = 0, rec_off_n = 0, flags_n = 0, colors_n = 0;
   } track;
   bool tracked = false;  // the current run's frames have advanced the slot state
+  int32_t color_cloud = CP_COLOR_CLOUD_STAGED;  // cp_set_color_cloud: what colour crops are cut from
   const uint8_t* in_ptr = nullptr;  // current batch input (d_in or caller memory)
   Layout layout{};
   HostGeom hg;
@@ -1477,10 +1478,26 @@ cp_status grow(cp_handle* h, T** p, size_t* have, size_t need) {
   return CP_OK;
 }
 
+// Whether a colour-path call on the staged input (cloud NULL) crops from the ground node's message: the handle is
+// set to CP_COLOR_CLOUD_GROUNDLESS and the last run fused ground removal.  The crops then need that run's sector
+// minima and final counters (cp_sync: the back half may be re-run), so the input must not have been staged since.
+static cp_status groundless_crops(cp_handle* h, const cp_cloud_view* cloud, bool* groundless) {
+  *groundless = false;
+  if (cloud || h->color_cloud != CP_COLOR_CLOUD_GROUNDLESS) return CP_OK;
+  if (!h->ran) {
+    h->err = "groundless colour crops need a run on the staged input (none since it was staged)";
+    return CP_E_STATE;
+  }
+  if (!h->rp_has_ground) return CP_OK;
+  *groundless = true;
+  return cp_sync(h);
+}
+
 // Resolves the cloud a colour-path call works on and enqueues the box gather of all centres.
 // On return crop offsets are in h->color.off (device) and the packed crops in h->color.pts.
+// groundless: crop frame `frame` of the staged input as the ground node's message of the last run (color_kernels.cuh).
 cp_status enqueue_cone_crops(cp_handle* h, const cp_cloud_view* cloud, u32 frame, const cp_cone_center* centers,
-                             u32 n_centers, float cone_width, size_t want_cap) {
+                             u32 n_centers, float cone_width, size_t want_cap, bool groundless) {
   if (n_centers && !centers) {
     h->err = "NULL centers";
     return CP_E_PARAM;
@@ -1512,30 +1529,35 @@ cp_status enqueue_cone_crops(cp_handle* h, const cp_cloud_view* cloud, u32 frame
   const u32 cap = (u32)std::min<size_t>(cb.pts_n, 0xFFFFFFFFu);
   CK(cudaMemsetAsync(cb.off, 0, sizeof(u32), h->stream));
   const double hw = (double)cone_width / 1.5;  // CONE_WIDTH / 1.5: float / double literal
+  const u32* low_key = groundless ? h->d_low_key + (size_t)frame * kSectStride : nullptr;
+  const u32* fc = groundless ? h->d_fc : nullptr;
   for (u32 k0 = 0; k0 < n_centers; k0 += kConeChunk) {
     ConeBoxes B;
     memset(&B, 0, sizeof(B));
     B.n = std::min<u32>(kConeChunk, n_centers - k0);
+    u64 origin = 0;  // boxes that hold the ground node's zero padding points
     for (u32 k = 0; k < B.n; ++k) {
       box_bounds(centers[k0 + k].x, hw, &B.xlo[k], &B.xhi[k]);
       box_bounds(centers[k0 + k].y, hw, &B.ylo[k], &B.yhi[k]);
+      if (groundless && B.xlo[k] <= 0.0f && B.xhi[k] >= 0.0f && B.ylo[k] <= 0.0f && B.yhi[k] >= 0.0f)
+        origin |= 1ull << k;
     }
     CK(cudaMemsetAsync(cb.mask, 0, sizeof(u32) * (size_t)B.n * std::max<u32>(n_rows, 1), h->stream));
     CK(cudaMemsetAsync(cb.tcount, 0, sizeof(u32) * (size_t)B.n * n_tiles, h->stream));
     const u32 mgrid = (n_rows + kStreamWarps - 1) / kStreamWarps;
     if (n_points) {
       switch (h->layout.mode) {
-        case 0: cone_box_mask_kernel<0><<<mgrid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, first_point, n_points, B, n_rows, n_tiles, cb.mask, cb.tcount); break;
-        case 1: cone_box_mask_kernel<1><<<mgrid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, first_point, n_points, B, n_rows, n_tiles, cb.mask, cb.tcount); break;
-        default: cone_box_mask_kernel<2><<<mgrid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, first_point, n_points, B, n_rows, n_tiles, cb.mask, cb.tcount); break;
+        case 0: cone_box_mask_kernel<0><<<mgrid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, first_point, n_points, B, low_key, n_rows, n_tiles, cb.mask, cb.tcount); break;
+        case 1: cone_box_mask_kernel<1><<<mgrid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, first_point, n_points, B, low_key, n_rows, n_tiles, cb.mask, cb.tcount); break;
+        default: cone_box_mask_kernel<2><<<mgrid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, first_point, n_points, B, low_key, n_rows, n_tiles, cb.mask, cb.tcount); break;
       }
     }
-    cone_box_scan_kernel<<<1, 1024, 0, h->stream>>>(B.n, k0, n_tiles, cb.tcount, cb.texcl, cb.off);
+    cone_box_scan_kernel<<<1, 1024, 0, h->stream>>>(B.n, k0, n_tiles, origin, fc, frame, cb.tcount, cb.texcl, cb.off);
     if (n_points) {
       switch (h->layout.mode) {
-        case 0: cone_box_gather_kernel<0><<<n_tiles, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, first_point, B.n, k0, n_rows, n_tiles, cb.mask, cb.tcount, cb.texcl, cb.off, cap, cb.pts); break;
-        case 1: cone_box_gather_kernel<1><<<n_tiles, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, first_point, B.n, k0, n_rows, n_tiles, cb.mask, cb.tcount, cb.texcl, cb.off, cap, cb.pts); break;
-        default: cone_box_gather_kernel<2><<<n_tiles, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, first_point, B.n, k0, n_rows, n_tiles, cb.mask, cb.tcount, cb.texcl, cb.off, cap, cb.pts); break;
+        case 0: cone_box_gather_kernel<0><<<n_tiles, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, first_point, B.n, k0, n_rows, n_tiles, origin, fc, frame, cb.mask, cb.tcount, cb.texcl, cb.off, cap, cb.pts); break;
+        case 1: cone_box_gather_kernel<1><<<n_tiles, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, first_point, B.n, k0, n_rows, n_tiles, origin, fc, frame, cb.mask, cb.tcount, cb.texcl, cb.off, cap, cb.pts); break;
+        default: cone_box_gather_kernel<2><<<n_tiles, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, first_point, B.n, k0, n_rows, n_tiles, origin, fc, frame, cb.mask, cb.tcount, cb.texcl, cb.off, cap, cb.pts); break;
       }
     }
   }
@@ -1620,20 +1642,22 @@ static cp_status enqueue_color_net(cp_handle* h, const uint8_t* images_dev, cons
   return CP_OK;
 }
 
-// cp_batch_cone_colors: crops of every cluster of the run, straight from the run's raw input (color_kernels.cuh).
+// cp_batch_cone_colors: crops of every cluster of the run, straight from the run's raw input (color_kernels.cuh),
+// or from the ground node's messages of the run (groundless).
 // Returns the kernel launches; on return the crop offsets are in color.off and the crops in color.pts.
 template <int MODE>
 static u32 enqueue_batch_crops(cp_handle* h, u32 K, double ext, double hw, u32 row_bits, u32 key_bits,
-                               u32 max_key_bits) {
+                               u32 max_key_bits, bool groundless) {
   cp_handle::ColorBufs& cb = h->color;
   const u32 cap = (u32)std::min<size_t>(cb.pts_n, 0xFFFFFFFFu);
   const Geom g = device_geom(h);
   batch_box_kernel<<<(K + 255) / 256, 256, 0, h->stream>>>(h->d_clusters, h->d_k_off, g.n_frames, K, ext, hw,
-                                                           key_bits, cb.box, cb.kframe, cb.cnt, cb.tcnt, cb.bctl);
+                                                           key_bits, groundless ? h->d_fc : nullptr, cb.box,
+                                                           cb.kframe, cb.cnt, cb.tcnt, cb.bctl);
   const u32 mgrid = std::max<u32>(1, std::min<u32>(g.n_tiles, (u32)h->sms * (u32)h->stream_ctas_per_sm));
   batch_mark_kernel<MODE><<<mgrid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, g, h->d_k_off, cb.box,
-                                                                   row_bits, cap, cb.keys_a, cb.vals_a, cb.cnt,
-                                                                   cb.tcnt, cb.bctl);
+                                                                   groundless ? h->d_low_key : nullptr, row_bits, cap,
+                                                                   cb.keys_a, cb.vals_a, cb.cnt, cb.tcnt, cb.bctl);
   batch_scan_kernel<<<1, kBatchScanThreads, 0, h->stream>>>(K, cb.cnt, cb.tcnt, cb.off, cb.toff, cap, cb.bctl);
   SortArgs sa;
   sa.keys_a = cb.keys_a;
@@ -2815,9 +2839,11 @@ cp_status cp_cone_crops(cp_handle* h, const cp_cloud_view* cloud, uint32_t frame
     return CP_E_PARAM;
   }
   CK(cudaSetDevice(h->cfg.device));
-  cp_status st = color_pin(h, n_centers);
+  bool groundless;
+  cp_status st = groundless_crops(h, cloud, &groundless);
   if (st) return st;
-  st = enqueue_cone_crops(h, cloud, frame, centers, n_centers, cone_width, crop_xyzi ? cap_points : 0);
+  if ((st = color_pin(h, n_centers))) return st;
+  st = enqueue_cone_crops(h, cloud, frame, centers, n_centers, cone_width, crop_xyzi ? cap_points : 0, groundless);
   if (st) return st;
   CK(cudaMemcpyAsync(pin_off(h), h->color.off, sizeof(u32) * ((size_t)n_centers + 1), cudaMemcpyDeviceToHost, h->stream));
   // the first crop points ride along speculatively: a typical frame's crops fit, so one synchronisation serves
@@ -2851,14 +2877,16 @@ cp_status cp_cone_images(cp_handle* h, const cp_cloud_view* cloud, uint32_t fram
     return CP_E_PARAM;
   }
   CK(cudaSetDevice(h->cfg.device));
-  cp_status st = color_pin(h, n_centers);
+  bool groundless;
+  cp_status st = groundless_crops(h, cloud, &groundless);
   if (st) return st;
+  if ((st = color_pin(h, n_centers))) return st;
   size_t want = h->color.pts_n;
   for (int attempt = 0; attempt < 2; ++attempt) {
     // the cloud is staged by the first attempt only; a retry (crop buffer too small) reuses it.
     // Crops, raster and the copies go out back to back; the crop total is checked after the one sync.
     st = enqueue_cone_crops(h, attempt == 0 ? cloud : nullptr, attempt == 0 ? frame : (cloud ? 0 : frame), centers,
-                            n_centers, cone_width, want);
+                            n_centers, cone_width, want, groundless);
     if (st) return st;
     if ((st = enqueue_raster(h, n_centers))) return st;
     CK(cudaMemcpyAsync(pin_off(h), h->color.off, sizeof(u32) * ((size_t)n_centers + 1), cudaMemcpyDeviceToHost, h->stream));
@@ -3004,13 +3032,15 @@ cp_status cp_cone_colors(cp_handle* h, const cp_cloud_view* cloud, uint32_t fram
     return CP_E_STATE;
   }
   CK(cudaSetDevice(h->cfg.device));
-  cp_status st = color_pin(h, n_centers);
+  bool groundless;
+  cp_status st = groundless_crops(h, cloud, &groundless);
   if (st) return st;
+  if ((st = color_pin(h, n_centers))) return st;
   size_t want = h->color.pts_n;
   for (int attempt = 0; attempt < 2; ++attempt) {
     // crops -> range images -> classifier, back to back on the stream; one synchronisation, n_centers bytes back
     st = enqueue_cone_crops(h, attempt == 0 ? cloud : nullptr, attempt == 0 ? frame : (cloud ? 0 : frame), centers,
-                            n_centers, cone_width, want);
+                            n_centers, cone_width, want, groundless);
     if (st) return st;
     if ((st = enqueue_raster(h, n_centers))) return st;
     if ((st = enqueue_color_net(h, h->color.img, h->color.flags, n_centers))) return st;
@@ -3036,6 +3066,8 @@ static cp_status batch_colors(cp_handle* h, float cone_width, double extension_l
                               float* probs, uint32_t* flags) {
   cp_status st;
   u32 max_rows = 0;
+  // the ground node's messages of the run (cp_set_color_cloud); the caller has synchronised the run
+  const bool groundless = h->color_cloud == CP_COLOR_CLOUD_GROUNDLESS && h->rp_has_ground;
 
   for (u32 n : h->hg.frame_n) max_rows = std::max(max_rows, (n + 31) / 32);
   const u32 row_bits = ceil_log2_host(max_rows);
@@ -3062,9 +3094,9 @@ static cp_status batch_colors(cp_handle* h, float cone_width, double extension_l
     if ((st = grow(h, &cb.vals_b, &cb.vals_b_n, cb.pts_n))) return st;
     if ((st = grow(h, &cb.sort_state, &cb.sort_state_n, 2 * kRadix * (cb.pts_n / kSortTile + 1)))) return st;
     switch (h->layout.mode) {
-      case 0: h->launches += enqueue_batch_crops<0>(h, K, extension_length, hw, row_bits, key_bits, max_key_bits); break;
-      case 1: h->launches += enqueue_batch_crops<1>(h, K, extension_length, hw, row_bits, key_bits, max_key_bits); break;
-      default: h->launches += enqueue_batch_crops<2>(h, K, extension_length, hw, row_bits, key_bits, max_key_bits); break;
+      case 0: h->launches += enqueue_batch_crops<0>(h, K, extension_length, hw, row_bits, key_bits, max_key_bits, groundless); break;
+      case 1: h->launches += enqueue_batch_crops<1>(h, K, extension_length, hw, row_bits, key_bits, max_key_bits, groundless); break;
+      default: h->launches += enqueue_batch_crops<2>(h, K, extension_length, hw, row_bits, key_bits, max_key_bits, groundless); break;
     }
     CK(cudaGetLastError());
     if ((st = enqueue_raster(h, K))) return st;
@@ -3086,6 +3118,18 @@ static cp_status batch_colors(cp_handle* h, float cone_width, double extension_l
     want = total;
   }
   return CP_OK;
+}
+
+cp_status cp_set_color_cloud(cp_handle* h, int32_t cloud) try {
+  if (!h) return CP_E_PARAM;
+  if (cloud != CP_COLOR_CLOUD_STAGED && cloud != CP_COLOR_CLOUD_GROUNDLESS) {
+    h->err = "cloud must be CP_COLOR_CLOUD_STAGED or CP_COLOR_CLOUD_GROUNDLESS";
+    return CP_E_PARAM;
+  }
+  h->color_cloud = cloud;
+  return CP_OK;
+} catch (...) {
+  return abi_exception(h);
 }
 
 cp_status cp_batch_cone_colors(cp_handle* h, float cone_width, double extension_length, uint8_t* colors, float* probs,

@@ -214,6 +214,10 @@ int ch_detector_load_color_model(void* dp, const void* model, uint64_t bytes) {
     return 4;
   }
 }
+// ConeDetector::groundless_color_crops
+void ch_detector_set_groundless_color_crops(void* dp, int on) {
+  static_cast<ConeDetector*>(dp)->groundless_color_crops = on != 0;
+}
 void ch_detector_color_probe(void* dp, uint64_t* n_inputs, uint64_t* n_points, uint64_t* digest) {
   const ColorProbe& pr = g_probes[dp];
   *n_inputs = pr.n_inputs;

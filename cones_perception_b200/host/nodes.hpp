@@ -276,9 +276,15 @@ class ConeDetector {
   std::string input_cloud_topic = "/cloud";
   std::string cones_topics[kNumberOfColors] = {"cones_cloud_unknowns", "cones_cloud_yellows", "cones_cloud_blues",
                                                "cones_cloud_oranges"};
-  // not in the reference: fuse the ground_removal node in front (one process, one H2D copy);
-  // equals running the two nodes chained through the groundless_cloud topic
+  // not in the reference: fuse the ground_removal node in front (one process, one H2D copy).  The cluster records
+  // equal those of the two nodes chained through the groundless_cloud topic; the colour crops equal the chain's only
+  // with groundless_color_crops (otherwise they are cut from the raw cloud, ground returns included)
   bool fused_ground_removal = false;
+  // not in the reference: with fused_ground_removal, cut the colour crops from the ground node's message, as the
+  // chained detector does (cp_set_color_cloud(CP_COLOR_CLOUD_GROUNDLESS)); clouds are then staged as the ground node
+  // reads them (intensity 0 without an intensity field).  No effect without fused_ground_removal.  kHostCrops holds
+  // no groundless cloud on the host and refuses it.
+  bool groundless_color_crops = false;
   int num_of_sectors = 16;
   float default_lowest_point = -0.1f;
   std::function<std::vector<Color>(const std::vector<std::vector<Point>>&)> get_colors;
@@ -340,7 +346,8 @@ class ConeDetector {
                        voxel_filter_leaf_size_x, voxel_filter_leaf_size_y, voxel_filter_leaf_size_z,
                        min_cluster_size, max_cluster_size, CONE_WIDTH, CONE_HEIGHT};
     cp_ground_params g{num_of_sectors, default_lowest_point};
-    cp_cloud_view in = make_view(cloud_msg, !intensity_in_cloud_);
+    set_color_cloud();
+    cp_cloud_view in = make_view(cloud_msg, !intensity_in_cloud_ && !groundless());
     clusters_.resize(4096);
     uint32_t n = 0;
     cp_status st = cp_detect(gpu_, &in, &d, fused_ground_removal ? &g : nullptr, clusters_.data(),
@@ -390,6 +397,7 @@ class ConeDetector {
     use_entry(kReplay);
     if (classify_colors && color_inputs != kGpuColors)
       throw GpuError(CP_E_PARAM, "replay classifies colours with the device net only (load_color_model)");
+    set_color_cloud();
     std::vector<std::vector<PointCloud2>> out;
     out.reserve(msgs.size());
     size_t i = 0;
@@ -403,7 +411,7 @@ class ConeDetector {
       for (; i < msgs.size() && views.size() < max_frames_; ++i) {
         const uint64_t n = static_cast<uint64_t>(msgs[i].width) * msgs[i].height;
         if (!views.empty() && pts + n > max_points_) break;
-        views.push_back(make_view(msgs[i], !intensity_in_cloud_));
+        views.push_back(make_view(msgs[i], !intensity_in_cloud_ && !groundless()));
         pts += n;
       }
       replay_batch(msgs, i - views.size(), views, &out);
@@ -414,6 +422,14 @@ class ConeDetector {
   const std::vector<cp_cluster>& last_clusters() const { return clusters_; }
 
  private:
+  bool groundless() const { return fused_ground_removal && groundless_color_crops; }
+  void set_color_cloud() {
+    if (groundless() && classify_colors && color_inputs == kHostCrops)
+      throw GpuError(CP_E_PARAM, "groundless_color_crops needs the device crops (kGpuCrops, kGpuImages, kGpuColors): "
+                                 "kHostCrops has no groundless cloud on the host");
+    cp_status st = cp_set_color_cloud(gpu_, groundless() ? CP_COLOR_CLOUD_GROUNDLESS : CP_COLOR_CLOUD_STAGED);
+    if (st != CP_OK) throw GpuError(st, cp_last_error(gpu_));
+  }
   static std::vector<Point> from_msg(const PointCloud2& m, const cp_cloud_view& v) {
     std::vector<Point> out(static_cast<size_t>(m.width) * m.height);
     for (uint32_t r = 0; r < m.height; ++r)

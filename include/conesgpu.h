@@ -276,7 +276,9 @@ enum {
  * pass: the points of the raw cloud with |x-cx| <= CONE_WIDTH/1.5 and |y-cy| <= CONE_WIDTH/1.5 (the reference's
  * double-precision comparisons, both ends inclusive), in cloud order.
  *   cloud: the raw cloud, or NULL to use frame `frame` of the input already on the device (the cloud the last
- *          cp_detect / cp_batch_set_*_input call of this handle staged) — no second host-to-device copy.
+ *          cp_detect / cp_batch_set_*_input call of this handle staged) — no second host-to-device copy.  With
+ *          cp_set_color_cloud(h, CP_COLOR_CLOUD_GROUNDLESS) and a last run that fused ground removal, NULL crops
+ *          that frame's ground-node message instead (see cp_set_color_cloud).
  *   crop_offsets[n_centers+1]: cone c owns crop_xyzi[4*crop_offsets[c] .. 4*crop_offsets[c+1]).
  *   crop_xyzi: x, y, z, intensity per point (cap_points points); NULL to get the offsets only.
  * CP_E_CAPACITY if the crops hold more than cap_points points (crop_offsets is still complete). */
@@ -326,7 +328,8 @@ cp_status cp_cone_colors(cp_handle* h, const cp_cloud_view* cloud, uint32_t fram
  * (scripts/color_classifier_server.py:78-126) for EVERY cluster record of the run, entirely on the device.
  * Cluster k (the k-th record cp_batch_results returns, frame-major, canonical order) is classified at its
  * centroid moved radially by extension_length (src/cone_detection.cpp:276-278, restated exactly), using the
- * raw cloud of its own frame from the run's staged input.  One pass over the batch finds every crop.
+ * raw cloud of its own frame from the run's staged input (or, with CP_COLOR_CLOUD_GROUNDLESS after a run with
+ * ground removal, that frame's ground-node message: cp_set_color_cloud).  One pass over the batch finds every crop.
  *   colors[k]: 0 unknown, 1 yellow, 2 blue, 3 orange, 255 no answer (as cp_cone_colors)
  *   probs  (optional) [K][n_classes], flags (optional) CP_CONE_* bits, counts (optional) crop points per cluster.
  * The output is per cluster: the service's response rules (a shorter response when a crop is empty, a failed
@@ -339,6 +342,21 @@ cp_status cp_cone_colors(cp_handle* h, const cp_cloud_view* cloud, uint32_t fram
  * CP_E_CAPACITY: cap < number of clusters. */
 cp_status cp_batch_cone_colors(cp_handle* h, float cone_width, double extension_length, uint8_t* colors,
                                float* probs, uint32_t* flags, uint32_t* counts, uint64_t cap);
+/* Which cloud colour crops of the staged input are cut from: cp_cone_crops / cp_cone_images / cp_cone_colors with
+ * cloud NULL, cp_batch_cone_colors and cp_batch_track in colour mode.  An explicit cloud argument is used as given.
+ *   CP_COLOR_CLOUD_STAGED (the default): the staged cloud itself.
+ *   CP_COLOR_CLOUD_GROUNDLESS: when the last run fused ground removal (cp_detect, cp_batch_run or cp_detect_batch
+ *     with non-NULL ground), frame f is cropped from the message the ground node publishes for it
+ *     (src/ground_removal.cpp:54-79): the points its filter keeps, in input order, then N_f - G_f points (0, 0, 0,
+ *     intensity 0).  That is what cp_batch_ground_remove writes for the frame, so the crops, images and colours equal
+ *     those of the reference's two-node launch (ground_removal:=true), where the detector crops from the
+ *     groundless_cloud message.  Intensities are what the staged view reads: stage clouds without an intensity
+ *     field with off_intensity < 0, as the ground node reads them.  After a run without ground removal the output
+ *     is the same as with CP_COLOR_CLOUD_STAGED.
+ * CP_E_PARAM: any other value.  The colour calls then return CP_E_STATE with CP_COLOR_CLOUD_GROUNDLESS and cloud
+ * NULL when no run has been made on the staged input (the sector minima would belong to another input). */
+enum { CP_COLOR_CLOUD_STAGED = 0, CP_COLOR_CLOUD_GROUNDLESS = 1 };
+cp_status cp_set_color_cloud(cp_handle* h, int32_t cloud);
 /* --- what the cone-detection node publishes, over frame sequences (src/cone_detection.cpp:276-340) ---------------
  * After a run (cp_batch_run, cp_detect_batch or cp_detect): the radial extension, the temporal gate / points buffer,
  * the colour carry-over from the previous frame's colour clouds, the colour service's response rules and the four
@@ -351,8 +369,8 @@ cp_status cp_batch_cone_colors(cp_handle* h, float cone_width, double extension_
  *   out: the published cones, frame-major, then by cloud 0..3 (unknown, yellow, blue, orange); within a cloud the
  *     node's push_back order (cones with a carried colour in record order, then the cones that needed a colour).
  *   cloud_offsets[4 * n_frames + 1]: cloud c of frame f is out[cloud_offsets[4 f + c] .. cloud_offsets[4 f + c + 1]).
- * Colour mode (classify_colors != 0) classifies every record on the device (the chain of cp_batch_cone_colors, needs
- * a loaded net) and applies the service's response rules to each frame's need list: a bad crop (CP_CONE_BAD_*) leaves
+ * Colour mode (classify_colors != 0) classifies every record on the device (the chain of cp_batch_cone_colors, on the
+ * cloud cp_set_color_cloud selects; needs a loaded net) and applies the service's response rules to each frame's need list: a bad crop (CP_CONE_BAD_*) leaves
  * every needed cone unknown; otherwise the answers of the non-empty crops fill the need list from the front.
  * Calls cp_sync first and leaves the run's results untouched.  No slot changes on any error.
  * CP_E_PARAM: non-finite threshold or extension length, cone_width not positive and finite in colour mode, n_seqs

@@ -30,6 +30,9 @@ class ConeDetectorNode {
     private_param("fused_ground_removal", core_.fused_ground_removal);
     private_param("num_of_sectors", core_.num_of_sectors);
     private_param("default_lowest_point", core_.default_lowest_point);
+    // extension (off by default): with fused_ground_removal, colour crops from the ground node's message, as the
+    // detector of the two-node launch cuts them
+    private_param("groundless_color_crops", core_.groundless_color_crops);
     // extension (off by default): the classifier network on the device instead of the color_classifier service;
     // the value is what the reference's launch file passes to the Python service as ~model_path
     std::string color_model_path;
