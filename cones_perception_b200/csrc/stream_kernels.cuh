@@ -318,22 +318,27 @@ __device__ __forceinline__ void sector_min_tile(const float4 (&p)[kStreamRows], 
   }
 }
 
+// The streaming pass 1 keeps the CTA's shared table but no per-tile barrier: each warp takes its prefilter
+// bounds from the table on its own, once per tile.  Other warps may lower entries at any time, so a warp's
+// bounds can be stale, but only ever too high: a stale bound lets more points through to the exact
+// `zk < smin[s]` test and cannot change a minimum.  On top of the per-point quadrant bound, a row whose lowest
+// key is not below the all-sector bound is dropped whole (one redux next to the one rowmax needs anyway).
 template <int MODE>
 __global__ void __launch_bounds__(kStreamThreads, 4)
 ground_sector_min_kernel(const uint8_t* __restrict__ in, Layout L, Geom g, u32* __restrict__ low_key,
                          u32* __restrict__ rowmax) {
   __shared__ u32 smin[kSectStride];
-  __shared__ u32 s_bound[5];
   // contiguous chunk of tiles per CTA so the shared table is flushed once per frame change
   const u32 per = (g.n_tiles + gridDim.x - 1) / gridDim.x;
   const u32 t0 = blockIdx.x * per;
   const u32 t1 = t0 + per < g.n_tiles ? t0 + per : g.n_tiles;
+  const int lane = lane_id();
   u32 cur_frame = 0xFFFFFFFFu;
   for (u32 tile = t0; tile < t1; ++tile) {
     u32 frame, local0, count;
     u64 first;
     tile_lookup(g, tile, frame, local0, count, first);
-    if (frame != cur_frame) {
+    if (frame != cur_frame) {  // CTA-uniform: every warp walks the same tiles
       __syncthreads();
       if (cur_frame != 0xFFFFFFFFu && threadIdx.x < kNSect)
         atomicMin(&low_key[cur_frame * kSectStride + threadIdx.x], smin[threadIdx.x]);
@@ -341,24 +346,39 @@ ground_sector_min_kernel(const uint8_t* __restrict__ in, Layout L, Geom g, u32* 
       if (threadIdx.x < kSectStride)
         smin[threadIdx.x] = threadIdx.x < kNSect ? __ldcg(&low_key[frame * kSectStride + threadIdx.x]) : 0u;
       cur_frame = frame;
+      __syncthreads();
     }
-    __syncthreads();
-    sector_bounds(smin, s_bound);
     float4 p[kStreamRows];
     load_tile<MODE>(in, L, first + local0, count, __int_as_float(0x7f800000), p);
-    sector_min_tile(p, smin, s_bound);
-    // highest z of every 32-point row (as an ordered key): pass 2 skips rows that lie entirely
-    // below the lowest ground threshold without reading them
-    if (rowmax) {
-      u32 mine = 0;
+    // quadrant q = 1 + (x<0) + 2*(y<0) reaches sectors {0..4}, {4..8}, {12..16}, {8..12}
+    const u32 v = lane < kNSect ? *(volatile const u32*)&smin[lane] : 0u;
+    const u32 ball = __reduce_max_sync(kFull, v);
+    const u32 b1 = __reduce_max_sync(kFull, lane <= 4 ? v : 0u);
+    const u32 b2 = __reduce_max_sync(kFull, (lane >= 4 && lane <= 8) ? v : 0u);
+    const u32 b3 = __reduce_max_sync(kFull, (lane >= 12 && lane <= 16) ? v : 0u);
+    const u32 b4 = __reduce_max_sync(kFull, (lane >= 8 && lane <= 12) ? v : 0u);
+    u32 mine = 0;
 #pragma unroll
-      for (int r = 0; r < kStreamRows; ++r) {
-        const u32 m = __reduce_max_sync(kFull, f2ord(p[r].z));
-        if (lane_id() == r) mine = m;
+    for (int r = 0; r < kStreamRows; ++r) {
+      // out-of-range lanes carry z = +inf: a key above every bound
+      const u32 zk = f2ord(p[r].z);
+      if (__reduce_min_sync(kFull, zk) < ball) {
+        const float x = p[r].x, y = p[r].y;
+        // points on an axis (or with a vanishing product) use the all-sector bound
+        const u32 bq = (x * y == 0.0f) ? ball : (y < 0.0f ? (x < 0.0f ? b4 : b3) : (x < 0.0f ? b2 : b1));
+        if (zk < bq && finite3(x, y, p[r].z)) {
+          bool ok;
+          const float a = atan2_approx(y, x, ok);
+          const int s = sector_of(x, y, a, ok);
+          if (zk < smin[s]) atomicMin(&smin[s], zk);   // src/ground_removal.cpp:65-67
+        }
       }
-      if (lane_id() < kStreamRows)
-        rowmax[(u64)tile * kTileWords + (threadIdx.x >> 5) * kStreamRows + lane_id()] = mine;
+      // highest z of every 32-point row (as an ordered key): pass 2 skips rows that lie entirely
+      // below the lowest ground threshold without reading them
+      const u32 m = __reduce_max_sync(kFull, zk);
+      if (lane == r) mine = m;
     }
+    if (rowmax && lane < kStreamRows) rowmax[(u64)tile * kTileWords + (threadIdx.x >> 5) * kStreamRows + lane] = mine;
   }
   __syncthreads();
   if (cur_frame != 0xFFFFFFFFu && threadIdx.x < kNSect)
