@@ -19,7 +19,7 @@ LIB_PATH = os.path.join(_HERE, "_lib", "libconesgpu.so")
 CP_OK, CP_E_PARAM, CP_E_BADFIELD, CP_E_CAPACITY, CP_E_CUDA, CP_E_NOMEM, CP_E_STATE = range(7)
 
 TAP_SECTOR_LOW, TAP_CROP_INDEX, TAP_CROP_POINTS, TAP_CROP_OFFSETS, TAP_VOXEL_KEYS, TAP_VOXEL_ORDER, \
-    TAP_VOXEL_CLOUD, TAP_VOXEL_OFFSETS, TAP_LABELS = range(9)
+    TAP_VOXEL_CLOUD, TAP_VOXEL_OFFSETS, TAP_LABELS, TAP_PLANE_HYPOTHESES, TAP_PLANE_COUNTS = range(11)
 
 # every symbol include/conesgpu.h declares
 ABI_SYMBOLS = [
@@ -33,6 +33,7 @@ ABI_SYMBOLS = [
     "cp_color_net_load", "cp_color_net_load_tflite", "cp_cone_colors", "cp_classify_images",
     "cp_batch_cone_colors", "cp_batch_track", "cp_track_reset", "cp_debug_track",
     "cp_batch_ground_remove", "cp_batch_ground_device_output", "cp_set_color_cloud",
+    "cp_set_ground_plane", "cp_ground_planes",
 ]
 
 CONE_IMG_ROWS, CONE_IMG_COLS = 15, 12
@@ -72,6 +73,17 @@ def track_params(classify_colors=False, use_points_buffer=False, match=0.5, ext=
 class CTrackedCone(C.Structure):
     """cp_tracked_cone."""
     _fields_ = [("x", C.c_float), ("y", C.c_float), ("cluster", C.c_uint32), ("color", C.c_uint32)]
+
+
+class CPlaneParams(C.Structure):
+    """cp_plane_params: the plane ground model (cp_set_ground_plane).  PARITY UNPINNED: the reference has none."""
+    _fields_ = [("seed", C.c_uint64), ("n_hypotheses", C.c_uint32), ("inlier_distance", C.c_float),
+                ("ground_height", C.c_float), ("max_tilt_deg", C.c_float)]
+
+
+def plane_params(seed=0, n_hypotheses=64, inlier_distance=0.1, ground_height=0.1, max_tilt_deg=15.0) -> CPlaneParams:
+    """cp_plane_params from keywords (anything with these attribute names also works with set_ground_plane)."""
+    return CPlaneParams(int(seed), int(n_hypotheses), float(inlier_distance), float(ground_height), float(max_tilt_deg))
 
 
 class ConesGpuError(RuntimeError):
@@ -152,6 +164,8 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.cp_batch_ground_remove.argtypes = [vp, C.POINTER(CGroundParams), vp, u64, vp, vp]
     lib.cp_batch_ground_device_output.argtypes = [vp, C.POINTER(vp), C.POINTER(u64)]
     lib.cp_set_color_cloud.argtypes = [vp, C.c_int32]
+    lib.cp_set_ground_plane.argtypes = [vp, C.POINTER(CPlaneParams)]
+    lib.cp_ground_planes.argtypes = [vp, vp, vp, vp, u32]
     lib.cp_pinned_alloc.argtypes = [C.c_int32, C.c_size_t, C.c_int32, C.POINTER(vp)]
     lib.cp_pinned_free.argtypes = [vp]
     lib.cp_pinned_free.restype = None
@@ -245,7 +259,7 @@ class ConesGpu:
     # ---- node-equivalent calls --------------------------------------------------------
     def ground_remove(self, msg: PointCloud2, g: GroundParams, copy: bool = True):
         """GroundRemover::cloud_handler body (src/ground_removal.cpp:54-79).
-        Returns (cloud32 [N,8] float32 in PCL layout, n_kept, low17)."""
+        Returns (cloud32 [N,8] float32 in PCL layout, n_kept, low17; low17 None under the plane model)."""
         view = make_view(msg, fake_missing_intensity=False)
         n = msg.n_points
         if getattr(self, "_gr_n", None) != n:            # the output buffer is reused between calls (a node
@@ -255,10 +269,11 @@ class ConesGpu:
         low = np.empty(17, dtype=np.float32)
         kept = C.c_uint32()
         cg = to_c_ground(g)
+        plane = getattr(self, "_plane", False)
         self._ck(self.lib.cp_ground_remove(self._h, C.byref(view), C.byref(cg), out.ctypes.data, C.byref(kept),
-                                           low.ctypes.data))
+                                           None if plane else low.ctypes.data))
         self.n_frames, self.n_points = 1, n   # the frame stays staged
-        return out.copy() if copy else out, kept.value, low
+        return out.copy() if copy else out, kept.value, None if plane else low
 
     def detect(self, msg: PointCloud2, d: DetectParams, g: GroundParams | None = None, cap: int = 4096,
                fake_missing_intensity: bool = True):
@@ -443,20 +458,44 @@ class ConesGpu:
         """GroundRemover::cloud_handler (src/ground_removal.cpp:54-79) for every frame of the staged batch (stage host
         clouds with fake_missing_intensity=False, as the ground node reads them).  Returns (cloud32 [sum N_f, 8]
         float32, frame f's message at rows P_f .. P_f + N_f, or None when host is False; n_kept u32 [F];
-        low f32 [F, 17]).  The messages stay on the device: ground_device_output()."""
+        low f32 [F, 17], None under the plane model).  The messages stay on the device: ground_device_output()."""
+        plane = getattr(self, "_plane", False)
         out = np.empty((self.n_points, 8), np.float32) if host else None
         kept = np.zeros(self.n_frames, np.uint32)
         low = np.zeros((self.n_frames, 17), np.float32)
         cg = to_c_ground(g)
         self._ck(self.lib.cp_batch_ground_remove(self._h, C.byref(cg), out.ctypes.data if host else None,
-                                                 self.n_points if host else 0, kept.ctypes.data, low.ctypes.data))
-        return out, kept, low
+                                                 self.n_points if host else 0, kept.ctypes.data,
+                                                 None if plane else low.ctypes.data))
+        return out, kept, None if plane else low
 
     def ground_device_output(self):
         """(device pointer, n_points) of the messages of the last batch_ground_remove (32 B per point)."""
         p, n = C.c_void_p(), C.c_uint64()
         self._ck(self.lib.cp_batch_ground_device_output(self._h, C.byref(p), C.byref(n)))
         return p.value, n.value
+
+    def set_ground_plane(self, p=None):
+        """The plane ground model (cp_set_ground_plane) for every later call with ground params, or the sector model
+        (the default) with p None.  p: a CPlaneParams or anything with its field names (oracle.plane_oracle.PlaneParams)."""
+        if p is None:
+            self._ck(self.lib.cp_set_ground_plane(self._h, None))
+            self._plane = False
+            return
+        c = p if isinstance(p, CPlaneParams) else plane_params(p.seed, p.n_hypotheses, p.inlier_distance,
+                                                                 p.ground_height, p.max_tilt_deg)
+        self._ck(self.lib.cp_set_ground_plane(self._h, C.byref(c)))
+        self._plane = True
+
+    def ground_planes(self):
+        """The plane each frame chose in the last run or ground call with the plane model: (planes f32 [F, 4] a, b, c, d,
+        inliers u32 [F], hypothesis i32 [F], -1 where no hypothesis was valid)."""
+        F = self.n_frames
+        planes = np.zeros((F, 4), np.float32)
+        inl = np.zeros(F, np.uint32)
+        hyp = np.zeros(F, np.int32)
+        self._ck(self.lib.cp_ground_planes(self._h, planes.ctypes.data, inl.ctypes.data, hyp.ctypes.data, F))
+        return planes, inl, hyp
 
     def run(self, d: DetectParams, g: GroundParams | None = None):
         cd = to_c_detect(d)
@@ -557,9 +596,11 @@ class ConesGpu:
     # ---- parity taps ------------------------------------------------------------------
     def tap(self, which: int) -> np.ndarray:
         dt = {TAP_SECTOR_LOW: np.float32, TAP_CROP_POINTS: np.float32, TAP_VOXEL_CLOUD: np.float32,
-              TAP_LABELS: np.int32}.get(which, np.uint32)
-        width = 4 if which in (TAP_CROP_POINTS, TAP_VOXEL_CLOUD) else 1
+              TAP_LABELS: np.int32, TAP_PLANE_HYPOTHESES: np.float32}.get(which, np.uint32)
+        width = 4 if which in (TAP_CROP_POINTS, TAP_VOXEL_CLOUD, TAP_PLANE_HYPOTHESES) else 1
         cap = (self.max_points + self.max_frames + 64) * max(1, width) * 4 + self.max_frames * 17 * 4
+        if which in (TAP_PLANE_HYPOTHESES, TAP_PLANE_COUNTS):
+            cap = self.max_frames * 256 * width * 4
         buf = np.empty(cap // 4, dtype=dt)
         n = C.c_uint64()
         self._ck(self.lib.cp_debug_tap(self._h, which, buf.ctypes.data, buf.nbytes, C.byref(n)))

@@ -21,6 +21,7 @@
 #include "common.cuh"
 #include "copy_pool.hpp"
 #include "frame_kernels.cuh"
+#include "plane_kernels.cuh"
 #include "radix_sort.cuh"
 #include "single_frame.cuh"
 #include "stream_kernels.cuh"
@@ -89,7 +90,8 @@ struct cp_handle {
   bool use_graph = true, capturing = false, key_valid = false, graph_key_valid = false;
   cudaGraphExec_t graph_exec = nullptr;
   u32 graph_launches = 0;
-  alignas(8) unsigned char last_key[192], graph_key[192];
+  bool graph_plane_run = false;  // the captured run was the plane chain (replays restore the run state below)
+  alignas(8) unsigned char last_key[224], graph_key[224];
   // peer-memory gather of the result block (multi-GPU result path)
   struct {
     bool open = false, owner = false;
@@ -170,6 +172,18 @@ struct cp_handle {
   int32_t color_cloud = CP_COLOR_CLOUD_STAGED;  // cp_set_color_cloud: what colour crops are cut from
   const uint8_t* in_ptr = nullptr;  // current batch input (d_in or caller memory)
   Layout layout{};
+  // what the run (or ground call) in flight reads: the staged input, or under the plane model the plane ground node's
+  // messages in d_out32 (the colour paths always read the staged input)
+  const uint8_t* run_in = nullptr;
+  Layout run_layout{};
+  // plane ground model (cp_set_ground_plane, plane_kernels.cuh)
+  bool plane_on = false;
+  cp_plane_params plane{};
+  double plane_cos = 0.0;
+  bool plane_run = false;    // the last run was the plane chain
+  bool plane_valid = false;  // the last run or ground call used the plane model: the plane buffers describe it
+  u32 plane_frames = 0, plane_h = 0;
+  PlaneBufs pb{};
   HostGeom hg;
   u32 *d_frame_n = nullptr, *d_frame_tile0 = nullptr, *d_tile_frame = nullptr;
   u64* d_frame_off = nullptr;
@@ -577,10 +591,10 @@ void launch_keep_mask(cp_handle* h, const Geom& g, const CropK& c, const GroundK
   while (split_log2 < 3 && (((u64)g.n_tiles * 2u) << (split_log2 + 1)) <= total_warps) ++split_log2;
   if (split_log2) grid = grid_for((((u64)g.n_tiles * 2u) << split_log2) * 32u, kStreamThreads, h->sms, h->stream_ctas_per_sm);
   const u32* rm = h->rowmax_valid ? h->d_rowmax : nullptr;
-  switch (h->layout.mode) {
-    case 0: keep_mask_kernel<0><<<grid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, g, c, gk, h->d_thr_f, rm, mo, split_log2); break;
-    case 1: keep_mask_kernel<1><<<grid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, g, c, gk, h->d_thr_f, rm, mo, split_log2); break;
-    default: keep_mask_kernel<2><<<grid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, g, c, gk, h->d_thr_f, rm, mo, split_log2); break;
+  switch (h->run_layout.mode) {
+    case 0: keep_mask_kernel<0><<<grid, kStreamThreads, 0, h->stream>>>(h->run_in, h->run_layout, g, c, gk, h->d_thr_f, rm, mo, split_log2); break;
+    case 1: keep_mask_kernel<1><<<grid, kStreamThreads, 0, h->stream>>>(h->run_in, h->run_layout, g, c, gk, h->d_thr_f, rm, mo, split_log2); break;
+    default: keep_mask_kernel<2><<<grid, kStreamThreads, 0, h->stream>>>(h->run_in, h->run_layout, g, c, gk, h->d_thr_f, rm, mo, split_log2); break;
   }
   if (h->stage_timing) cudaEventRecord(h->ev_k[3], h->stream);
   h->launches++;
@@ -601,10 +615,10 @@ void launch_scan_gather(cp_handle* h, const Geom& g, const GroundK& gk, u32 cap)
   tile_scan_kernel<<<(h->tile_ctas || stiles < (u32)h->sms * 4) ? stiles : (u32)h->sms * 4, kScanThreads, 0, h->stream>>>(
       g, h->d_tile_count, h->d_tile_excl, h->d_c_off, h->d_desc_a, h->d_ctl, cap);
   const u32 ggrid = grid_for((u64)g.n_tiles * 32, 256, h->sms, 8);
-  switch (h->layout.mode) {
-    case 0: gather_survivors_kernel<0><<<ggrid, 256, 0, h->stream>>>(h->in_ptr, h->layout, g, gk, h->d_mask, h->d_tile_count, h->d_tile_excl, go); break;
-    case 1: gather_survivors_kernel<1><<<ggrid, 256, 0, h->stream>>>(h->in_ptr, h->layout, g, gk, h->d_mask, h->d_tile_count, h->d_tile_excl, go); break;
-    default: gather_survivors_kernel<2><<<ggrid, 256, 0, h->stream>>>(h->in_ptr, h->layout, g, gk, h->d_mask, h->d_tile_count, h->d_tile_excl, go); break;
+  switch (h->run_layout.mode) {
+    case 0: gather_survivors_kernel<0><<<ggrid, 256, 0, h->stream>>>(h->run_in, h->run_layout, g, gk, h->d_mask, h->d_tile_count, h->d_tile_excl, go); break;
+    case 1: gather_survivors_kernel<1><<<ggrid, 256, 0, h->stream>>>(h->run_in, h->run_layout, g, gk, h->d_mask, h->d_tile_count, h->d_tile_excl, go); break;
+    default: gather_survivors_kernel<2><<<ggrid, 256, 0, h->stream>>>(h->run_in, h->run_layout, g, gk, h->d_mask, h->d_tile_count, h->d_tile_excl, go); break;
   }
   h->launches += 2;
   h->gathered = true;
@@ -629,8 +643,8 @@ void launch_mask_compact(cp_handle* h, const Geom& g, const CropK& c, const Grou
   const u32 grid = std::min<u32>(g.n_tiles ? g.n_tiles : 1u, (u32)h->sms * 4u);
   u32* ticket = &h->d_ctl->ticket[0];
 #define CP_MC(M) mask_compact_kernel<M, OUT32><<<grid, kStreamThreads, 0, h->stream>>>(                         \
-      h->in_ptr, h->layout, g, c, gk, h->d_thr_f, rm, h->d_desc_a, ticket, go, h->d_c_off, h->d_gcount, h->d_ctl)
-  switch (h->layout.mode) {
+      h->run_in, h->run_layout, g, c, gk, h->d_thr_f, rm, h->d_desc_a, ticket, go, h->d_c_off, h->d_gcount, h->d_ctl)
+  switch (h->run_layout.mode) {
     case 0: CP_MC(0); break;
     case 1: CP_MC(1); break;
     default: CP_MC(2); break;
@@ -641,13 +655,13 @@ void launch_mask_compact(cp_handle* h, const Geom& g, const CropK& c, const Grou
 }
 // single HBM pass: one 16-CTA cluster per frame, points stashed in shared memory (cluster_front.cuh)
 bool cluster_front_eligible(const cp_handle* h, const Geom& g, bool ground) {
-  return h->use_cluster && ground && g.uniform_n && h->layout.mode == 0 &&
+  return h->use_cluster && ground && g.uniform_n && h->run_layout.mode == 0 &&
          g.uniform_n <= (u32)kClusterSize * kClMaxPtsPerCta;
 }
 
 bool launch_front_cluster(cp_handle* h, const Geom& g, const CropK& c, const GroundK& gk, float default_low) {
   ClusterArgs a;
-  a.in = reinterpret_cast<const float4*>(h->in_ptr);
+  a.in = reinterpret_cast<const float4*>(h->run_in);
   a.n_frames = g.n_frames;
   a.n = g.uniform_n;
   const u32 per = (g.uniform_n + kClusterSize - 1) / kClusterSize;
@@ -728,10 +742,10 @@ void launch_front_fused(cp_handle* h, const Geom& g, const CropK& c, const Groun
   const u32 items = fa.n_groups * fa.group_tiles * 2u;
   const u32 grid = items < h->fused_grid ? items : h->fused_grid;
   if (h->stage_timing) cudaEventRecord(h->ev_k[0], h->stream);
-  switch (h->layout.mode) {
-    case 0: front_fused_kernel<0><<<grid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, g, c, gk, h->d_low_key, mo, fa); break;
-    case 1: front_fused_kernel<1><<<grid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, g, c, gk, h->d_low_key, mo, fa); break;
-    default: front_fused_kernel<2><<<grid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, g, c, gk, h->d_low_key, mo, fa); break;
+  switch (h->run_layout.mode) {
+    case 0: front_fused_kernel<0><<<grid, kStreamThreads, 0, h->stream>>>(h->run_in, h->run_layout, g, c, gk, h->d_low_key, mo, fa); break;
+    case 1: front_fused_kernel<1><<<grid, kStreamThreads, 0, h->stream>>>(h->run_in, h->run_layout, g, c, gk, h->d_low_key, mo, fa); break;
+    default: front_fused_kernel<2><<<grid, kStreamThreads, 0, h->stream>>>(h->run_in, h->run_layout, g, c, gk, h->d_low_key, mo, fa); break;
   }
   if (h->stage_timing) cudaEventRecord(h->ev_k[1], h->stream);
   h->launches++;
@@ -740,7 +754,7 @@ void launch_front_fused(cp_handle* h, const Geom& g, const CropK& c, const Groun
 template <int MODE>
 void launch_sector_min_mode(cp_handle* h, const Geom& g, u32 grid) {
   if (!h->tail_priority) {
-    ground_sector_min_kernel<MODE><<<grid, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, g, h->d_low_key, h->d_rowmax);
+    ground_sector_min_kernel<MODE><<<grid, kStreamThreads, 0, h->stream>>>(h->run_in, h->run_layout, g, h->d_low_key, h->d_rowmax);
     return;
   }
   // the stream runs at the greatest priority; pass 1 alone is demoted, so that the short kernels behind
@@ -754,12 +768,12 @@ void launch_sector_min_mode(cp_handle* h, const Geom& g, u32 grid) {
   at[0].val.priority = h->prio_low;
   cfg.attrs = at;
   cfg.numAttrs = 1;
-  cudaLaunchKernelEx(&cfg, ground_sector_min_kernel<MODE>, h->in_ptr, h->layout, g, h->d_low_key, h->d_rowmax);
+  cudaLaunchKernelEx(&cfg, ground_sector_min_kernel<MODE>, h->run_in, h->run_layout, g, h->d_low_key, h->d_rowmax);
 }
 void launch_sector_min(cp_handle* h, const Geom& g, u32 grid) {
   if (h->k1_ctas_per_sm)
     grid = grid_for((u64)g.n_tiles * kStreamThreads, kStreamThreads, h->sms, h->k1_ctas_per_sm);
-  switch (h->layout.mode) {
+  switch (h->run_layout.mode) {
     case 0: launch_sector_min_mode<0>(h, g, grid); break;
     case 1: launch_sector_min_mode<1>(h, g, grid); break;
     default: launch_sector_min_mode<2>(h, g, grid); break;
@@ -981,8 +995,8 @@ void launch_frame_kernel(cp_handle* h, const FrameArgs& fa) {
 FrameArgs frame_args(cp_handle* h, const RunParams& rp) {
   FrameArgs fa;
   fa.n_frames = h->hg.n_frames;
-  fa.in = h->in_ptr;
-  fa.layout = h->layout;
+  fa.in = h->run_in;
+  fa.layout = h->run_layout;
   fa.geom = device_geom(h);
   fa.mask = h->run_fused_mask ? nullptr : h->d_mask;
   fa.rowmax = h->rowmax_valid ? h->d_rowmax : nullptr;
@@ -1059,7 +1073,7 @@ bool launch_single_frame_t(cp_handle* h, const SingleArgs& a, size_t smem) {
 }
 
 bool single_frame_eligible(const cp_handle* h, const Geom& g) {
-  return h->use_single && g.n_frames == 1 && g.uniform_n != 0 && h->layout.mode <= 1 && !h->taps && !h->stage_timing &&
+  return h->use_single && !h->plane_run && g.n_frames == 1 && g.uniform_n != 0 && h->run_layout.mode <= 1 && !h->taps && !h->stage_timing &&
          h->back_mode < 3 && !h->gather.open && g.uniform_n <= (u32)kSfCluster * kSfMaxPtsPerCta;
 }
 
@@ -1087,7 +1101,7 @@ bool launch_single_frame(cp_handle* h, const RunParams& rp, float default_low) {
 #define CP_SF(CM, VM)                                                                                         \
   do {                                                                                                        \
     const size_t smem = std::max(stash, sizeof(FrameSmem<CM, VM, kSfThreads>));                               \
-    ok = h->layout.mode == 0 ? launch_single_frame_t<CM, VM, 0>(h, a, smem) : launch_single_frame_t<CM, VM, 1>(h, a, smem); \
+    ok = h->run_layout.mode == 0 ? launch_single_frame_t<CM, VM, 0>(h, a, smem) : launch_single_frame_t<CM, VM, 1>(h, a, smem); \
   } while (0)
   if (h->back_mode == 0) CP_SF(1024, 512);
   else if (h->back_mode == 1) CP_SF(2048, 1024);
@@ -1110,7 +1124,7 @@ void enqueue_back_fast(cp_handle* h, const RunParams& rp) {
   // the crop taps (survivor arrays, offsets) come from the global keep mask + gather
   if (h->taps && !h->masked) launch_keep_mask(h, fa.geom, rp.crop, rp.gk, h->run_sgrid);
   if (h->taps && !h->gathered) launch_scan_gather(h, fa.geom, rp.gk, (u32)h->cap_c);
-  switch (h->layout.mode) {
+  switch (h->run_layout.mode) {
     case 0: launch_frame_kernel<CMAX, VMAX, 0, T>(h, fa); break;
     case 1: launch_frame_kernel<CMAX, VMAX, 1, T>(h, fa); break;
     default: launch_frame_kernel<CMAX, VMAX, 2, T>(h, fa); break;
@@ -1187,6 +1201,9 @@ cp_status enqueue_back(cp_handle* h, bool retry) {
   else if (h->back_mode == 1) enqueue_back_fast<2048, 1024, 512>(h, rp);
   else if (h->back_mode == 2) enqueue_back_fast<4096, 2048, 512>(h, rp);
   else {
+    // the pass over the scan below counts the ground survivors again (atomically); a per-frame kernel that evaluated
+    // pass 2 itself has already stored them
+    if (retry && !h->masked) CK(cudaMemsetAsync(h->d_gcount, 0, sizeof(u32) * h->hg.n_frames, h->stream));
     if (!h->masked && !h->gathered) {
       launch_mask_compact<false>(h, device_geom(h), rp.crop, rp.gk, (u32)h->cap_c, nullptr);
     } else {   // a keep mask exists already (single-pass front ends, a retried one-launch frame)
@@ -1194,6 +1211,10 @@ cp_status enqueue_back(cp_handle* h, bool retry) {
       if (!h->gathered) launch_scan_gather(h, device_geom(h), rp.gk, (u32)h->cap_c);
     }
     enqueue_back_general(h, rp);
+  }
+  if (h->plane_run) {
+    plane_counters_kernel<<<(h->hg.n_frames + 255) / 256, 256, 0, h->stream>>>(h->hg.n_frames, h->pb.kept, h->d_fc);
+    h->launches++;
   }
   if (h->gather.open) enqueue_gather_publish(h, retry);
   if (!h->capturing) cudaEventRecord(h->ev1, h->stream);
@@ -1241,7 +1262,57 @@ cp_status enqueue_result_fetch(cp_handle* h) {
   return CP_OK;
 }
 
+cp_status ensure_out32(cp_handle* h) {
+  if (h->d_out32) return CP_OK;
+  cudaError_t e = cudaMalloc(&h->d_out32, (size_t)h->cfg.max_points * 32);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    h->err = "cudaMalloc of the 32-byte output cloud failed";
+    return CP_E_NOMEM;
+  }
+  return CP_OK;
+}
+
+// The plane ground node over the staged input (plane_kernels.cuh): every frame's message into d_out32, G_f into
+// pb.kept, the chosen planes into pb.sel / pb.info.  Five launches.  count_rows: add every row to rows_loaded (the
+// ground calls; in a run the detector's own pass over the messages counts them).
+template <int MODE>
+void launch_plane_node_t(cp_handle* h, const Geom& g, const PlaneK& k, u32 hgrid, Ctl* ctl) {
+  plane_hyp_kernel<MODE><<<hgrid, 256, 0, h->stream>>>(h->in_ptr, h->layout, g, k, h->pb);
+  plane_score_kernel<MODE><<<g.n_tiles, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, g, k, h->pb);
+  plane_select_kernel<<<(g.n_frames + 3) / 4, 128, 0, h->stream>>>(g.n_frames, k, h->pb);
+  plane_count_kernel<MODE><<<g.n_tiles, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, g, k, h->pb);
+  plane_write_kernel<MODE><<<g.n_tiles, kStreamThreads, 0, h->stream>>>(h->in_ptr, h->layout, g, k, h->pb, h->d_out32,
+                                                                        ctl);
+}
+cp_status enqueue_plane_node(cp_handle* h, bool count_rows) {
+  const Geom g = device_geom(h);
+  PlaneK k;
+  k.seed = h->plane.seed;
+  k.H = h->plane.n_hypotheses;
+  k.inlier = h->plane.inlier_distance;
+  k.height = h->plane.ground_height;
+  k.cos_tilt = h->plane_cos;
+  const u32 hgrid = grid_for((u64)g.n_frames * k.H, 256, h->sms, 8);
+  Ctl* ctl = count_rows ? h->d_ctl : nullptr;
+  switch (h->layout.mode) {
+    case 0: launch_plane_node_t<0>(h, g, k, hgrid, ctl); break;
+    case 1: launch_plane_node_t<1>(h, g, k, hgrid, ctl); break;
+    default: launch_plane_node_t<2>(h, g, k, hgrid, ctl); break;
+  }
+  h->launches += 5;
+  h->plane_valid = true;
+  h->plane_frames = g.n_frames;
+  h->plane_h = k.H;
+  CK(cudaGetLastError());
+  return CP_OK;
+}
+
 cp_status enqueue_pipeline(cp_handle* h, const cp_detect_params* d, const cp_ground_params* ground) {
+  // the plane model (cp_set_ground_plane): the plane ground node's messages, then the detector without ground
+  // removal on them — the two-node chain, on the device
+  const bool plane = ground && h->plane_on;
+  if (plane) ground = nullptr;
   if (!d) {
     h->err = "NULL detect params";
     return CP_E_PARAM;
@@ -1275,6 +1346,10 @@ cp_status enqueue_pipeline(cp_handle* h, const cp_detect_params* d, const cp_gro
 
   const Geom g = device_geom(h);
   h->launches = 0;
+  h->plane_run = plane;
+  if (!plane) h->plane_valid = false;
+  h->run_in = plane ? h->d_out32 : h->in_ptr;
+  h->run_layout = plane ? make_layout(32, 0, 4, 8, 16) : h->layout;
   h->rp.d = *d;
   h->rp.vk = vk;
   h->rp.ck = ck;
@@ -1303,6 +1378,10 @@ cp_status enqueue_pipeline(cp_handle* h, const cp_detect_params* d, const cp_gro
   }
   if (!h->capturing) cudaEventRecord(h->ev0, h->stream);
   launch_init(h, ground ? ground->default_lowest_point : 0.0f);
+  if (plane) {
+    st = enqueue_plane_node(h, false);
+    if (st) return st;
+  }
   h->masked = false;
   h->run_fused_mask = false;
   h->ran_frame_kernel = false;
@@ -1328,7 +1407,9 @@ cp_status enqueue_pipeline(cp_handle* h, const cp_detect_params* d, const cp_gro
     // pass 2 (ground verdicts + crop) normally runs inside the per-frame kernel; the separate streaming kernel
     // serves the general back half and — a few frames without ground removal, where every row is live and one
     // CTA per frame would be too few — small unskippable batches
-    h->run_fused_mask = h->fuse_mask && h->back_mode < 3 && (ground != nullptr || g.n_frames >= (u32)h->sms || h->fuse_mask_always);
+    // (the plane chain too, so that its launch count does not depend on the number of frames)
+    h->run_fused_mask = h->fuse_mask && h->back_mode < 3 &&
+                        (ground != nullptr || plane || g.n_frames >= (u32)h->sms || h->fuse_mask_always);
     // (the general back half judges and compacts the points in one pass of its own: no keep mask for it)
     if (!h->run_fused_mask && h->back_mode < 3) launch_keep_mask(h, g, crop, gk, sgrid);
   }
@@ -1486,6 +1567,10 @@ static cp_status groundless_crops(cp_handle* h, const cp_cloud_view* cloud, bool
   if (cloud || h->color_cloud != CP_COLOR_CLOUD_GROUNDLESS) return CP_OK;
   if (!h->ran) {
     h->err = "groundless colour crops need a run on the staged input (none since it was staged)";
+    return CP_E_STATE;
+  }
+  if (h->plane_run) {
+    h->err = "groundless colour crops re-derive the sector model's verdict: not available after a plane-model run";
     return CP_E_STATE;
   }
   if (!h->rp_has_ground) return CP_OK;
@@ -1969,6 +2054,7 @@ cp_status cp_batch_set_device_input(cp_handle* h, const void* d_points, uint32_t
   CK(cudaSetDevice(h->cfg.device));
   h->batch_ready = false;
   h->ground_out = false;
+  h->plane_valid = false;   // the planes belong to the previous input
   cp_status st = set_geometry(h, frame_points, n_frames);
   if (st) return st;
   h->layout = make_layout(point_step, off_x, off_y, off_z, off_intensity);
@@ -1990,6 +2076,7 @@ cp_status cp_batch_set_host_input(cp_handle* h, const cp_cloud_view* frames, uin
   CK(cudaSetDevice(h->cfg.device));
   h->batch_ready = false;
   h->ground_out = false;
+  h->plane_valid = false;   // the planes belong to the previous input
   std::vector<u32> fp(n_frames);
   size_t bytes = 0;
   for (u32 f = 0; f < n_frames; ++f) {
@@ -2071,6 +2158,9 @@ struct RunKey {
   const void* gather_base;
   cp_detect_params d;
   cp_ground_params g;
+  // the ground model: a graph captured under one model is never replayed under the other
+  u32 plane_on;
+  cp_plane_params plane;
 };
 
 static RunKey make_key(const cp_handle* h, const cp_detect_params* d, const cp_ground_params* ground) {
@@ -2091,6 +2181,10 @@ static RunKey make_key(const cp_handle* h, const cp_detect_params* d, const cp_g
   k.gather_base = h->gather.base;
   k.d = *d;
   if (ground) k.g = *ground;
+  if (ground && h->plane_on) {
+    k.plane_on = 1;
+    k.plane = h->plane;
+  }
   return k;
 }
 
@@ -2114,6 +2208,17 @@ cp_status cp_batch_run(cp_handle* h, const cp_detect_params* d, const cp_ground_
     if (!h->graph_self_published) cudaEventRecord(h->ev0, h->stream);
     CK(cudaGraphLaunch(h->graph_exec, h->stream));
     if (!h->graph_self_published) cudaEventRecord(h->ev1, h->stream);
+    // the host state the enqueue set, for cp_sync's back-half retry, the taps and the colour calls
+    h->plane_run = h->graph_plane_run;
+    h->run_in = h->plane_run ? h->d_out32 : h->in_ptr;
+    h->run_layout = h->plane_run ? make_layout(32, 0, 4, 8, 16) : h->layout;
+    if (h->plane_run) {
+      h->plane_valid = true;
+      h->plane_frames = h->hg.n_frames;
+      h->plane_h = h->plane.n_hypotheses;
+    } else {
+      h->plane_valid = false;
+    }
     h->launches = h->graph_launches;
     h->gathered = false;
     h->self_published = h->graph_self_published;
@@ -2154,6 +2259,7 @@ cp_status cp_batch_run(cp_handle* h, const cp_detect_params* d, const cp_ground_
   h->graph_key_valid = true;
   h->graph_launches = h->launches;
   h->graph_self_published = h->self_published;
+  h->graph_plane_run = h->plane_run;
   if (!h->self_published) cudaEventRecord(h->ev0, h->stream);
   CK(cudaGraphLaunch(h->graph_exec, h->stream));
   if (!h->self_published) cudaEventRecord(h->ev1, h->stream);
@@ -2271,17 +2377,17 @@ namespace {
 // The ground node over the staged batch (cp_ground_remove, cp_batch_ground_remove): pass 1 (sector minima), then
 // every frame's complete message into d_out32 in one pass (mask_compact_kernel<*, true>).  Enqueued only.
 cp_status enqueue_ground(cp_handle* h, const cp_ground_params* g) {
-  if (!h->d_out32) {
-    cudaError_t e = cudaMalloc(&h->d_out32, (size_t)h->cfg.max_points * 32);
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      h->err = "cudaMalloc of the 32-byte output cloud failed";
-      return CP_E_NOMEM;
-    }
-  }
+  cp_status st = ensure_out32(h);
+  if (st) return st;
   const Geom geo = device_geom(h);
   h->launches = 0;
+  h->key_valid = false;   // the run state below is the ground call's: the next run is enqueued, not replayed
+  h->plane_run = false;
+  h->run_in = h->in_ptr;
+  h->run_layout = h->layout;
   launch_init(h, g->default_lowest_point);
+  if (h->plane_on) return enqueue_plane_node(h, true);
+  h->plane_valid = false;
   const u32 sgrid = grid_for((u64)geo.n_tiles * kStreamThreads, kStreamThreads, h->sms, 8);
   launch_sector_min(h, geo, sgrid);
   h->launches++;
@@ -2328,12 +2434,17 @@ cp_status cp_ground_remove(cp_handle* h, const cp_cloud_view* in, const cp_groun
     h->err = "NULL ground params or output";
     return CP_E_PARAM;
   }
+  if (low17 && h->plane_on) {
+    h->err = "low17 (sector minima) requested under the plane ground model";
+    return CP_E_PARAM;
+  }
   cp_status st = cp_batch_set_host_input(h, in, 1);
   if (st) return st;
   const u32 n = h->hg.frame_n[0];
   st = enqueue_ground(h, g);
   if (st) return st;
   CK(cudaMemcpyAsync(h->h_ctl, h->d_ctl, sizeof(Ctl), cudaMemcpyDeviceToHost, h->stream));
+  if (h->plane_on) CK(cudaMemcpyAsync(&h->h_ctl->n_surv, h->pb.kept, sizeof(u32), cudaMemcpyDeviceToHost, h->stream));
   static_assert(kNSect <= kSectStride, "h_frame_u32 holds at least kSectStride words");
   if (low17) CK(cudaMemcpyAsync(h->h_frame_u32, h->d_low_key, sizeof(u32) * kNSect, cudaMemcpyDeviceToHost, h->stream));
   uint8_t* out8 = static_cast<uint8_t*>(out_xyzi32);
@@ -2362,6 +2473,10 @@ cp_status cp_batch_ground_remove(cp_handle* h, const cp_ground_params* g, void* 
     h->err = "NULL ground params";
     return CP_E_PARAM;
   }
+  if (low17 && h->plane_on) {
+    h->err = "low17 (sector minima) requested under the plane ground model";
+    return CP_E_PARAM;
+  }
   if (!h->batch_ready) {
     h->err = "cp_batch_ground_remove before cp_batch_set_device_input / cp_batch_set_host_input";
     return CP_E_STATE;
@@ -2383,7 +2498,8 @@ cp_status cp_batch_ground_remove(cp_handle* h, const cp_ground_params* g, void* 
   u32* h_kept = h->h_ground;
   u32* h_low = h->h_ground + F;
   CK(cudaMemcpyAsync(h->h_ctl, h->d_ctl, sizeof(Ctl), cudaMemcpyDeviceToHost, h->stream));   // cp_last_rows_loaded
-  CK(cudaMemcpyAsync(h_kept, h->d_c_off + 1, sizeof(u32) * F, cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(h_kept, h->plane_on ? h->pb.kept : h->d_c_off + 1, sizeof(u32) * F, cudaMemcpyDeviceToHost,
+                     h->stream));
   if (low17) CK(cudaMemcpyAsync(h_low, h->d_low_key, sizeof(u32) * kSectStride * F, cudaMemcpyDeviceToHost, h->stream));
   uint8_t* out8 = static_cast<uint8_t*>(out_xyzi32);
   if (out8) fill_pad_host(h, out8, (size_t)n * 32);
@@ -2426,6 +2542,72 @@ cp_status cp_batch_ground_device_output(cp_handle* h, const void** d_out_xyzi32,
   }
   *d_out_xyzi32 = h->d_out32;
   *n_points = h->ground_points;
+  return CP_OK;
+} catch (...) {
+  return abi_exception(h);
+}
+
+cp_status cp_set_ground_plane(cp_handle* h, const cp_plane_params* p) try {
+  if (!h) return CP_E_PARAM;
+  if (!p) {
+    h->plane_on = false;
+    return CP_OK;
+  }
+  if (p->n_hypotheses < 1 || p->n_hypotheses > kPlaneMaxH || !std::isfinite(p->inlier_distance) ||
+      !(p->inlier_distance > 0.0f) || !std::isfinite(p->ground_height) ||
+      !(p->max_tilt_deg > 0.0f && p->max_tilt_deg <= 90.0f)) {
+    h->err = "plane params: n_hypotheses 1..256, inlier_distance finite and > 0, ground_height finite, "
+             "max_tilt_deg in (0, 90]";
+    return CP_E_PARAM;
+  }
+  CK(cudaSetDevice(h->cfg.device));
+  cp_status st = ensure_out32(h);
+  if (st) return st;
+  if (!h->pb.hyp) {
+    const size_t F = h->cfg.max_frames;
+    if ((st = dalloc(h, &h->pb.hyp, F * kPlaneMaxH))) return st;
+    if ((st = dalloc(h, &h->pb.cnt, F * kPlaneMaxH))) return st;
+    if ((st = dalloc(h, &h->pb.sel, F))) return st;
+    if ((st = dalloc(h, &h->pb.info, 2 * F))) return st;
+    if ((st = dalloc(h, &h->pb.tcount, (size_t)std::max<u32>(h->tiles_cap, 1)))) return st;
+    if ((st = dalloc(h, &h->pb.kept, F))) return st;
+  }
+  h->plane = *p;
+  h->plane_cos = cos((double)p->max_tilt_deg * (M_PI / 180.0));
+  h->plane_on = true;
+  return CP_OK;
+} catch (...) {
+  return abi_exception(h);
+}
+
+cp_status cp_ground_planes(cp_handle* h, float* planes, uint32_t* inliers, int32_t* hypothesis, uint32_t cap_frames) try {
+  if (!h) return CP_E_PARAM;
+  CK(cudaSetDevice(h->cfg.device));
+  cp_status st = cp_sync(h);
+  if (st) return st;
+  if (!h->plane_valid) {
+    h->err = "the last run or ground call did not use the plane ground model";
+    return CP_E_STATE;
+  }
+  const u32 F = h->plane_frames;
+  if (cap_frames < F) {
+    h->err = "cap_frames is smaller than the number of frames";
+    return CP_E_CAPACITY;
+  }
+  std::vector<float4> sel(F);
+  std::vector<u32> info(2 * (size_t)F);
+  CK(cudaMemcpy(sel.data(), h->pb.sel, sizeof(float4) * F, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(info.data(), h->pb.info, sizeof(u32) * 2 * F, cudaMemcpyDeviceToHost));
+  for (u32 f = 0; f < F; ++f) {
+    if (planes) {
+      planes[4 * f] = sel[f].x;
+      planes[4 * f + 1] = sel[f].y;
+      planes[4 * f + 2] = sel[f].z;
+      planes[4 * f + 3] = sel[f].w;
+    }
+    if (inliers) inliers[f] = info[2 * f];
+    if (hypothesis) hypothesis[f] = (int32_t)info[2 * f + 1];
+  }
   return CP_OK;
 } catch (...) {
   return abi_exception(h);
@@ -2724,8 +2906,29 @@ void* cp_stream(cp_handle* h) { return h ? (void*)h->stream : nullptr; }
 cp_status cp_debug_tap(cp_handle* h, cp_tap which, void* out, uint64_t cap_bytes, uint64_t* count) try {
   if (!h || !out || !count) return CP_E_PARAM;
   CK(cudaSetDevice(h->cfg.device));
+  if (which == CP_TAP_PLANE_HYPOTHESES || which == CP_TAP_PLANE_COUNTS) {
+    if (!h->plane_valid) {
+      h->err = "the last run or ground call did not use the plane ground model";
+      return CP_E_STATE;
+    }
+    cp_status st = cp_sync(h);
+    if (st) return st;
+    const u64 n = (u64)h->plane_frames * h->plane_h, esz = which == CP_TAP_PLANE_COUNTS ? 4 : 16;
+    if (n * esz > cap_bytes) {
+      h->err = "tap buffer too small";
+      return CP_E_CAPACITY;
+    }
+    if (n) CK(cudaMemcpy(out, which == CP_TAP_PLANE_COUNTS ? (const void*)h->pb.cnt : (const void*)h->pb.hyp, n * esz,
+                         cudaMemcpyDeviceToHost));
+    *count = n;
+    return CP_OK;
+  }
   if (!h->ran) {
     h->err = "cp_debug_tap before a batch ran";
+    return CP_E_STATE;
+  }
+  if (which == CP_TAP_SECTOR_LOW && h->plane_run) {
+    h->err = "no sector minima: the last run used the plane ground model";
     return CP_E_STATE;
   }
   cp_status st = cp_sync(h);
@@ -3147,6 +3350,10 @@ cp_status cp_batch_cone_colors(cp_handle* h, float cone_width, double extension_
     h->err = "no colour net loaded (cp_color_net_load / cp_color_net_load_tflite)";
     return CP_E_STATE;
   }
+  if (h->plane_run && h->color_cloud == CP_COLOR_CLOUD_GROUNDLESS) {
+    h->err = "groundless colour crops re-derive the sector model's verdict: not available after a plane-model run";
+    return CP_E_STATE;
+  }
   cp_status st = cp_sync(h);  // the final records: cp_sync may re-run the back half
   if (st) return st;
   const u64 K64 = h->h_ctl->n_clusters;
@@ -3321,6 +3528,10 @@ cp_status cp_batch_track(cp_handle* h, const cp_track_params* t, const uint32_t*
   }
   if (t->classify_colors && !h->color.net_loaded) {
     h->err = "no colour net loaded (cp_color_net_load / cp_color_net_load_tflite)";
+    return CP_E_STATE;
+  }
+  if (t->classify_colors && h->plane_run && h->color_cloud == CP_COLOR_CLOUD_GROUNDLESS) {
+    h->err = "groundless colour crops re-derive the sector model's verdict: not available after a plane-model run";
     return CP_E_STATE;
   }
   CK(cudaSetDevice(h->cfg.device));

@@ -361,6 +361,30 @@ int ch_ground_publish(void* gp, const float* xyzi, const uint32_t* frame_n, uint
   }
 }
 
+// the node parameters ~ground_model (plane != 0: "plane", else "sectors") and ~plane_* of either node (nodes.hpp
+// GroundModelParams); read at the next message
+namespace {
+void set_ground_model(GroundModelParams* m, int plane, int seed, int hypotheses, double inlier_distance,
+                      double ground_height, double max_tilt_deg) {
+  m->ground_model = plane ? "plane" : "sectors";
+  m->plane_seed = seed;
+  m->plane_hypotheses = hypotheses;
+  m->plane_inlier_distance = inlier_distance;
+  m->plane_ground_height = ground_height;
+  m->plane_max_tilt_deg = max_tilt_deg;
+}
+}  // namespace
+void ch_ground_set_ground_model(void* gp, int plane, int seed, int hypotheses, double inlier_distance,
+                                double ground_height, double max_tilt_deg) {
+  set_ground_model(static_cast<GroundRemover*>(gp), plane, seed, hypotheses, inlier_distance, ground_height,
+                   max_tilt_deg);
+}
+void ch_detector_set_ground_model(void* dp, int plane, int seed, int hypotheses, double inlier_distance,
+                                  double ground_height, double max_tilt_deg) {
+  set_ground_model(static_cast<ConeDetector*>(dp), plane, seed, hypotheses, inlier_distance, ground_height,
+                   max_tilt_deg);
+}
+
 int ch_ground_handle(void* gp, const float* xyzi, uint32_t n, int with_intensity_field, void* out32,
                      uint32_t* kept, uint32_t* out_point_step, uint32_t* out_stamp_nsec, uint32_t* out_n_fields) {
   try {

@@ -37,7 +37,37 @@ class GpuError : public std::runtime_error {
   cp_status status;
 };
 
-class GroundRemover {
+// Not in the reference (PARITY UNPINNED, cp_plane_params in include/conesgpu.h): the ground model of a node, node
+// parameter ~ground_model: "sectors" (the reference's per-sector minima, the default) or "plane" (a seeded RANSAC plane
+// per frame, for a pitching or rolling sensor), with the plane model's ~plane_* parameters.
+struct GroundModelParams {
+  std::string ground_model = "sectors";
+  int plane_seed = 0;
+  int plane_hypotheses = 64;
+  double plane_inlier_distance = 0.1;
+  double plane_ground_height = 0.1;
+  double plane_max_tilt_deg = 15.0;
+
+ protected:
+  // selects the model on the handle before a call with ground removal
+  void apply_ground_model(cp_handle* h) const {
+    cp_status st;
+    if (ground_model == "sectors") {
+      st = cp_set_ground_plane(h, nullptr);
+    } else if (ground_model == "plane") {
+      const cp_plane_params p{static_cast<uint64_t>(static_cast<uint32_t>(plane_seed)),
+                              plane_hypotheses > 0 ? static_cast<uint32_t>(plane_hypotheses) : 0u,
+                              static_cast<float>(plane_inlier_distance), static_cast<float>(plane_ground_height),
+                              static_cast<float>(plane_max_tilt_deg)};
+      st = cp_set_ground_plane(h, &p);
+    } else {
+      throw GpuError(CP_E_PARAM, "ground_model must be \"sectors\" or \"plane\", not \"" + ground_model + "\"");
+    }
+    if (st != CP_OK) throw GpuError(st, cp_last_error(h));
+  }
+};
+
+class GroundRemover : public GroundModelParams {
  public:
   // members, src/ground_removal.cpp:18-27 (set them before the first cloud_handler call; the
   // reference reads them once in its constructor, :31-39)
@@ -67,6 +97,7 @@ class GroundRemover {
   PointCloud2 cloud_handler(const PointCloud2& cloud_msg) {
     cp_cloud_view in = make_view(cloud_msg, /*fake_missing_intensity=*/false);
     cp_ground_params g{num_of_sectors, default_lowest_point};
+    apply_ground_model(gpu_);
     PointCloud2 out = published_shell(cloud_msg);
     cp_status st = cp_ground_remove(gpu_, &in, &g, out.data.data(), &last_kept_, nullptr);
     if (st != CP_OK) throw GpuError(st, cp_last_error(gpu_));
@@ -80,6 +111,7 @@ class GroundRemover {
     std::vector<PointCloud2> out;
     out.reserve(msgs.size());
     cp_ground_params g{num_of_sectors, default_lowest_point};
+    apply_ground_model(gpu_);
     size_t i = 0;
     while (i < msgs.size()) {
       std::vector<cp_cloud_view> views;
@@ -254,7 +286,7 @@ class ConeTracker {
   std::shared_ptr<std::vector<Point>> prev_centroid_clouds_[kNumberOfColors];
 };
 
-class ConeDetector {
+class ConeDetector : public GroundModelParams {
  public:
   // members, src/cone_detection.cpp:22-51, same names / types / defaults
   const float CONE_WIDTH = 0.228f;
@@ -278,7 +310,8 @@ class ConeDetector {
                                                "cones_cloud_oranges"};
   // not in the reference: fuse the ground_removal node in front (one process, one H2D copy).  The cluster records
   // equal those of the two nodes chained through the groundless_cloud topic; the colour crops equal the chain's only
-  // with groundless_color_crops (otherwise they are cut from the raw cloud, ground returns included)
+  // with groundless_color_crops (otherwise they are cut from the raw cloud, ground returns included).  The fused
+  // node uses the ground model of GroundModelParams (ground_model = "plane": groundless_color_crops is refused)
   bool fused_ground_removal = false;
   // not in the reference: with fused_ground_removal, cut the colour crops from the ground node's message, as the
   // chained detector does (cp_set_color_cloud(CP_COLOR_CLOUD_GROUNDLESS)); clouds are then staged as the ground node
@@ -346,6 +379,7 @@ class ConeDetector {
                        voxel_filter_leaf_size_x, voxel_filter_leaf_size_y, voxel_filter_leaf_size_z,
                        min_cluster_size, max_cluster_size, CONE_WIDTH, CONE_HEIGHT};
     cp_ground_params g{num_of_sectors, default_lowest_point};
+    if (fused_ground_removal) apply_ground_model(gpu_);
     set_color_cloud();
     cp_cloud_view in = make_view(cloud_msg, !intensity_in_cloud_ && !groundless());
     clusters_.resize(4096);
@@ -512,6 +546,7 @@ class ConeDetector {
                        voxel_filter_leaf_size_x, voxel_filter_leaf_size_y, voxel_filter_leaf_size_z,
                        min_cluster_size, max_cluster_size, CONE_WIDTH, CONE_HEIGHT};
     cp_ground_params g{num_of_sectors, default_lowest_point};
+    if (fused_ground_removal) apply_ground_model(gpu_);
     const uint32_t F = static_cast<uint32_t>(views.size());
     std::vector<uint32_t> k_off(F + 1);
     uint64_t K = 0;

@@ -64,6 +64,27 @@ typedef struct cp_ground_params {
   float default_lowest_point;
 } cp_ground_params;
 
+/* Optional second ground model (the reference has none: PARITY UNPINNED): a seeded RANSAC plane per frame, for
+ * scans from a pitching or rolling sensor, where the sector model's "z < lowest z of the sector + 0.1" keeps the far
+ * ground.  Selected per handle with cp_set_ground_plane; the sector model stays the default.  Frame f has N_f points.
+ *   Draw:     hypothesis h takes the frame-local indices idx_j = (u32)((((splitmix64(seed + 3h + j)) >> 32) * N_f) >> 32),
+ *             j = 0, 1, 2 (splitmix64: the standard finaliser, golden-ratio increment added first).  The draw depends
+ *             on (seed, h, N_f) alone, never on the frame's place in the batch.  N_f < 3: no hypotheses.
+ *   Plane:    in double, no contraction: u = p1 - p0, v = p2 - p0, n = u x v, L = |n|.  Invalid if a sample point is
+ *             not finite, L is 0 or not finite, or nz/L < cos(max_tilt) after flipping n to nz >= 0.  Otherwise
+ *             n /= L, d = -(nx p0x + ny p0y + nz p0z); a, b, c, d rounded to float.  cos(max_tilt) in double.
+ *   Distance: s = fmaf(c, z, fmaf(b, y, fmaf(a, x, d))) in fp32.
+ *   Score:    finite points with fabsf(s) <= inlier_distance.  Best: the highest count, ties to the lowest h.
+ *   Verdict:  keep iff the point is finite and s >= ground_height; no valid plane: keep every finite point.
+ * The ground node's message keeps its format (survivors in input order, then N_f - G_f padding points). */
+typedef struct cp_plane_params {
+  uint64_t seed;
+  uint32_t n_hypotheses;   /* 1 .. 256 */
+  float inlier_distance;   /* scoring: |s| <= inlier_distance; finite, > 0 */
+  float ground_height;     /* verdict: keep iff s >= ground_height; finite */
+  float max_tilt_deg;      /* (0, 90]: a plane whose normal is further than this from +z is invalid */
+} cp_plane_params;
+
 /* ConeDetector members, src/cone_detection.cpp:22-43, same types and (typo'd) names as
  * config/cones_detection_params_*.yaml. */
 typedef struct cp_detect_params {
@@ -177,6 +198,23 @@ cp_status cp_batch_ground_remove(cp_handle* h, const cp_ground_params* g, void* 
  * included).  Valid until the next cp_ground_remove / cp_batch_ground_remove on this handle.
  * CP_E_PARAM: NULL argument.  CP_E_STATE: no cp_batch_ground_remove since the last staging or run. */
 cp_status cp_batch_ground_device_output(cp_handle* h, const void** d_out_xyzi32, uint64_t* n_points);
+
+/* Select the ground model of this handle.  p NULL: the sector model of the reference (the default).  p non-NULL: the
+ * plane model (cp_plane_params) for every later cp_ground_remove, cp_batch_ground_remove, cp_detect, cp_batch_run
+ * and cp_detect_batch with non-NULL ground params, whose num_of_sectors and default_lowest_point are then ignored.
+ * A run with the plane model is the two-node chain on the device: the plane ground node's messages, then the detector
+ * without ground removal on them, so its crop taps (CP_TAP_CROP_INDEX ...) index the messages, not the input; the
+ * counters' n_ground_kept is G_f.  Under the plane model: a non-NULL low17 returns CP_E_PARAM, CP_TAP_SECTOR_LOW
+ * returns CP_E_STATE, and so do the colour calls with CP_COLOR_CLOUD_GROUNDLESS and a NULL cloud, cp_batch_cone_colors
+ * and cp_batch_track in colour mode under CP_COLOR_CLOUD_GROUNDLESS (STAGED crops work as before).
+ * CP_E_PARAM: n_hypotheses outside 1..256, inlier_distance not finite and > 0, ground_height not finite, max_tilt_deg
+ * outside (0, 90]. */
+cp_status cp_set_ground_plane(cp_handle* h, const cp_plane_params* p);
+/* The plane each frame chose in the last run or ground call made with the plane model (calls cp_sync first):
+ * planes[n_frames][4] (a, b, c, d), inliers[n_frames] (its score), hypothesis[n_frames] (-1: no valid plane, then the
+ * plane is NaN and the inliers 0).  Any pointer may be NULL.  CP_E_STATE: the last run or ground call did not use
+ * the plane model.  CP_E_CAPACITY: cap_frames < n_frames. */
+cp_status cp_ground_planes(cp_handle* h, float* planes, uint32_t* inliers, int32_t* hypothesis, uint32_t cap_frames);
 
 /* Enqueue the whole pipeline for the current batch on the handle's stream (async). */
 cp_status cp_batch_run(cp_handle* h, const cp_detect_params* d, const cp_ground_params* ground);
@@ -416,7 +454,10 @@ typedef enum cp_tap {
   CP_TAP_VOXEL_ORDER = 5,  /* uint32  [C_total]  survivor position of each sorted record  */
   CP_TAP_VOXEL_CLOUD = 6,  /* float4  [V_total]  voxel centroids x,y,z,intensity          */
   CP_TAP_VOXEL_OFFSETS = 7,/* uint32  [n_frames+1]                                        */
-  CP_TAP_LABELS = 8        /* int32   [V_total]  frame-local min voxel index of component */
+  CP_TAP_LABELS = 8,       /* int32   [V_total]  frame-local min voxel index of component */
+  /* plane model (cp_set_ground_plane), last run or ground call with it; H = n_hypotheses */
+  CP_TAP_PLANE_HYPOTHESES = 9, /* float4 [n_frames*H]  a, b, c, d of every hypothesis, NaN when invalid */
+  CP_TAP_PLANE_COUNTS = 10     /* uint32 [n_frames*H]  inliers of every hypothesis                     */
 } cp_tap;
 cp_status cp_debug_tap(cp_handle* h, cp_tap which, void* out, uint64_t cap_bytes, uint64_t* count);
 

@@ -30,6 +30,14 @@ class ConeDetectorNode {
     private_param("fused_ground_removal", core_.fused_ground_removal);
     private_param("num_of_sectors", core_.num_of_sectors);
     private_param("default_lowest_point", core_.default_lowest_point);
+    // extension (default "sectors", the reference's model): with fused_ground_removal, "plane" removes the ground by a
+    // seeded RANSAC plane per frame
+    private_param("ground_model", core_.ground_model);
+    private_param("plane_seed", core_.plane_seed);
+    private_param("plane_hypotheses", core_.plane_hypotheses);
+    private_param("plane_inlier_distance", core_.plane_inlier_distance);
+    private_param("plane_ground_height", core_.plane_ground_height);
+    private_param("plane_max_tilt_deg", core_.plane_max_tilt_deg);
     // extension (off by default): with fused_ground_removal, colour crops from the ground node's message, as the
     // detector of the two-node launch cuts them
     private_param("groundless_color_crops", core_.groundless_color_crops);

@@ -12,6 +12,13 @@ class GroundRemoverNode {
     cones_ros::private_param("output_cloud_topic", out_topic);               // src/ground_removal.cpp:31
     cones_ros::private_param("num_of_sectors", core_.num_of_sectors);        // :34
     cones_ros::private_param("default_lowest_point", core_.default_lowest_point);  // :37
+    // extension (default "sectors", the reference's model): "plane", a seeded RANSAC plane per frame
+    cones_ros::private_param("ground_model", core_.ground_model);
+    cones_ros::private_param("plane_seed", core_.plane_seed);
+    cones_ros::private_param("plane_hypotheses", core_.plane_hypotheses);
+    cones_ros::private_param("plane_inlier_distance", core_.plane_inlier_distance);
+    cones_ros::private_param("plane_ground_height", core_.plane_ground_height);
+    cones_ros::private_param("plane_max_tilt_deg", core_.plane_max_tilt_deg);
     sub_ = nh_.subscribe<sensor_msgs::PointCloud2>(core_.input_cloud_topic, 2, &GroundRemoverNode::cloud_handler, this);  // :41
     pub_ = nh_.advertise<sensor_msgs::PointCloud2>(out_topic, 1);            // :42
   }
