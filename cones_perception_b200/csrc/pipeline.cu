@@ -135,8 +135,11 @@ struct cp_handle {
     // classifier (color_net.cuh): weights in one device block, per-cone outputs
     float* net_w = nullptr;
     size_t net_w_n = 0;
-    ColorNetDev net{};
+    ColorNetDev net{};            // net.classes and net.threshold hold for either kernel
     bool net_loaded = false;
+    bool graph_kernel = false;    // the loaded model runs on color_graph_kernel (any other graph than dam_net's)
+    ColorGraphDev graph{};
+    u32 graph_smem = 0;           // its dynamic shared memory, bytes
     uint8_t* colors = nullptr;
     float* probs = nullptr;     // [n][classes] probabilities, then [n][classes] logits
     u32* net_flags = nullptr;
@@ -1705,10 +1708,43 @@ static cp_status load_color_net(cp_handle* h, const cp_color_net* n) {
   cb.net = ColorNetDev{cb.net_w + o_w1, cb.net_w + o_b1, cb.net_w + o_w2, cb.net_w + o_b2, cb.net_w + o_sc,
                        cb.net_w + o_sh, cb.net_w + o_wd, cb.net_w + o_bd, C1, C2, NC, n->threshold};
   cb.net_loaded = true;
+  cb.graph_kernel = false;
   return CP_OK;
 }
 
-// cone_color_kernel over n images already on the device (cb.img or `images_dev`); outputs stay in cb.colors/probs
+// A graph read_color_graph accepted: its weights into the one device block, its layer program for color_graph_kernel
+static cp_status load_color_graph(cp_handle* h, const cp_tflite::ColorGraph& g, float threshold) {
+  if (!(threshold >= 0.f && threshold <= 1.f)) {
+    h->err = "colour net threshold outside [0, 1]";
+    return CP_E_PARAM;
+  }
+  cp_handle::ColorBufs& cb = h->color;
+  CK(cudaSetDevice(h->cfg.device));
+  // every handle on the device may run any accepted graph: allow the whole budget once
+  CK(cudaFuncSetAttribute(color_graph_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cp_tflite::kGraphSmemBytes));
+  cb.net_loaded = false;
+  cp_status st = grow(h, &cb.net_w, &cb.net_w_n, std::max<size_t>(g.weights.size(), 1));
+  if (st) return st;
+  CK(cudaStreamSynchronize(h->stream));
+  if (!g.weights.empty()) CK(cudaMemcpy(cb.net_w, g.weights.data(), sizeof(float) * g.weights.size(), cudaMemcpyHostToDevice));
+  cb.graph = ColorGraphDev{};
+  cb.graph.w = cb.net_w;
+  cb.graph.n_layers = (u32)g.layers.size();
+  cb.graph.classes = g.classes;
+  cb.graph.out = g.out;
+  cb.graph.logits = g.logits;
+  cb.graph.threshold = threshold;
+  std::copy(g.layers.begin(), g.layers.end(), cb.graph.layer);
+  cb.graph_smem = g.smem_floats * (u32)sizeof(float);
+  cb.net = ColorNetDev{};
+  cb.net.classes = g.classes;
+  cb.net.threshold = threshold;
+  cb.net_loaded = true;
+  cb.graph_kernel = true;
+  return CP_OK;
+}
+
+// cone_color_kernel or color_graph_kernel over n images already on the device (cb.img or `images_dev`); outputs stay in cb.colors/probs
 static cp_status enqueue_color_net(cp_handle* h, const uint8_t* images_dev, const u32* raster_flags, u32 n) {
   cp_handle::ColorBufs& cb = h->color;
   if (!cb.net_loaded) {
@@ -1719,7 +1755,10 @@ static cp_status enqueue_color_net(cp_handle* h, const uint8_t* images_dev, cons
   if ((st = grow(h, &cb.colors, &cb.colors_n, (size_t)std::max<u32>(n, 1)))) return st;
   if ((st = grow(h, &cb.probs, &cb.probs_n, (size_t)std::max<u32>(n, 1) * 2 * kNetMaxClasses))) return st;
   if ((st = grow(h, &cb.net_flags, &cb.net_flags_n, (size_t)std::max<u32>(n, 1)))) return st;
-  if (n)
+  if (n && cb.graph_kernel)
+    color_graph_kernel<<<n, kGraphThreads, cb.graph_smem, h->stream>>>(images_dev, raster_flags, cb.graph, cb.colors, cb.probs,
+                                                                       cb.probs + (size_t)n * cb.net.classes, cb.net_flags);
+  else if (n)
     cone_color_kernel<<<n, kNetThreads, 0, h->stream>>>(images_dev, raster_flags, cb.net, cb.colors, cb.probs,
                                                         cb.probs + (size_t)n * cb.net.classes, cb.net_flags);
   CK(cudaGetLastError());
@@ -3166,12 +3205,17 @@ cp_status cp_color_net_load_tflite(cp_handle* h, const void* data, size_t bytes,
     h->err = "NULL model data";
     return CP_E_PARAM;
   }
+  // dam_net's architecture keeps cone_color_kernel; every other accepted graph runs on color_graph_kernel
   cp_tflite::ColorNetWeights w;
   try {
     w = cp_tflite::read_color_net(static_cast<const uint8_t*>(data), bytes);
-  } catch (const cp_tflite::Error& e) {
-    h->err = "TFLite model refused: " + e.what;
-    return CP_E_PARAM;
+  } catch (const cp_tflite::Error&) {
+    try {
+      return load_color_graph(h, cp_tflite::read_color_graph(static_cast<const uint8_t*>(data), bytes), threshold);
+    } catch (const cp_tflite::Error& e) {
+      h->err = "TFLite model refused: " + e.what;
+      return CP_E_PARAM;
+    }
   }
   cp_color_net n{};
   n.c1 = w.c1;

@@ -352,8 +352,22 @@ typedef struct cp_color_net {
   float threshold;            /* 0.8: below it the colour is 0 = unknown (color_classifier_server.py:116-120) */
 } cp_color_net;
 cp_status cp_color_net_load(cp_handle* h, const cp_color_net* net);
-/* The same from the bytes of the .tflite file the reference's launch parameter ~model_path names.  Any graph other
- * than the architecture above is refused with CP_E_PARAM (cp_last_error says why). */
+/* The same from the bytes of the .tflite file the reference's launch parameter ~model_path names: dam_net or a
+ * retrained / reconverted classifier.  Accepted: one subgraph, one float32 input [1,15,12,1], one output [1,n] with
+ * 1 <= n <= 3 (colour = argmax + 1 when the largest output is >= threshold), at most 64 operators forming a chain
+ * (each one's first input, or either input of MUL / ADD, is the previous output; every other input is a constant),
+ * float32 tensors without quantisation, and only
+ *   CONV_2D, DEPTHWISE_CONV_2D  SAME or VALID, any stride, dilation 1
+ *   MAX_POOL_2D, AVERAGE_POOL_2D  SAME or VALID, any filter and stride
+ *   MEAN over axes {1,2} (keep_dims either way); MUL / ADD with a scalar, [C] or [1,1,1,C] constant; RELU; RELU6
+ *   RESHAPE (element count unchanged); FULLY_CONNECTED (default weights format, bias optional); SOFTMAX, last,
+ *   any finite beta; fused activations NONE, RELU, RELU6, RELU_N1_TO_1.
+ * The largest input + output pair of one layer must fit 227 KB (the shared memory of one CTA on sm_100a).  Anything
+ * else (TANH, dilation, other types, branches, custom operators) is refused with CP_E_PARAM and cp_last_error names
+ * the operator or field.  dam_net's own architecture runs on the kernel cp_color_net_load uses; every other graph
+ * on a layer-program kernel with the same arithmetic order.  The outputs of the colour calls: probs = the output
+ * tensor ([n] per cone: the softmax when the graph ends in one), logits (cp_classify_images) = the input of the
+ * final SOFTMAX, or the output itself when there is none.  n_classes of the probs / logits arrays is the graph's n. */
 cp_status cp_color_net_load_tflite(cp_handle* h, const void* data, size_t bytes, float threshold);
 /* handle_classify_color (scripts/color_classifier_server.py:78-126) for n_centers cones, entirely on the device:
  * box gather -> to_image -> network.  colors[c]: 0 unknown, 1 yellow, 2 blue, 3 orange, 255 = no answer for this
